@@ -23,6 +23,13 @@ roofline = FP32 CUDA-core pipe: 17 algorithmic FLOP per ray-sphere test (SURVEY.
          by the kernel / trace-kernel time measured with CUDA events by the library.
 cpu_baseline = the oracle (CPU port of the reference; the Zig reference cannot be built here) timed on
          this box's host cores on a bounded sample of the same workload.
+
+--dump-outputs DIR writes what the last timed step computed, so that two builds can be compared output for
+output (the inputs are seeded, hence identical from run to run): DIR/image.npy, the frame a caller receives
+(uint8 [H, W, 3]) as float32, or, for a frame larger than the dump budget, DIR/image_sample.npy with a fixed
+seeded sample of its pixels ([k, 3], float32) and their flat pixel indices in DIR/image_sample_index.npy
+(float64); and DIR/stats.npy, the frame's work counters (STAT_FIELDS, float64).  Nothing is written to the
+source tree, which may be read-only.
 """
 from __future__ import annotations
 
@@ -40,6 +47,7 @@ from pathlib import Path
 
 ROOT = Path(__file__).resolve().parent
 sys.path.insert(0, str(ROOT))
+sys.dont_write_bytecode = True   # no __pycache__ in the tree from the modules imported below
 
 SEED = 0xDEADBEEF
 WORKLOADS = {
@@ -50,6 +58,32 @@ WORKLOADS = {
 }
 FLOP_PER_TEST = 17.0  # SURVEY.md §8d / BASELINE.md §3
 TILE = (4, 4)
+STAT_FIELDS = ("samples", "segments", "sphere_tests", "depth_capped", "absorbed", "nan_samples")
+DUMP_BYTES = 64 << 20
+DUMP_SEED = 0x5EED
+
+
+def counters(stats) -> list[float]:
+    """The work counters of an rtz_stats, in STAT_FIELDS order."""
+    return [float(getattr(stats, f)) for f in STAT_FIELDS]
+
+
+def dump_outputs(dirname: str, image, stat_counters) -> None:
+    """Write one frame (uint8 [H, W, 3]) and its work counters as described in the module docstring."""
+    import numpy as np
+    d = Path(dirname)
+    d.mkdir(parents=True, exist_ok=True)
+    img = np.asarray(image, dtype=np.float32)
+    budget = DUMP_BYTES - (1 << 20)                     # headroom for stats.npy and the .npy headers
+    if img.nbytes <= budget:
+        np.save(d / "image.npy", img)
+    else:
+        flat = img.reshape(-1, 3)
+        k = budget // (flat.itemsize * 3 + 8)           # a float32 pixel plus its float64 index
+        idx = np.sort(np.random.Generator(np.random.PCG64(DUMP_SEED)).choice(flat.shape[0], k, replace=False))
+        np.save(d / "image_sample.npy", flat[idx])
+        np.save(d / "image_sample_index.npy", idx.astype(np.float64))
+    np.save(d / "stats.npy", np.array(stat_counters, dtype=np.float64))
 
 
 def measured_peaks():
@@ -103,7 +137,8 @@ class ClockSampler:
 def oracle_throughput(width: int, spp: int, threads: int | None = None):
     """Time the f64 CPU restatement of the reference on `threads` host threads (all by default) on
     the workload's scene and camera at `spp` samples per pixel.  Returns (Msamples/s, threads, samples,
-    seconds, Mtests/s)."""
+    seconds, Mtests/s, image uint8 [H, W, 3], stats)."""
+    import numpy as np
     sys.path.insert(0, str(ROOT / "tests"))
     import rtzlib as R
     orc = R.oracle()
@@ -119,7 +154,8 @@ def oracle_throughput(width: int, spp: int, threads: int | None = None):
         rc = orc.orc_render_philox64(C.byref(cam), sp, n, SEED, threads, rgb, None, C.byref(st))
     dt = time.perf_counter() - t0
     assert rc == 0
-    return st.samples / dt / 1e6, threads, int(st.samples), dt, st.sphere_tests / dt / 1e6
+    img = np.frombuffer(rgb, dtype=np.uint8).reshape(int(cam.height), int(cam.width), 3)
+    return st.samples / dt / 1e6, threads, int(st.samples), dt, st.sphere_tests / dt / 1e6, img, st
 
 
 def run_reference(args, rank: int):
@@ -129,9 +165,11 @@ def run_reference(args, rank: int):
     spp = args.ref_spp
     vals = []
     for i in range(args.warmup + args.steps):
-        v, threads, samples, dt, mt = oracle_throughput(width, spp)
+        v, threads, samples, dt, mt, img, st = oracle_throughput(width, spp)
         if i >= args.warmup:
             vals.append((v, dt, mt))
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, img, counters(st))
     value = sum(v for v, _, _ in vals) / len(vals)
     ms = 1e3 * sum(d for _, d, _ in vals) / len(vals)
     sample = f"{desc.split(':')[0]} scene+camera at {spp} of {spp_full} spp ({samples / 1e6:.2f} M samples per step)"
@@ -218,6 +256,12 @@ def run_ours(args, rank: int, world: int, local_rank: int):
         t_wall = time.perf_counter() - t_wall0
         clk = clocks.stop()
         barrier()
+    if args.dump_outputs:   # before anything below renders into `out` again
+        last_counters = torch.tensor(counters(stats[-1]), dtype=torch.float64, device=dev)
+        if world > 1:
+            dist.all_reduce(last_counters)          # each rank counted its own tiles
+        if rank == 0:
+            dump_outputs(args.dump_outputs, last["img"].cpu().numpy(), last_counters.tolist())
     dev_ms = sum(s.elapsed_time(e) for s, e in ev)
     samples = sum(int(st.samples) for st in stats)
     tests = sum(int(st.sphere_tests) for st in stats)
@@ -336,8 +380,8 @@ def run_ours(args, rank: int, world: int, local_rank: int):
     # ---- CPU baseline beside it (rank 0, N=1 only; bounded sample) ------------------------------
     cpu = None
     if world == 1 and not args.no_cpu_baseline:
-        v_all, threads, smp, dt, mt = oracle_throughput(width, args.ref_spp)
-        v_one, _, smp1, dt1, _ = oracle_throughput(400, 10, threads=1)
+        v_all, threads, smp, dt, mt, _, _ = oracle_throughput(width, args.ref_spp)
+        v_one, _, smp1, dt1, _, _, _ = oracle_throughput(400, 10, threads=1)
         cpu = {"value": round(v_all, 4), "unit": "Msamples/s", "cores": threads, "kind": "port",
                "sample": f"{args.workload.upper()} scene+camera at {args.ref_spp} of {spp} spp ({smp / 1e6:.2f} M samples, {dt:.1f} s)",
                "mtests_per_s": round(mt, 1),
@@ -414,7 +458,11 @@ def main():
     ap.add_argument("--spp", type=int, default=0, help="override samples per pixel (dev only; invalidates the headline)")
     ap.add_argument("--ref-spp", type=int, default=48, help="spp of the bounded CPU sample (cost per sample does not depend on spp)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's outputs as .npy files under DIR (see the module docstring)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

@@ -38,10 +38,17 @@ def _stale(target: Path, sources) -> bool:
     return any(Path(s).stat().st_mtime > t for s in sources)
 
 
+def _librtz_sources():
+    return sorted(CSRC.glob("*.cu")) + sorted(CSRC.glob("*.cuh")) + [ROOT / "include" / "rtz.h"]
+
+
+def _host_sources():
+    return sorted(HOST.glob("*.cpp")) + sorted(HOST.glob("*.hpp")) + [ROOT / "include" / "rtz.h", CSRC / "librtz.so"]
+
+
 def build_librtz(force: bool = False, verbose: bool = False) -> Path:
     so = CSRC / "librtz.so"
-    srcs = sorted(CSRC.glob("*.cu")) + sorted(CSRC.glob("*.cuh")) + [ROOT / "include" / "rtz.h"]
-    if force or _stale(so, srcs):
+    if force or _stale(so, _librtz_sources()):
         cmd = [_nvcc(), *NVCC_FLAGS, "-o", str(so), str(CSRC / "rtz_api.cu")]
         if verbose:
             cmd.insert(1, "-Xptxas=-v")
@@ -57,17 +64,17 @@ def build_host(force: bool = False) -> Path:
     so = HOST / "librtz_host.so"
     if not (HOST / "rtz_host_c.cpp").exists():
         return so
-    srcs = sorted(HOST.glob("*.cpp")) + sorted(HOST.glob("*.hpp")) + [ROOT / "include" / "rtz.h"]
+    srcs = _host_sources()
     cxx = os.environ.get("CXX", "g++")
     common = ["-O2", "-std=c++17", "-fPIC", "-ffp-contract=off", "-Wall", "-Wextra", f"-I{ROOT / 'include'}"]
     rpath = ["-Wl,-rpath,$ORIGIN/../csrc", f"-L{CSRC}", "-lrtz"]
-    if force or _stale(so, srcs + [CSRC / "librtz.so"]):
+    if force or _stale(so, srcs):
         r = subprocess.run([cxx, *common, "-shared", "-o", str(so), str(HOST / "rtz_host_c.cpp"), *rpath],
                            capture_output=True, text=True)
         if r.returncode != 0:
             raise RuntimeError("host library build failed:\n" + r.stdout + r.stderr)
     exe = HOST / "rtz_main"
-    if force or _stale(exe, srcs + [CSRC / "librtz.so"]):
+    if force or _stale(exe, srcs):
         r = subprocess.run([cxx, *common, "-o", str(exe), str(HOST / "main.cpp"), *rpath], capture_output=True, text=True)
         if r.returncode != 0:
             raise RuntimeError("rtz_main build failed:\n" + r.stdout + r.stderr)
@@ -75,8 +82,13 @@ def build_host(force: bool = False) -> Path:
 
 
 def build_all(force: bool = False, verbose: bool = False) -> None:
-    """Build everything; serialised with a file lock so that N torchrun ranks can all call it."""
+    """Build everything; serialised with a file lock so that N torchrun ranks can all call it.  Writes nothing
+    when every product is up to date, so a built tree may be read-only."""
     import fcntl
+    if not force and not any(_stale(t, s) for t, s in ((CSRC / "librtz.so", _librtz_sources()),
+                                                        (HOST / "librtz_host.so", _host_sources()),
+                                                        (HOST / "rtz_main", _host_sources()))):
+        return
     with open(PKG / ".build.lock", "w") as lock:
         fcntl.flock(lock, fcntl.LOCK_EX)
         try:

@@ -133,11 +133,17 @@ _oracle = None
 def build_oracle(force: bool = False) -> Path:
     so = ORACLE_DIR / "liboracle.so"
     srcs = list(ORACLE_DIR.glob("*.cpp")) + list(ORACLE_DIR.glob("*.h")) + [ROOT / "include" / "rtz.h"]
+
+    def stale():
+        return force or not so.exists() or any(s.stat().st_mtime > so.stat().st_mtime for s in srcs)
+
+    if not stale():   # nothing to write: a built tree may be read-only
+        return so
     import fcntl
     with open(ORACLE_DIR / ".build.lock", "w") as lock:   # N ranks / xdist workers may race here
         fcntl.flock(lock, fcntl.LOCK_EX)
         try:
-            if force or not so.exists() or any(s.stat().st_mtime > so.stat().st_mtime for s in srcs):
+            if stale():
                 subprocess.run(["make", "-C", str(ORACLE_DIR), "-B", "liboracle.so"], check=True, capture_output=True)
         finally:
             fcntl.flock(lock, fcntl.LOCK_UN)
