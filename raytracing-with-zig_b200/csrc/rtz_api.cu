@@ -104,6 +104,10 @@ struct rtz_context {
     DevBuf<float> wexp;  // w of the pair layout as a plain row
     DevBuf<rtz::DSphere> dspheres;
     std::vector<float4> h_pairs;
+    // padded boxes of the 32-sphere blocks (TraceParamsConst::boxes) and whether the constant-bank kernel culls with them
+    std::vector<float4> h_boxes;
+    float cull_r2 = 0.0f;
+    bool cull = false;
     // RTZ_MODE_PATH_BVH (extension): hierarchy over the same FP32 spheres, built on the first render that
     // asks for it (h_geom / h_w are the host copies it is built from)
     DevBuf<rtz::BvhNode> bvh_nodes;
@@ -323,7 +327,11 @@ int32_t enqueue_path(rtz_context* ctx, const rtz_camera* cam, const rtz::ShardGe
         else if (ctx->n_pad <= 64)
             // lockstep kernel on a shading-bound scene: warps, not registers (<128,8>: 64 registers, 32 warps per SM)
             rc = launch_trace(ctx, rtz::trace_kernel_const<128, 8>, C, P.n_chunks, 128, 0);
-        else
+        else if (ctx->cull) {
+            std::memcpy(C.boxes, ctx->h_boxes.data(), ctx->h_boxes.size() * sizeof(float4));
+            C.cull_r2 = ctx->cull_r2;
+            rc = launch_trace(ctx, rtz::trace_kernel_const_cull<128, 6>, C, P.n_chunks, 128, 0);
+        } else
             rc = launch_trace(ctx, rtz::trace_kernel_const<128, 6>, C, P.n_chunks, 128, 0);
     } else if (use_global) {
         rc = launch_trace(ctx, rtz::trace_kernel_global<128, 5>, P, P.n_chunks, 128, 0);
@@ -653,6 +661,44 @@ int32_t rtz_scene_upload(rtz_context* c, const rtz_sphere* sp, uint64_t n) {
         pr[2 * p] = make_float4(A.x, B.x, A.y, B.y);
         pr[2 * p + 1] = make_float4(A.z, B.z, w[2 * p], w[2 * p + 1]);
     }
+    // Bounds of the sweep's 32-sphere blocks for the culled constant-bank kernel (box_reach in rtz_kernels.cuh states
+    // the exactness contract these paddings serve).  R covers every ray origin within twice the farthest point of
+    // a sphere outside block 0; block 0 (the ground of the book's scenes) has no box: it is always swept.
+    const int n_blocks = (n_pad + 31) / 32;
+    std::vector<float4> bx(2 * (size_t)std::max(n_blocks, 1), make_float4(0.f, 0.f, 0.f, 0.f));
+    double reach = 0.0;
+    for (uint64_t i = 32; i < n; ++i) {
+        const float4 s = g[i];
+        reach = std::max(reach, std::sqrt((double)s.x * s.x + (double)s.y * s.y + (double)s.z * s.z) + std::sqrt(-(double)s.w));
+    }
+    const double R = 2.0 * reach;
+    double lo_all[3] = {INFINITY, INFINITY, INFINITY}, hi_all[3] = {-INFINITY, -INFINITY, -INFINITY}, vol_sum = 0.0;
+    std::vector<double> vols;
+    for (int b = 1; b < n_blocks; ++b) {
+        double lo[3] = {INFINITY, INFINITY, INFINITY}, hi[3] = {-INFINITY, -INFINITY, -INFINITY};
+        for (uint64_t i = 32ull * b; i < std::min<uint64_t>(n, 32ull * b + 32); ++i) {
+            const float4 s = g[i];
+            const double c[3] = {s.x, s.y, s.z}, r = std::sqrt(-(double)s.w);
+            const double cn = std::sqrt(c[0] * c[0] + c[1] * c[1] + c[2] * c[2]);
+            const double pad = 1e-4 * (1.0 + r + std::fabs(c[0]) + std::fabs(c[1]) + std::fabs(c[2])) +
+                               1e-6 * (1.001 * R + cn) * (1.001 * R + cn) / r;
+            for (int a = 0; a < 3; ++a) lo[a] = std::min(lo[a], c[a] - r - pad), hi[a] = std::max(hi[a], c[a] + r + pad);
+        }
+        float fl[3], fh[3];  // rounded outwards
+        for (int a = 0; a < 3; ++a) {
+            fl[a] = std::nextafter((float)lo[a], -INFINITY), fh[a] = std::nextafter((float)hi[a], INFINITY);
+            lo_all[a] = std::min(lo_all[a], lo[a]), hi_all[a] = std::max(hi_all[a], hi[a]);
+        }
+        bx[2 * b] = make_float4(fl[0], fh[0], fl[1], fh[1]);
+        bx[2 * b + 1] = make_float4(fl[2], fh[2], 0.f, 0.f);
+        vols.push_back((hi[0] - lo[0]) * (hi[1] - lo[1]) * (hi[2] - lo[2]));
+    }
+    // Culling pays where the blocks are small against the region they share (the book's scenes: strips of the ground
+    // grid, about 1 % of it each); where every block spans the scene, as in a uniform cloud of spheres, the box tests
+    // would be pure overhead, so the plain sweep runs.
+    for (double v : vols) vol_sum += v;
+    const double vol_all = (hi_all[0] - lo_all[0]) * (hi_all[1] - lo_all[1]) * (hi_all[2] - lo_all[2]);
+    const bool cull = !vols.empty() && std::isfinite(R) && vol_sum < 0.25 * vols.size() * vol_all;
     // Not failure-atomic by itself (growing a buffer frees the old one), so the context holds NO scene from here
     // until every copy has been enqueued: a failed upload leaves an empty world behind, never stale geometry.
     c->n_spheres = c->n_pad = 0;
@@ -675,6 +721,9 @@ int32_t rtz_scene_upload(rtz_context* c, const rtz_sphere* sp, uint64_t n) {
     RTZ_CUDA(cudaMemcpyAsync(c->dspheres.p, ds.data(), ds.size() * sizeof(rtz::DSphere), cudaMemcpyHostToDevice,
                              c->stream));
     c->h_pairs.swap(pr);  // host copy: small scenes travel to the kernel as a __grid_constant__ parameter
+    c->h_boxes.swap(bx);
+    c->cull_r2 = (float)(R * R);
+    c->cull = cull;
     g.resize(n), w.resize(n);
     c->h_geom.swap(g), c->h_w.swap(w);  // what the BVH extension is built from, if it is ever asked for
     c->n_spheres = (int)n, c->n_pad = n_pad;

@@ -57,6 +57,11 @@ constexpr int kMaxConstSpheres = 512;  // 8 KiB: what the constant cache serves 
 struct TraceParamsConst {
     TraceParams p;
     float4 pairs[kMaxConstSpheres];
+    // trace_kernel_const<.., true> only: the padded box of every 32-sphere block of the sweep,
+    // [2b] = {lo.x, hi.x, lo.y, hi.y}, [2b+1] = {lo.z, hi.z, 0, 0} (block 0 is always swept), and the squared
+    // distance from the world origin beyond which a ray origin was not accounted for in the padding
+    float4 boxes[2 * (kMaxConstSpheres / 32)];
+    float cull_r2;
 };
 
 // local (compact, padded) pixel index -> global pixel; false for tile padding
@@ -180,6 +185,29 @@ __device__ __forceinline__ void test_pair(const float4 p0, const float4 p1, cons
     mask = __funnelshift_l(__float_as_uint(disc.y), mask, 1);  // ... then sphere 2p+1
 }
 
+// Can the segment (0, closest] of a path reach the padded box of a block?  Slab test; `ix, iy, iz` = 1 / d.
+//
+// Exactness contract of the block cull: a lane may report "no" only if the FP32 pipeline (sign of the expanded
+// discriminant, then the direct-form root in (t_min * |d|, closest)) would accept no sphere of the block.
+//  * An accepted root lies inside the padded box.  Both discriminant gates must pass, and each is off by at most
+//    about 12 eps |c - o|^2 (eps = 2^-24), so an accepted point p = o + t d — a self hit, o + 2 h d, included — has
+//    |p - c|^2 <= r^2 + 24 eps |c - o|^2: |p - c| <= r + 12 eps |c - o|^2 / r.  The host pads every sphere by
+//    1e-6 (R + |c|)^2 / r for |o| <= R (1e-6 > 16 eps) on top of the BVH builder's 1e-4 (1 + r + |c|_1); a ray
+//    starting farther out than R (|o|^2 > cull_r2) needs every block.
+//  * The test itself errs towards "yes": the interval is [0, closest], a superset of (t_min |d|, closest), and
+//    compared with <=, never strictly; an accepted point sits at least the padding inside every face, far beyond
+//    the few ulps of (lo - o) * (1 / d); fminf / fmaxf drop the NaN of 0 * inf (an axis-parallel ray in the plane
+//    of a face), which is then outside the box by the padding; an origin inside the box gives t_near = 0 <= t_far.
+__device__ __forceinline__ bool box_reach(const float4 b0, const float4 b1, const Path& p, float ix, float iy, float iz,
+                                          float closest) {
+    const float2 tx = __fmul2_rn(__fadd2_rn(make_float2(b0.x, b0.y), make_float2(-p.ox, -p.ox)), make_float2(ix, ix));
+    const float2 ty = __fmul2_rn(__fadd2_rn(make_float2(b0.z, b0.w), make_float2(-p.oy, -p.oy)), make_float2(iy, iy));
+    const float2 tz = __fmul2_rn(__fadd2_rn(make_float2(b1.x, b1.y), make_float2(-p.oz, -p.oz)), make_float2(iz, iz));
+    const float tn = fmaxf(fmaxf(fminf(tx.x, tx.y), fminf(ty.x, ty.y)), fmaxf(fminf(tz.x, tz.y), 0.0f));
+    const float tf = fminf(fminf(fmaxf(tx.x, tx.y), fmaxf(ty.x, ty.y)), fminf(fmaxf(tz.x, tz.y), closest));
+    return tn <= tf;
+}
+
 // HittableList.hit for the two paths of a thread.  `pairs` is warp-uniform storage (shared memory
 // or the constant bank): per sphere pair 2 LDS.128 + 2 x (7 FFMA2 + 1 FADD2 + 2 SHF) for FOUR tests.
 // n_pad is a multiple of 8; padding spheres have w = -inf -> disc = -inf -> never a candidate.
@@ -188,17 +216,36 @@ __device__ __forceinline__ void test_pair(const float4 p0, const float4 p1, cons
 // (Deferring the candidates of several blocks to per-lane lists and resolving them together was built twice and
 // measured on one box: +3.7 % warp-instructions, +0.4 % time.  The 64 paths of a warp come from one pixel, so
 // their candidates coincide and one pass per non-empty block already serves all lanes.)
-template <bool kConstBank, bool kSkipSelf = false>
+// kCull (constant-bank lockstep kernel): a block of 32 spheres that no path of the warp can reach over (0, closest]
+// is skipped as a whole — a warp-uniform branch, so the loop stays on the uniform datapath.  Block 0 (the ground of
+// the book's scenes) is always swept first, which gives most paths a short closest hit before the bounds are tested.
+template <bool kConstBank, bool kSkipSelf = false, bool kCull = false>
 __device__ __forceinline__ void sweep2(const float4* __restrict__ pairs, const float4* __restrict__ gather, int n_pad,
                                        float tmin, float tmax, const Path& a, const Path& b, float& ta, int& ia,
-                                       float& tb, int& ib) {
+                                       float& tb, int& ib, const float4* __restrict__ boxes = nullptr,
+                                       float cull_r2 = 0.0f) {
     RayK ka = ray_constants(a), kb = ray_constants(b);
-    // pin 2*o in registers: left alone, ptxas keeps o and re-adds it for every block of 32 spheres
-    if (kConstBank) asm volatile("" : "+f"(ka.tx), "+f"(ka.ty), "+f"(ka.tz), "+f"(kb.tx), "+f"(kb.ty), "+f"(kb.tz));
+    // pin 2*o in registers: left alone, ptxas keeps o and re-adds it for every block of 32 spheres (not in the culled
+    // sweep: its six reciprocals need those registers, and with the pin it spills under the 80-register cap)
+    if (kConstBank && !kCull) asm volatile("" : "+f"(ka.tx), "+f"(ka.ty), "+f"(ka.tz), "+f"(kb.tx), "+f"(kb.ty), "+f"(kb.tz));
     // Interval(t_min, t_max) of Scene.interval in distance units (directions are unit length)
     float ca = tmax * a.len, cb = tmax * b.len;
     int ba = -1, bb = -1;
+    float iax = 0.f, iay = 0.f, iaz = 0.f, ibx = 0.f, iby = 0.f, ibz = 0.f;
+    if (kCull) {
+        // an origin the padding does not cover (|o|^2 > cull_r2) gets NaN reciprocals: box_reach then sees the whole
+        // segment [0, closest] and the path needs every block (no predicate register held across the sweep)
+        iax = 1.0f / a.dx, iay = 1.0f / a.dy, iaz = 1.0f / a.dz;
+        ibx = 1.0f / b.dx, iby = 1.0f / b.dy, ibz = 1.0f / b.dz;
+        if (!(-ka.nk2 <= cull_r2)) iax = iay = iaz = __int_as_float(0x7fffffff);
+        if (!(-kb.nk2 <= cull_r2)) ibx = iby = ibz = __int_as_float(0x7fffffff);
+    }
     for (int base = 0; base < n_pad; base += 32) {
+        if (kCull && base > 0) {
+            const float4 b0 = boxes[base >> 4], b1 = boxes[(base >> 4) + 1];
+            const bool need = box_reach(b0, b1, a, iax, iay, iaz, ca) | box_reach(b0, b1, b, ibx, iby, ibz, cb);
+            if (!__any_sync(0xFFFFFFFFu, need)) continue;
+        }
         const int cnt = min(32, n_pad - base);
         unsigned ma = 0xFFFFFFFFu, mb = 0xFFFFFFFFu;  // 1 = miss
         const float4* g = pairs + base;
@@ -358,9 +405,10 @@ __device__ __forceinline__ void take_camera_ray(const float* stage, uint32_t j, 
 }
 constexpr int kStageFloats = 7 * 64;  // per warp: 7 rows (origin, unit direction, |direction|) of 64 rays (two slots per lane)
 
-template <bool kConstBank, int kBlock>
+template <bool kConstBank, int kBlock, bool kCull = false>
 __device__ __forceinline__ void trace_body(const TraceParams& P, const float4* __restrict__ pairs,
-                                           const float4* __restrict__ gather, float* __restrict__ stage_mem) {
+                                           const float4* __restrict__ gather, float* __restrict__ stage_mem,
+                                           const float4* __restrict__ boxes = nullptr, float cull_r2 = 0.0f) {
     float* const stage = stage_mem + (threadIdx.x >> 5) * kStageFloats;
     unsigned long long* const tl =
         P.timeline ? P.timeline + 4ull * ((unsigned long long)blockIdx.x * (kBlock / 32) + (threadIdx.x >> 5)) : nullptr;
@@ -477,7 +525,8 @@ __device__ __forceinline__ void trace_body(const TraceParams& P, const float4* _
         prev_a = live_a, prev_b = live_b;
         float ta = 0.f, tb = 0.f;
         int ia = -1, ib = -1;
-        sweep2<kConstBank>(pairs, gather, P.n_pad, cam.tmin, cam.tmax, A.path, B.path, ta, ia, tb, ib);
+        sweep2<kConstBank, false, kCull>(pairs, gather, P.n_pad, cam.tmin, cam.tmax, A.path, B.path, ta, ia, tb, ib,
+                                         boxes, cull_r2);
         if (A.alive) finish_or_continue(P, gather, s_aux, s_alb, A, ta, ia);
         if (B.alive) finish_or_continue(P, gather, s_aux, s_alb, B, tb, ib);
         // explicit reconvergence point: with it ptxas proves the loop top converged (no BRA.DIV before
@@ -753,6 +802,14 @@ template <int kBlock, int kMinBlocks>
 __global__ void __launch_bounds__(kBlock, kMinBlocks) trace_kernel_const(const __grid_constant__ TraceParamsConst C) {
     __shared__ float stage[(kBlock / 32) * kStageFloats];
     trace_body<true, kBlock>(C.p, C.pairs, C.p.geom, stage);
+}
+
+// K1a with block culling: the same body, but a block of 32 spheres whose padded box (C.boxes) no path of the warp
+// can reach is skipped.  The host takes it for scenes whose blocks are compact against the scene's extent.
+template <int kBlock, int kMinBlocks>
+__global__ void __launch_bounds__(kBlock, kMinBlocks) trace_kernel_const_cull(const __grid_constant__ TraceParamsConst C) {
+    __shared__ float stage[(kBlock / 32) * kStageFloats];
+    trace_body<true, kBlock, true>(C.p, C.pairs, C.p.geom, stage, C.boxes, C.cull_r2);
 }
 
 // K1b: geometry staged into shared memory by 1-D TMA bulk copies (cp.async.bulk + mbarrier): scenes
