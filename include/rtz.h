@@ -272,6 +272,11 @@ int32_t rtz_probe_scatter(const rtz_sphere* spheres, uint64_t n_spheres, int32_t
                           const double orig[3], const double dir[3], uint64_t seed, uint32_t pixel,
                           uint32_t sample, uint32_t bounce, rtz_scatter* out);
 
+/* The order in which the culled constant-bank sweep visits the spheres (host only, no device needed):
+ * order_out[slot] = index of the sphere in the list, for the n slots.  Sphere 0 stays in slot 0; the others are
+ * regrouped by median splits of their centres into compact blocks of 32 slots. */
+int32_t rtz_probe_sweep_order(const rtz_sphere* spheres, uint64_t n_spheres, int32_t* order_out);
+
 /* Color.toRgb (src/color.zig:63-80) on the device for `n` colours (3 f64 each). */
 int32_t rtz_probe_to_rgb(const double* linear, uint64_t n, uint8_t* rgb_out);
 

@@ -87,6 +87,7 @@ SIGNATURES = {
     "rtz_probe_scatter": (_i32, [C.POINTER(rtz_sphere), _u64, _i32, D3, D3, _u64, _u32, _u32, _u32,
                                  C.POINTER(rtz_scatter)]),
     "rtz_probe_to_rgb": (_i32, [_f64p, _u64, _u8p]),
+    "rtz_probe_sweep_order": (_i32, [C.POINTER(rtz_sphere), _u64, C.POINTER(_i32)]),
     "rtz_probe_uniform": (_i32, [_u64, _u32, _u32, _u32, _u64, _f32p]),
     "rtz_probe_camera_ray": (_i32, [C.POINTER(rtz_camera), _u64, _u64, _u64, _u64, _f32p, _f32p, _f32p]),
     "rtz_strerror": (C.c_char_p, [_i32]),

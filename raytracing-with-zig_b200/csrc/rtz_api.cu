@@ -108,6 +108,12 @@ struct rtz_context {
     std::vector<float4> h_boxes;
     float cull_r2 = 0.0f;
     bool cull = false;
+    // ... and the rows that kernel and its drain read: the spheres regrouped into compact blocks (sweep_order), slot s
+    // holding sphere rg_orig[s] of the caller's list.  Uploaded only for a scene that is culled.
+    DevBuf<float4> rg_geom, rg_aux, rg_albedo;
+    DevBuf<float> rg_wexp;
+    DevBuf<int> rg_orig;
+    std::vector<float4> h_rg_pairs;
     // RTZ_MODE_PATH_BVH (extension): hierarchy over the same FP32 spheres, built on the first render that
     // asks for it (h_geom / h_w are the host copies it is built from)
     DevBuf<rtz::BvhNode> bvh_nodes;
@@ -243,6 +249,7 @@ int32_t enqueue_path(rtz_context* ctx, const rtz_camera* cam, const rtz::ShardGe
     P.cam = to_dev_camera(*cam, seed);
     P.sh = sg;
     P.geom = ctx->geom.p, P.pairs = ctx->pairs.p, P.aux = ctx->aux.p, P.albedo = ctx->albedo.p, P.wexp = ctx->wexp.p;
+    P.orig = nullptr;
     P.n_spheres = ctx->n_spheres, P.n_pad = ctx->n_pad;
     pick_chunks(ctx, P, n_local_pixels);
     P.accum = ctx->accum.p;
@@ -328,6 +335,13 @@ int32_t enqueue_path(rtz_context* ctx, const rtz_camera* cam, const rtz::ShardGe
             // lockstep kernel on a shading-bound scene: warps, not registers (<128,8>: 64 registers, 32 warps per SM)
             rc = launch_trace(ctx, rtz::trace_kernel_const<128, 8>, C, P.n_chunks, 128, 0);
         else if (ctx->cull) {
+            // the culled kernel, and the drain after it, work on the regrouped rows: sphere indices (hits, Path.self,
+            // parked paths) are slots throughout, and only exact ties in t look up the original index.  The device
+            // pair rows have no reader here (the sweep reads C.pairs, the drain the plain rows).
+            P.geom = ctx->rg_geom.p, P.aux = ctx->rg_aux.p, P.albedo = ctx->rg_albedo.p, P.wexp = ctx->rg_wexp.p;
+            P.orig = ctx->rg_orig.p, P.pairs = nullptr;
+            C.p = P;
+            std::memcpy(C.pairs, ctx->h_rg_pairs.data(), (size_t)ctx->n_pad * sizeof(float4));
             std::memcpy(C.boxes, ctx->h_boxes.data(), ctx->h_boxes.size() * sizeof(float4));
             C.cull_r2 = ctx->cull_r2;
             rc = launch_trace(ctx, rtz::trace_kernel_const_cull<128, 6>, C, P.n_chunks, 128, 0);
@@ -549,6 +563,7 @@ int32_t rtz_context_destroy(rtz_context* c) {
     c->geom.release(), c->pairs.release(), c->aux.release(), c->albedo.release(), c->dspheres.release();
     c->accum.release(), c->counters.release(), c->rgb.release(), c->linear.release(), c->timeline.release(), c->pool.release();
     c->bvh_nodes.release(), c->bvh_order.release(), c->wexp.release();
+    c->rg_geom.release(), c->rg_aux.release(), c->rg_albedo.release(), c->rg_wexp.release(), c->rg_orig.release();
     for (auto& e : c->ev)
         if (e) cudaEventDestroy(e);
     if (c->h_counters) cudaFreeHost(c->h_counters);
@@ -558,6 +573,51 @@ int32_t rtz_context_destroy(rtz_context* c) {
 }
 
 namespace {
+// The order in which the culled kernel sweeps the spheres: slot -> index in the caller's list.  Sphere 0 (the
+// ground of the book's scenes) keeps slot 0, since block 0 is always swept first; the others are split
+// recursively at the median of the longest axis of their centres, with every cut on a multiple of 32 slots, so
+// that each 32-sphere block is a compact cluster with a small box.  Equal coordinates are ordered by index and
+// every final block is sorted by index: the order depends on the FP32 centres alone, the same on every device.
+void regroup(const std::vector<float4>& g, std::vector<int>& idx, int first, int cnt, int slot0) {
+    const int blocks = (slot0 + cnt + 31) / 32 - slot0 / 32;
+    if (blocks <= 1) {
+        std::sort(idx.begin() + first, idx.begin() + first + cnt);
+        return;
+    }
+    float lo[3] = {INFINITY, INFINITY, INFINITY}, hi[3] = {-INFINITY, -INFINITY, -INFINITY};
+    for (int q = first; q < first + cnt; ++q) {
+        const float c[3] = {g[idx[q]].x, g[idx[q]].y, g[idx[q]].z};
+        for (int a = 0; a < 3; ++a) lo[a] = std::min(lo[a], c[a]), hi[a] = std::max(hi[a], c[a]);
+    }
+    int axis = 0;
+    for (int a = 1; a < 3; ++a)
+        if (hi[a] - lo[a] > hi[axis] - lo[axis]) axis = a;
+    const int cut_slot = (slot0 / 32 + blocks / 2) * 32;
+    const int left = cut_slot - slot0;
+    auto key = [&](int i) { return axis == 0 ? g[i].x : axis == 1 ? g[i].y : g[i].z; };
+    std::nth_element(idx.begin() + first, idx.begin() + first + left, idx.begin() + first + cnt,
+                     [&](int x, int y) { return key(x) < key(y) || (key(x) == key(y) && x < y); });
+    regroup(g, idx, first, left, slot0);
+    regroup(g, idx, first + left, cnt - left, cut_slot);
+}
+std::vector<int> sweep_order(const std::vector<float4>& g, int n) {
+    std::vector<int> idx(n);
+    for (int i = 0; i < n; ++i) idx[i] = i;
+    if (n > 1) regroup(g, idx, 1, n - 1, 1);
+    return idx;
+}
+
+// sweep layout of the rows g / w: one FFMA2 = one ray x the two spheres of a pair
+std::vector<float4> pair_rows(const std::vector<float4>& g, const std::vector<float>& w, int n_pad) {
+    std::vector<float4> pr(std::max(n_pad, 1));
+    for (int p = 0; p < n_pad / 2; ++p) {
+        const float4 A = g[2 * p], B = g[2 * p + 1];
+        pr[2 * p] = make_float4(A.x, B.x, A.y, B.y);
+        pr[2 * p + 1] = make_float4(A.z, B.z, w[2 * p], w[2 * p + 1]);
+    }
+    return pr;
+}
+
 // Median-split BVH over the FP32 spheres {cx, cy, cz, -r^2} (RTZ_MODE_PATH_BVH).  Boxes are padded well beyond
 // the rounding of the slab test and of the hit point, so the traversal is conservative.
 struct BvhBuilder {
@@ -623,7 +683,7 @@ int32_t rtz_scene_upload(rtz_context* c, const rtz_sphere* sp, uint64_t n) {
     DeviceGuard guard;
     RTZ_CUDA(cudaSetDevice(c->device));
     const int n_pad = (int)((n + 7) & ~7ull);
-    std::vector<float4> g(n_pad ? n_pad : 1), pr(n_pad ? n_pad : 1), a(n_pad ? n_pad : 1), al(n_pad ? n_pad : 1);
+    std::vector<float4> g(n_pad ? n_pad : 1), a(n_pad ? n_pad : 1), al(n_pad ? n_pad : 1);
     std::vector<float> w(n_pad ? n_pad : 1);
     std::vector<rtz::DSphere> ds(n ? n : 1);
     for (uint64_t i = 0; i < n; ++i) {
@@ -656,19 +716,16 @@ int32_t rtz_scene_upload(rtz_context* c, const rtz_sphere* sp, uint64_t n) {
         a[i] = make_float4(0.f, 0.f, 0.f, bits_to_float(0));
         al[i] = make_float4(0.f, 0.f, 0.f, 0.f);
     }
-    for (int p = 0; p < n_pad / 2; ++p) {  // sweep layout: one FFMA2 = one ray x the two spheres of a pair
-        const float4 A = g[2 * p], B = g[2 * p + 1];
-        pr[2 * p] = make_float4(A.x, B.x, A.y, B.y);
-        pr[2 * p + 1] = make_float4(A.z, B.z, w[2 * p], w[2 * p + 1]);
-    }
-    // Bounds of the sweep's 32-sphere blocks for the culled constant-bank kernel (box_reach in rtz_kernels.cuh states
+    std::vector<float4> pr = pair_rows(g, w, n_pad);
+    // Bounds of the culled kernel's 32-sphere blocks, on its regrouped order (box_reach in rtz_kernels.cuh states
     // the exactness contract these paddings serve).  R covers every ray origin within twice the farthest point of
     // a sphere outside block 0; block 0 (the ground of the book's scenes) has no box: it is always swept.
+    const std::vector<int> order = sweep_order(g, (int)n);
     const int n_blocks = (n_pad + 31) / 32;
     std::vector<float4> bx(2 * (size_t)std::max(n_blocks, 1), make_float4(0.f, 0.f, 0.f, 0.f));
     double reach = 0.0;
-    for (uint64_t i = 32; i < n; ++i) {
-        const float4 s = g[i];
+    for (uint64_t q = 32; q < n; ++q) {
+        const float4 s = g[order[q]];
         reach = std::max(reach, std::sqrt((double)s.x * s.x + (double)s.y * s.y + (double)s.z * s.z) + std::sqrt(-(double)s.w));
     }
     const double R = 2.0 * reach;
@@ -676,8 +733,8 @@ int32_t rtz_scene_upload(rtz_context* c, const rtz_sphere* sp, uint64_t n) {
     std::vector<double> vols;
     for (int b = 1; b < n_blocks; ++b) {
         double lo[3] = {INFINITY, INFINITY, INFINITY}, hi[3] = {-INFINITY, -INFINITY, -INFINITY};
-        for (uint64_t i = 32ull * b; i < std::min<uint64_t>(n, 32ull * b + 32); ++i) {
-            const float4 s = g[i];
+        for (uint64_t q = 32ull * b; q < std::min<uint64_t>(n, 32ull * b + 32); ++q) {
+            const float4 s = g[order[q]];
             const double c[3] = {s.x, s.y, s.z}, r = std::sqrt(-(double)s.w);
             const double cn = std::sqrt(c[0] * c[0] + c[1] * c[1] + c[2] * c[2]);
             const double pad = 1e-4 * (1.0 + r + std::fabs(c[0]) + std::fabs(c[1]) + std::fabs(c[2])) +
@@ -693,16 +750,29 @@ int32_t rtz_scene_upload(rtz_context* c, const rtz_sphere* sp, uint64_t n) {
         bx[2 * b + 1] = make_float4(fl[2], fh[2], 0.f, 0.f);
         vols.push_back((hi[0] - lo[0]) * (hi[1] - lo[1]) * (hi[2] - lo[2]));
     }
-    // Culling pays where the blocks are small against the region they share (the book's scenes: strips of the ground
-    // grid, about 1 % of it each); where every block spans the scene, as in a uniform cloud of spheres, the box tests
-    // would be pure overhead, so the plain sweep runs.
+    // Culling pays where the blocks are small against the region they share; where every block spans the scene the
+    // box tests would be pure overhead, so the plain sweep runs.  Regrouped, even a uniform cloud of spheres has
+    // compact blocks (485 in a cube: about 7 % each), and it is faster culled (DESIGN.md §5).
     for (double v : vols) vol_sum += v;
     const double vol_all = (hi_all[0] - lo_all[0]) * (hi_all[1] - lo_all[1]) * (hi_all[2] - lo_all[2]);
-    const bool cull = !vols.empty() && std::isfinite(R) && vol_sum < 0.25 * vols.size() * vol_all;
+    const bool cull = n_pad <= rtz::kMaxConstSpheres && !vols.empty() && std::isfinite(R) &&
+                      vol_sum < 0.25 * vols.size() * vol_all;
+    // the rows of the culled kernel in its order; padding stays in slots n .. n_pad-1
+    std::vector<float4> rg(cull ? n_pad : 0), ra(cull ? n_pad : 0), ral(cull ? n_pad : 0), rpr;
+    std::vector<float> rw(cull ? n_pad : 0);
+    std::vector<int> ro(cull ? n_pad : 0);
+    if (cull) {
+        for (int q = 0; q < n_pad; ++q) {
+            const int i = q < (int)n ? order[q] : q;
+            rg[q] = g[i], ra[q] = a[i], ral[q] = al[i], rw[q] = w[i], ro[q] = i;
+        }
+        rpr = pair_rows(rg, rw, n_pad);
+    }
     // Not failure-atomic by itself (growing a buffer frees the old one), so the context holds NO scene from here
     // until every copy has been enqueued: a failed upload leaves an empty world behind, never stale geometry.
     c->n_spheres = c->n_pad = 0;
-    c->h_pairs.clear(), c->h_geom.clear(), c->h_w.clear();
+    c->h_pairs.clear(), c->h_rg_pairs.clear(), c->h_geom.clear(), c->h_w.clear();
+    c->cull = false;
     c->bvh_ready = false;
     if (n_pad) {
         RTZ_CUDA(c->geom.reserve(n_pad));
@@ -717,10 +787,23 @@ int32_t rtz_scene_upload(rtz_context* c, const rtz_sphere* sp, uint64_t n) {
         RTZ_CUDA(cudaMemcpyAsync(c->aux.p, a.data(), n_pad * sizeof(float4), cudaMemcpyHostToDevice, c->stream));
         RTZ_CUDA(cudaMemcpyAsync(c->albedo.p, al.data(), n_pad * sizeof(float4), cudaMemcpyHostToDevice, c->stream));
     }
+    if (cull) {
+        RTZ_CUDA(c->rg_geom.reserve(n_pad));
+        RTZ_CUDA(c->rg_aux.reserve(n_pad));
+        RTZ_CUDA(c->rg_albedo.reserve(n_pad));
+        RTZ_CUDA(c->rg_wexp.reserve(n_pad));
+        RTZ_CUDA(c->rg_orig.reserve(n_pad));
+        RTZ_CUDA(cudaMemcpyAsync(c->rg_geom.p, rg.data(), n_pad * sizeof(float4), cudaMemcpyHostToDevice, c->stream));
+        RTZ_CUDA(cudaMemcpyAsync(c->rg_aux.p, ra.data(), n_pad * sizeof(float4), cudaMemcpyHostToDevice, c->stream));
+        RTZ_CUDA(cudaMemcpyAsync(c->rg_albedo.p, ral.data(), n_pad * sizeof(float4), cudaMemcpyHostToDevice, c->stream));
+        RTZ_CUDA(cudaMemcpyAsync(c->rg_wexp.p, rw.data(), n_pad * sizeof(float), cudaMemcpyHostToDevice, c->stream));
+        RTZ_CUDA(cudaMemcpyAsync(c->rg_orig.p, ro.data(), n_pad * sizeof(int), cudaMemcpyHostToDevice, c->stream));
+    }
     RTZ_CUDA(c->dspheres.reserve(ds.size()));
     RTZ_CUDA(cudaMemcpyAsync(c->dspheres.p, ds.data(), ds.size() * sizeof(rtz::DSphere), cudaMemcpyHostToDevice,
                              c->stream));
     c->h_pairs.swap(pr);  // host copy: small scenes travel to the kernel as a __grid_constant__ parameter
+    c->h_rg_pairs.swap(rpr);
     c->h_boxes.swap(bx);
     c->cull_r2 = (float)(R * R);
     c->cull = cull;
@@ -1337,6 +1420,19 @@ int32_t rtz_probe_scatter(const rtz_sphere* sp, uint64_t n, int32_t index, const
             out->direction[k] = (double)h.d[k] * (double)h.len;
             out->attenuation[k] = h.att[k];
         }
+    return RTZ_OK;
+}
+
+int32_t rtz_probe_sweep_order(const rtz_sphere* sp, uint64_t n, int32_t* order_out) {
+    if ((!sp || !order_out) && n) return RTZ_ERR_BAD_ARG;
+    if (n > (1u << 20)) return RTZ_ERR_BAD_ARG;
+    std::vector<float4> g(n);
+    for (uint64_t i = 0; i < n; ++i) {
+        if (!finite3(sp[i].center)) return RTZ_ERR_BAD_ARG;
+        g[i] = make_float4((float)sp[i].center[0], (float)sp[i].center[1], (float)sp[i].center[2], 0.f);
+    }
+    const std::vector<int> order = sweep_order(g, (int)n);
+    std::copy(order.begin(), order.end(), order_out);
     return RTZ_OK;
 }
 

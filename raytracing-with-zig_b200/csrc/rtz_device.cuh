@@ -180,14 +180,21 @@ __device__ __forceinline__ void camera_ray(const DevCamera& c, const RngKey& k, 
 // Algorithmic cost per test: 17 FLOP (miss path of src/sphere.zig:27-33, |d|^2 and r^2 hoisted);
 // executed: 7 FFMA + 1 FADD on the expanded form.  The root is only evaluated for candidates.
 // ---------------------------------------------------------------------------------------------
+// Does root t of sphere i replace the running closest hit (closest, best)?  The ascending loop's rule is "strictly
+// nearer", so an exact tie keeps the earlier sphere.  A sweep that visits the spheres in another order (the culled
+// kernel's regrouped blocks) passes `orig`, slot -> index in the caller's list: a tie then goes to the lower
+// original index, which is the sphere the ascending loop keeps.  best < 0 (closest = t_max) never ties.
+__device__ __forceinline__ bool nearer(float t, int i, float closest, int best, const int* __restrict__ orig) {
+    return t < closest || (orig && t == closest && best >= 0 && __ldg(orig + i) < __ldg(orig + best));
+}
 __device__ __forceinline__ void slow_path(float h, float disc, int i, int self, float tmin_d, float& closest,
-                                          int& best) {
+                                          int& best, const int* __restrict__ orig = nullptr) {
     if (i == self) disc = h * h;  // exact c = 0 for the sphere we stand on
     const float sq = sqrtf(disc);
     float t = h - sq;  // (h - sqrtd)/a with a = 1
-    if (!(t > tmin_d && t < closest)) {  // Interval.surrounds is strict (src/interval.zig:36-38)
+    if (!(t > tmin_d && nearer(t, i, closest, best, orig))) {  // Interval.surrounds is strict (src/interval.zig:36-38)
         t = h + sq;
-        if (!(t > tmin_d && t < closest)) return;
+        if (!(t > tmin_d && nearer(t, i, closest, best, orig))) return;
     }
     closest = t;  // shrinking t_max; ties keep the earlier sphere
     best = i;
@@ -214,12 +221,12 @@ __device__ __forceinline__ float expanded_disc(float cx, float cy, float cz, flo
 }
 // root of a candidate from the direct form (src/sphere.zig:27-42); g = {cx, cy, cz, -r^2}
 __device__ __forceinline__ void candidate_root(const float4 g, float nr2, int i, const Path& p, float tmin_d,
-                                               float& closest, int& best) {
+                                               float& closest, int& best, const int* __restrict__ orig = nullptr) {
     const float ocx = g.x - p.ox, ocy = g.y - p.oy, ocz = g.z - p.oz;
     const float h = fmaf(p.dz, ocz, fmaf(p.dy, ocy, p.dx * ocx));
     const float c = fmaf(ocz, ocz, fmaf(ocy, ocy, fmaf(ocx, ocx, nr2)));
     const float disc = fmaf(h, h, -c);
-    if (disc >= 0.0f) slow_path(h, disc, i, p.self, tmin_d, closest, best);
+    if (disc >= 0.0f) slow_path(h, disc, i, p.self, tmin_d, closest, best, orig);
 }
 
 // scalar sweep over plain rows {cx, cy, cz, -r^2} + the pair layout's w: serves the one-ray probes;

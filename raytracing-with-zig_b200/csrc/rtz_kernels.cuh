@@ -25,6 +25,10 @@ struct TraceParams {
     const float4* aux;      // [n_pad] {r, 1/r, fuzz|ior, type}
     const float4* albedo;   // [n_pad] {r,g,b,1/ior}
     const float* wexp;      // [n_pad] w of the pair layout as a plain row (per-lane lookups: coop_hit, the BVH extension)
+    // The culled kernel and its drain sweep the spheres regrouped into compact blocks (rtz_scene_upload): the rows
+    // above then hold that order, and orig[slot] is the sphere's index in the caller's list, which breaks exact ties
+    // in t.  Null for every other kernel: slot = index.
+    const int* orig;
     int n_spheres;
     int n_pad;              // n rounded up to a multiple of 8 (padding spheres can never be hit)
     // Work chunks = runs of `chunk` samples of ONE pixel (a warp's 64 paths then share their camera geometry: warps
@@ -154,13 +158,14 @@ struct Slot {
 // (src/sphere.zig:35-42) with the shrinking t_max of HittableList.hit (src/hittable.zig:66-73).
 // `gather[i]` = {cx, cy, cz, -r^2} serves the per-lane (divergent) lookups.
 __device__ __forceinline__ void resolve_candidates(const float4* __restrict__ gather, unsigned cand, int base, int cnt,
-                                                   const Path& p, float tmin_d, float& closest, int& best) {
+                                                   const Path& p, float tmin_d, float& closest, int& best,
+                                                   const int* __restrict__ orig = nullptr) {
     while (cand) {
         const int bit = 31 - __clz(cand);  // highest bit = lowest sphere index: ascending order
         cand &= ~(1u << bit);
         const int i = base + (cnt - 1 - bit);
         const float4 g = gather[i];
-        candidate_root(g, g.w, i, p, tmin_d, closest, best);
+        candidate_root(g, g.w, i, p, tmin_d, closest, best, orig);
     }
 }
 
@@ -223,7 +228,7 @@ template <bool kConstBank, bool kSkipSelf = false, bool kCull = false>
 __device__ __forceinline__ void sweep2(const float4* __restrict__ pairs, const float4* __restrict__ gather, int n_pad,
                                        float tmin, float tmax, const Path& a, const Path& b, float& ta, int& ia,
                                        float& tb, int& ib, const float4* __restrict__ boxes = nullptr,
-                                       float cull_r2 = 0.0f) {
+                                       float cull_r2 = 0.0f, const int* __restrict__ orig = nullptr) {
     RayK ka = ray_constants(a), kb = ray_constants(b);
     // pin 2*o in registers: left alone, ptxas keeps o and re-adds it for every block of 32 spheres (not in the culled
     // sweep: its six reciprocals need those registers, and with the pin it spills under the 80-register cap)
@@ -269,8 +274,8 @@ __device__ __forceinline__ void sweep2(const float4* __restrict__ pairs, const f
             // registers across the whole sweep of the shared-memory kernel (96 registers at 5 CTAs per SM)
             float la = a.len, lb = b.len;
             if (!kConstBank) asm volatile("" : "+f"(la), "+f"(lb));
-            resolve_candidates(gather, canda, base, cnt, a, tmin * la, ca, ba);
-            resolve_candidates(gather, candb, base, cnt, b, tmin * lb, cb, bb);
+            resolve_candidates(gather, canda, base, cnt, a, tmin * la, ca, ba, orig);
+            resolve_candidates(gather, candb, base, cnt, b, tmin * lb, cb, bb, orig);
         }
     }
     ta = ca, ia = ba, tb = cb, ib = bb;
@@ -333,10 +338,11 @@ __device__ __forceinline__ unsigned long long globaltimer_ns() {
 // spheres with 64 slots for them, 6.5 us per bounce on an empty SM (measured with RTZ_TIMELINE: the last 1 % of
 // the warps used to finish 0.4 ms after the other 99 %).  The discriminants of 8 spheres per lane are evaluated
 // back to back so that their loads overlap (the rows are cold in L1: the sweep reads the constant bank).
+// `orig` (null = identity): the rows are in another order than the caller's list; ties go by original index.
 template <bool kUniform = false>  // kUniform: every lane already holds the path and wants the result
-__device__ __forceinline__ void coop_hit(const float4* __restrict__ geom, const float* __restrict__ wexp, int n,
-                                         float tmin, float tmax, const Path& mine, int src, unsigned lane, float& t_out,
-                                         int& best_out) {
+__device__ __forceinline__ void coop_hit(const float4* __restrict__ geom, const float* __restrict__ wexp,
+                                         const int* __restrict__ orig, int n, float tmin, float tmax, const Path& mine,
+                                         int src, unsigned lane, float& t_out, int& best_out) {
     Path q = mine;
     if (!kUniform) {
         q.ox = __shfl_sync(0xFFFFFFFFu, mine.ox, src), q.oy = __shfl_sync(0xFFFFFFFFu, mine.oy, src);
@@ -364,14 +370,16 @@ __device__ __forceinline__ void coop_hit(const float4* __restrict__ geom, const 
             cand &= cand - 1u;
             const int i = base + 32 * j;
             const float4 g = __ldg(geom + i);
-            candidate_root(g, g.w, i, q, tmin_d, closest, best);
+            candidate_root(g, g.w, i, q, tmin_d, closest, best, orig);
         }
     }
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) {
         const float t2 = __shfl_xor_sync(0xFFFFFFFFu, closest, o);
         const int b2 = __shfl_xor_sync(0xFFFFFFFFu, best, o);
-        if (t2 < closest || (t2 == closest && (unsigned)b2 < (unsigned)best)) closest = t2, best = b2;  // -1 = none
+        // on equal t the lower (original) index wins; -1 = none loses
+        const bool tie_won = t2 == closest && b2 >= 0 && (best < 0 || (orig ? __ldg(orig + b2) < __ldg(orig + best) : b2 < best));
+        if (t2 < closest || tie_won) closest = t2, best = b2;
     }
     if (kUniform || (int)lane == src) t_out = closest, best_out = best;
 }
@@ -526,7 +534,7 @@ __device__ __forceinline__ void trace_body(const TraceParams& P, const float4* _
         float ta = 0.f, tb = 0.f;
         int ia = -1, ib = -1;
         sweep2<kConstBank, false, kCull>(pairs, gather, P.n_pad, cam.tmin, cam.tmax, A.path, B.path, ta, ia, tb, ib,
-                                         boxes, cull_r2);
+                                         boxes, cull_r2, kCull ? P.orig : nullptr);
         if (A.alive) finish_or_continue(P, gather, s_aux, s_alb, A, ta, ia);
         if (B.alive) finish_or_continue(P, gather, s_aux, s_alb, B, tb, ib);
         // explicit reconvergence point: with it ptxas proves the loop top converged (no BRA.DIV before
@@ -1454,7 +1462,7 @@ __global__ void __launch_bounds__(128) drain_kernel(const __grid_constant__ Trac
         int best = -1;
         if (kWarp) {
             for (unsigned m = live; m; m &= m - 1u)
-                coop_hit<false>(P.geom, P.wexp, P.n_spheres, cam.tmin, cam.tmax, s.path, __ffs(m) - 1, lane, t, best);
+                coop_hit<false>(P.geom, P.wexp, P.orig, P.n_spheres, cam.tmin, cam.tmax, s.path, __ffs(m) - 1, lane, t, best);
         } else if (s.alive) {
             sweep_rows(P.geom, P.pairs, 0, P.n_spheres, s.path, cam.tmin, cam.tmax, t, best);
         }

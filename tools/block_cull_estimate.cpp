@@ -5,8 +5,9 @@
 // A-slots refilled before B-slots in lane order, one sweep per iteration, blocks of 32 spheres in order, each
 // path's running closest hit updated after every block) and reports the fraction of sphere tests a warp still
 // executes when it skips every block whose padded bound none of its live paths can reach over (0, closest].
-// Two block orders (the reference's, and a spatial regrouping by median splits) times two bounds (axis-aligned
-// boxes, bounding spheres).
+// Three block orders (the reference's; the spatial regrouping the culled kernel sweeps, sweep_order in
+// csrc/rtz_api.cu; the same blocks swept near to far from the camera) times two bounds (axis-aligned boxes,
+// bounding spheres).
 //
 // Build and run (a few seconds per 100 pixels on one core):
 //   g++ -O2 -std=c++17 -ffp-contract=off -mfma -pthread -o /tmp/bce tools/block_cull_estimate.cpp oracle/rtz_oracle.cpp
@@ -108,11 +109,15 @@ std::vector<Bound> make_bounds(const std::vector<MSphere>& ms, const std::vector
     return out;
 }
 
-// median splits along the longest axis of the centres, cut at multiples of 32 (offset by the ground in slot 0)
+// median splits along the longest axis of the centres, cut at multiples of 32 (offset by the ground in slot 0),
+// final blocks sorted by index: the product's regroup() in csrc/rtz_api.cu
 void kd_order(const std::vector<MSphere>& ms, std::vector<int>& idx, int first, int cnt, int slot0) {
     const int end_slot = slot0 + cnt;
     const int blocks = (end_slot + 31) / 32 - slot0 / 32;
-    if (blocks <= 1) return;
+    if (blocks <= 1) {
+        std::sort(idx.begin() + first, idx.begin() + first + cnt);
+        return;
+    }
     float lo[3] = {INFINITY, INFINITY, INFINITY}, hi[3] = {-INFINITY, -INFINITY, -INFINITY};
     for (int q = first; q < first + cnt; ++q) {
         const MSphere& s = ms[idx[q]];
@@ -136,8 +141,10 @@ struct Result {
 };
 
 // one warp runs all chunks in sequence (each chunk = the samples of one pixel)
+// `seq`: the order in which the blocks are swept (block 0 first)
 Result replay(const std::vector<std::vector<std::vector<Seg>>>& chunks, const std::vector<MSphere>& ms,
-              const std::vector<int>& order, int n_pad, const std::vector<Bound>& bounds, int kind, float tmin) {
+              const std::vector<int>& order, int n_pad, const std::vector<Bound>& bounds, const std::vector<int>& seq,
+              int kind, float tmin) {
     const int nb = (int)bounds.size();
     struct SlotState {
         int chunk = -1, sample = 0, seg = 0;
@@ -170,7 +177,7 @@ Result replay(const std::vector<std::vector<std::vector<Seg>>>& chunks, const st
                 if (t < rb[s][q / 32]) rb[s][q / 32] = t;
             }
         }
-        for (int b = 0; b < nb; ++b) {
+        for (int b : seq) {
             const int cnt = std::min(32, n_pad - 32 * b);
             R.total += cnt;
             bool need = bounds[b].all;
@@ -273,18 +280,29 @@ int main(int argc, char** argv) {
     std::vector<int> ref(n), kd(n);
     for (int i = 0; i < n; ++i) ref[i] = kd[i] = i;
     kd_order(ms, kd, 1, n - 1, 1);  // the ground stays in slot 0
-    const char* order_name[2] = {"reference order", "spatial regrouping"};
+    const char* order_name[3] = {"reference order", "spatial regrouping", "regrouped, near first"};
     const char* bound_name[2] = {"boxes", "spheres"};
-    std::printf("%-20s %-8s %10s %12s\n", "block order", "bound", "executed", "bound tests");
-    for (int o = 0; o < 2; ++o) {
+    std::printf("%-22s %-8s %10s %12s\n", "block order", "bound", "executed", "bound tests");
+    for (int o = 0; o < 3; ++o) {
         const std::vector<int>& order = o == 0 ? ref : kd;
         const auto bounds = make_bounds(ms, order, n_pad);
+        std::vector<int> seq(bounds.size());
+        for (int b = 0; b < (int)seq.size(); ++b) seq[b] = b;
+        if (o == 2) {  // blocks 1.. by the distance from the camera to the centre of their box
+            auto dist = [&](int b) {
+                const Bound& B = bounds[b];
+                double d2 = 0.0;
+                for (int a = 0; a < 3; ++a) d2 += std::pow(0.5 * (B.lo[a] + B.hi[a]) - from[a], 2);
+                return d2;
+            };
+            std::stable_sort(seq.begin() + 1, seq.end(), [&](int x, int y) { return dist(x) < dist(y); });
+        }
         for (int kind = 0; kind < 2; ++kind) {
-            const Result R = replay(chunks, ms, order, n_pad, bounds, kind, c.tmin);
+            const Result R = replay(chunks, ms, order, n_pad, bounds, seq, kind, c.tmin);
             const double frac = R.executed / R.total;
             // bound tests per path and iteration, in units of the sweep's n_pad tests per path and iteration
             const double bt = R.bound_tests / R.iters / n_pad;
-            std::printf("%-20s %-8s %9.1f%% %12.3f", order_name[o], bound_name[kind], 100.0 * frac, R.bound_tests / R.iters);
+            std::printf("%-22s %-8s %9.1f%% %12.3f", order_name[o], bound_name[kind], 100.0 * frac, R.bound_tests / R.iters);
             // predicted step time relative to today: the sweep is 87.7 % of the kernel's warp-instructions
             for (double cb : {1.0, 1.5, 3.0}) {
                 const double rel = (1.0 - 0.877) + 0.877 * (frac + cb * bt);
