@@ -272,6 +272,47 @@ int32_t rtz_probe_scatter(const rtz_sphere* spheres, uint64_t n_spheres, int32_t
                           const double orig[3], const double dir[3], uint64_t seed, uint32_t pixel,
                           uint32_t sample, uint32_t bounce, rtz_scatter* out);
 
+/* Batched probes: m records in one launch, one device thread each, through the per-ray device code of the
+ * render kernels.  Inputs and outputs are f32, as the device holds them, so a CPU restatement can be compared
+ * bit for bit.  The one-ray probes above are calls into these. */
+typedef struct rtz_probe_ray {
+    float orig[3];
+    float dir[3];          /* any length: normalised as the kernels normalise a scattered direction    */
+    int32_t self;          /* sphere the origin lies on (exact c = 0 for it), -1 for none              */
+} rtz_probe_ray;
+
+typedef struct rtz_ray_hit {
+    int32_t best;          /* index of the sphere hit, -1 = miss                                      */
+    int32_t front;         /* HitRecord.front                                                          */
+    float t;               /* closest hit in DISTANCE units (t_max * len on a miss)                   */
+    float len;             /* |dir|: t / len is the reference's t                                     */
+    float point[3];
+    float normal[3];       /* unit, against the ray                                                   */
+} rtz_ray_hit;
+
+/* HittableList.hit(ray, Interval(t_min, t_max)) for m rays (set_direction, then the sweep's gate and root). */
+int32_t rtz_probe_hits(const rtz_sphere* spheres, uint64_t n_spheres, const rtz_probe_ray* rays, uint64_t m,
+                       double t_min, double t_max, rtz_ray_hit* out);
+
+typedef struct rtz_probe_bounce {
+    int32_t sphere;        /* the sphere the ray hits; t_min = 0.001, t_max = +inf, no self            */
+    float orig[3];
+    float dir[3];
+    uint32_t pixel, sample, bounce;  /* the counter-based RNG stream of the scatter                    */
+} rtz_probe_bounce;
+
+typedef struct rtz_ray_scatter {
+    int32_t term;          /* -1 scattered, 1 absorbed, -2 the ray misses the sphere                  */
+    float orig[3];         /* the scattered ray (term == -1)                                           */
+    float dir[3];          /* unit                                                                     */
+    float len;             /* length of the direction before normalisation                             */
+    float attenuation[3];
+} rtz_ray_scatter;
+
+/* Sphere.hit then Material.scatter (the kernels' shade) for m records, RNG keyed by `seed`. */
+int32_t rtz_probe_scatters(const rtz_sphere* spheres, uint64_t n_spheres, const rtz_probe_bounce* recs, uint64_t m,
+                           uint64_t seed, rtz_ray_scatter* out);
+
 /* The order in which the culled constant-bank sweep visits the spheres (host only, no device needed):
  * order_out[slot] = index of the sphere in the list, for the n slots.  Sphere 0 stays in slot 0; the others are
  * regrouped by median splits of their centres into compact blocks of 32 slots. */

@@ -131,6 +131,29 @@ inline void cameraRay(const MCamera& c, const Rng& g, uint32_t i, uint32_t j, Pa
     p.bounce = 0;
 }
 
+// The candidate gate's margin (the device's kGateSlack, DESIGN.md §4): the gate tests
+// disc + 64 eps (|o|^2 + |c|^2) >= 0, the per-ray half folded into -|o|^2, the per-sphere half into nq.
+constexpr float kGateSlack = 0x1p-18f;
+inline float gate_nk2(const F3& o) { return -std::fmaf(o.z, o.z, std::fmaf(o.y, o.y, o.x * o.x)) * (1.0f - kGateSlack); }
+
+inline MSphere mirror_sphere(const rtz_sphere& s) {
+    MSphere m;
+    const float r = (float)(s.radius < 0 ? 0.0 : s.radius);
+    m.cx = (float)s.center[0], m.cy = (float)s.center[1], m.cz = (float)s.center[2], m.r2 = r * r;
+    const double c2 = (double)m.cx * m.cx + (double)m.cy * m.cy + (double)m.cz * m.cz;
+    m.nq = -(float)((c2 - (double)r * r) - (double)kGateSlack * c2);
+    m.r = r, m.inv_r = 1.0f / r;
+    m.param = s.mat_type == RTZ_MAT_METAL ? (float)s.fuzz : (float)s.refraction_index;
+    m.type = s.mat_type;
+    m.ar = (float)s.albedo[0], m.ag = (float)s.albedo[1], m.ab = (float)s.albedo[2];
+    m.inv_ior = 1.0f / (float)s.refraction_index;
+    return m;
+}
+
+// Test-only: false sends every sphere to the direct form (orc_mirror_set_gate).  A conservative gate only filters,
+// so the mirror's results must not depend on it.
+bool g_gate = true;
+
 inline void sweep(const std::vector<MSphere>& sp, const Path& p, float tmin, float tmax, float& t_out, int& best_out) {
     const float tmin_d = tmin * p.len;  // Scene.interval in distance units
     float closest = tmax * p.len;
@@ -138,15 +161,16 @@ inline void sweep(const std::vector<MSphere>& sp, const Path& p, float tmin, flo
     const int n = (int)sp.size();
     // per-ray constants of the expanded discriminant
     const float k1 = -std::fmaf(p.d.z, p.o.z, std::fmaf(p.d.y, p.o.y, p.d.x * p.o.x));
-    const float nk2 = -std::fmaf(p.o.z, p.o.z, std::fmaf(p.o.y, p.o.y, p.o.x * p.o.x));
+    const float nk2 = gate_nk2(p.o);
     const float tx = 2.0f * p.o.x, ty = 2.0f * p.o.y, tz = 2.0f * p.o.z;
+    const bool gate = g_gate;
     for (int i = 0; i < n; ++i) {
         const MSphere& s = sp[i];
-        // candidate test: h = d.c - d.o ; w = (2 o.c - |o|^2) - (|c|^2 - r^2) ; disc = h^2 + w
+        // candidate test: h = d.c - d.o ; w = (2 o.c - |o|^2) - (|c|^2 - r^2) - margin ; disc = h^2 + w
         const float he = std::fmaf(p.d.z, s.cz, std::fmaf(p.d.y, s.cy, std::fmaf(p.d.x, s.cx, k1)));
         const float w = std::fmaf(tz, s.cz, std::fmaf(ty, s.cy, std::fmaf(tx, s.cx, nk2))) + s.nq;
         const float de = std::fmaf(he, he, w);
-        if (std::signbit(de)) continue;
+        if (gate && std::signbit(de)) continue;
         // root from the direct form (reference src/sphere.zig:27-42, unit direction)
         const float ocx = s.cx - p.o.x, ocy = s.cy - p.o.y, ocz = s.cz - p.o.z;
         const float h = std::fmaf(p.d.z, ocz, std::fmaf(p.d.y, ocy, p.d.x * ocx));
@@ -262,18 +286,7 @@ int orc_render_mirror(const rtz_camera* cam, const rtz_sphere* sp, uint64_t n, u
     if (!cam || !sp || cam->mode != RTZ_MODE_PATH) return RTZ_ERR_BAD_ARG;
     if (threads < 1) threads = 1;
     std::vector<MSphere> ms(n);
-    for (uint64_t i = 0; i < n; ++i) {
-        const rtz_sphere& s = sp[i];
-        MSphere& m = ms[i];
-        const float r = (float)(s.radius < 0 ? 0.0 : s.radius);
-        m.cx = (float)s.center[0], m.cy = (float)s.center[1], m.cz = (float)s.center[2], m.r2 = r * r;
-        m.nq = -(float)(((double)m.cx * m.cx + (double)m.cy * m.cy + (double)m.cz * m.cz) - (double)r * r);
-        m.r = r, m.inv_r = 1.0f / r;
-        m.param = s.mat_type == RTZ_MAT_METAL ? (float)s.fuzz : (float)s.refraction_index;
-        m.type = s.mat_type;
-        m.ar = (float)s.albedo[0], m.ag = (float)s.albedo[1], m.ab = (float)s.albedo[2];
-        m.inv_ior = 1.0f / (float)s.refraction_index;
-    }
+    for (uint64_t i = 0; i < n; ++i) ms[i] = mirror_sphere(sp[i]);
     MCamera c;
     c.p0 = f3(cam->pixel0), c.du = f3(cam->du), c.dv = f3(cam->dv), c.c = f3(cam->center);
     c.uu = f3(cam->defocus_disk_u), c.vv = f3(cam->defocus_disk_v);
@@ -369,6 +382,76 @@ void orc_mirror_camera_ray(const rtz_camera* cam, uint64_t seed, uint32_t i, uin
         d[3 * k] = p.d.x, d[3 * k + 1] = p.d.y, d[3 * k + 2] = p.d.z;
         if (len) len[k] = p.len;
     }
+}
+
+// Test-only: on = 0 sends every sphere to the direct form in the mirror's renders and probes.
+void orc_mirror_set_gate(int on) { g_gate = on != 0; }
+
+// twin of rtz_probe_hits: the mirror's sweep for m rays
+void orc_mirror_hits(const rtz_sphere* sp, uint64_t n, const rtz_probe_ray* rays, uint64_t m, double tmin, double tmax,
+                     rtz_ray_hit* out) {
+    std::vector<MSphere> ms(n);
+    for (uint64_t i = 0; i < n; ++i) ms[i] = mirror_sphere(sp[i]);
+    for (uint64_t k = 0; k < m; ++k) {
+        const rtz_probe_ray& r = rays[k];
+        Path p;
+        p.o = {r.orig[0], r.orig[1], r.orig[2]}, p.self = r.self, p.bounce = 0, p.tr = p.tg = p.tb = 1.0f;
+        setDirection(p, r.dir[0], r.dir[1], r.dir[2]);
+        float t;
+        int best;
+        sweep(ms, p, (float)tmin, (float)tmax, t, best);
+        rtz_ray_hit h = {best, 0, t, p.len, {0.f, 0.f, 0.f}, {0.f, 0.f, 0.f}};
+        if (best >= 0) {
+            const MSphere& s = ms[best];
+            const float px = std::fmaf(t, p.d.x, p.o.x), py = std::fmaf(t, p.d.y, p.o.y), pz = std::fmaf(t, p.d.z, p.o.z);
+            float nx = (px - s.cx) * s.inv_r, ny = (py - s.cy) * s.inv_r, nz = (pz - s.cz) * s.inv_r;
+            const bool front = std::fmaf(p.d.z, nz, std::fmaf(p.d.y, ny, p.d.x * nx)) < 0.0f;
+            if (!front) nx = -nx, ny = -ny, nz = -nz;
+            h.front = front, h.point[0] = px, h.point[1] = py, h.point[2] = pz;
+            h.normal[0] = nx, h.normal[1] = ny, h.normal[2] = nz;
+        }
+        out[k] = h;
+    }
+}
+
+// twin of rtz_probe_scatters: Sphere.hit on the record's sphere, then the mirror's shade
+void orc_mirror_scatters(const rtz_sphere* sp, uint64_t n, const rtz_probe_bounce* recs, uint64_t m, uint64_t seed,
+                         rtz_ray_scatter* out) {
+    std::vector<MSphere> ms(n);
+    for (uint64_t i = 0; i < n; ++i) ms[i] = mirror_sphere(sp[i]);
+    MCamera c{};
+    c.tmin = 1e-3f, c.tmax = INFINITY, c.bounce_max = 0xFFFFFFFFu;
+    c.k0 = (uint32_t)seed, c.k1 = (uint32_t)(seed >> 32);
+    for (uint64_t k = 0; k < m; ++k) {
+        const rtz_probe_bounce& r = recs[k];
+        Path p;
+        p.o = {r.orig[0], r.orig[1], r.orig[2]}, p.self = -1, p.bounce = r.bounce, p.tr = p.tg = p.tb = 1.0f;
+        setDirection(p, r.dir[0], r.dir[1], r.dir[2]);
+        const std::vector<MSphere> one{ms[r.sphere]};
+        float t;
+        int best;
+        sweep(one, p, c.tmin, c.tmax, t, best);
+        rtz_ray_scatter s = {-2, {0.f, 0.f, 0.f}, {0.f, 0.f, 0.f}, 0.f, {0.f, 0.f, 0.f}};
+        if (best >= 0) {
+            const Rng g{{c.k0, c.k1}, r.pixel, r.sample};
+            float sr, sg, sb;
+            int term = -1;
+            if (shade(c, g, ms, p, t, r.sphere, sr, sg, sb, term)) {
+                s.term = term;
+            } else {
+                s.term = -1;
+                s.orig[0] = p.o.x, s.orig[1] = p.o.y, s.orig[2] = p.o.z;
+                s.dir[0] = p.d.x, s.dir[1] = p.d.y, s.dir[2] = p.d.z, s.len = p.len;
+                s.attenuation[0] = p.tr, s.attenuation[1] = p.tg, s.attenuation[2] = p.tb;
+            }
+        }
+        out[k] = s;
+    }
+}
+
+// the mirror's (cos 2 pi u, sin 2 pi u) for the 2^24 uniforms u = i * 2^-24, i = 0 .. 2^24 - 1
+void orc_mirror_cos_sin_all(float* c, float* s) {
+    for (uint32_t i = 0; i < (1u << 24); ++i) cosSin2Pi(i << 8, c[i], s[i]);
 }
 
 // one-ray mirrors of the device probes

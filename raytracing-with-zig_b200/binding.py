@@ -86,6 +86,8 @@ SIGNATURES = {
     "rtz_probe_hit": (_i32, [C.POINTER(rtz_sphere), _u64, D3, D3, _f64, _f64, C.POINTER(rtz_hit)]),
     "rtz_probe_scatter": (_i32, [C.POINTER(rtz_sphere), _u64, _i32, D3, D3, _u64, _u32, _u32, _u32,
                                  C.POINTER(rtz_scatter)]),
+    "rtz_probe_hits": (_i32, [C.POINTER(rtz_sphere), _u64, _vp, _u64, _f64, _f64, _vp]),
+    "rtz_probe_scatters": (_i32, [C.POINTER(rtz_sphere), _u64, _vp, _u64, _u64, _vp]),
     "rtz_probe_to_rgb": (_i32, [_f64p, _u64, _u8p]),
     "rtz_probe_sweep_order": (_i32, [C.POINTER(rtz_sphere), _u64, C.POINTER(_i32)]),
     "rtz_probe_uniform": (_i32, [_u64, _u32, _u32, _u32, _u64, _f32p]),

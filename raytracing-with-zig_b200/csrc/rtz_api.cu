@@ -700,8 +700,10 @@ int32_t rtz_scene_upload(rtz_context* c, const rtz_sphere* sp, uint64_t n) {
             return RTZ_ERR_BAD_ARG;
         }
         const float cx = (float)s.center[0], cy = (float)s.center[1], cz = (float)s.center[2];
-        // q = |c|^2 - r^2 of the FP32-rounded sphere, evaluated in f64 and rounded once
-        const double q = ((double)cx * cx + (double)cy * cy + (double)cz * cz) - (double)r * r;
+        // q = |c|^2 - r^2 of the FP32-rounded sphere less the per-sphere half of the gate's margin (kGateSlack at
+        // ray_constants), evaluated in f64 and rounded once
+        const double c2 = (double)cx * cx + (double)cy * cy + (double)cz * cz;
+        const double q = (c2 - (double)r * r) - (double)rtz::kGateSlack * c2;
         g[i] = make_float4(cx, cy, cz, -(r * r));
         w[i] = -(float)q;
         const float param = s.mat_type == RTZ_MAT_METAL ? (float)s.fuzz : (float)s.refraction_index;
@@ -1362,30 +1364,76 @@ int32_t rtz_render_multi(const rtz_camera* cam, const rtz_sphere* sp, uint64_t n
 extern "C" {
 
 // ---- probes -------------------------------------------------------------------------------------
-int32_t rtz_probe_hit(const rtz_sphere* sp, uint64_t n, const double o[3], const double d[3], double tmin, double tmax,
-                      rtz_hit* out) {
-    if (!sp || !n || !o || !d || !out) return RTZ_ERR_BAD_ARG;
+}  // extern "C"
+
+namespace {
+// Upload the scene to a fresh context, copy the m records in, run `launch(ctx, in, out)` and copy the m results out.
+template <class In, class Out, class Launch>
+int32_t run_probe(const rtz_sphere* sp, uint64_t n, const In* in, uint64_t m, Out* out, Launch launch) {
     ScopedCtx sc;
     int32_t rc = rtz_context_create(-1, nullptr, &sc.c);
     if (rc != RTZ_OK) return rc;
     rc = rtz_scene_upload(sc.c, sp, n);
     if (rc != RTZ_OK) return rc;
-    rtz::ProbeHitOut* dout;
-    RTZ_CUDA(cudaMalloc(&dout, sizeof(*dout)));
-    rtz::probe_hit_kernel<<<1, 1, 0, sc.c->stream>>>(sc.c->geom.p, sc.c->pairs.p, sc.c->aux.p, sc.c->n_pad, (float)o[0], (float)o[1],
-                                                    (float)o[2], (float)d[0], (float)d[1], (float)d[2], (float)tmin,
-                                                    (float)tmax, dout);
-    rtz::ProbeHitOut h;
-    cudaError_t e = cudaMemcpyAsync(&h, dout, sizeof(h), cudaMemcpyDeviceToHost, sc.c->stream);
+    In* din = nullptr;
+    Out* dout = nullptr;
+    cudaError_t e = cudaMalloc(&din, m * sizeof(In));
+    if (e == cudaSuccess) e = cudaMalloc(&dout, m * sizeof(Out));
+    if (e == cudaSuccess) e = cudaMemcpyAsync(din, in, m * sizeof(In), cudaMemcpyHostToDevice, sc.c->stream);
+    if (e == cudaSuccess) {
+        launch(sc.c, din, dout, (unsigned)((m + 127) / 128));
+        e = cudaGetLastError();
+    }
+    if (e == cudaSuccess) e = cudaMemcpyAsync(out, dout, m * sizeof(Out), cudaMemcpyDeviceToHost, sc.c->stream);
     if (e == cudaSuccess) e = cudaStreamSynchronize(sc.c->stream);
+    cudaFree(din);
     cudaFree(dout);
     RTZ_CUDA(e);
+    return RTZ_OK;
+}
+}  // namespace
+
+extern "C" {
+
+int32_t rtz_probe_hits(const rtz_sphere* sp, uint64_t n, const rtz_probe_ray* rays, uint64_t m, double tmin,
+                       double tmax, rtz_ray_hit* out) {
+    if (!sp || !n || (!rays && m) || (!out && m) || m > (1ull << 31)) return RTZ_ERR_BAD_ARG;
+    if (!m) return RTZ_OK;
+    return run_probe(sp, n, rays, m, out, [&](rtz_context* c, const rtz_probe_ray* din, rtz_ray_hit* dout, unsigned blocks) {
+        rtz::probe_hits_kernel<<<blocks, 128, 0, c->stream>>>(c->geom.p, c->pairs.p, c->aux.p, c->n_pad, din, m,
+                                                             (float)tmin, (float)tmax, dout);
+    });
+}
+
+int32_t rtz_probe_scatters(const rtz_sphere* sp, uint64_t n, const rtz_probe_bounce* recs, uint64_t m, uint64_t seed,
+                           rtz_ray_scatter* out) {
+    if (!sp || !n || (!recs && m) || (!out && m) || m > (1ull << 31)) return RTZ_ERR_BAD_ARG;
+    for (uint64_t k = 0; k < m; ++k)
+        if (recs[k].sphere < 0 || (uint64_t)recs[k].sphere >= n) return RTZ_ERR_BAD_ARG;
+    if (!m) return RTZ_OK;
+    rtz_camera cam;
+    std::memset(&cam, 0, sizeof(cam));
+    cam.t_min = 1e-3, cam.t_max = INFINITY, cam.bounce_max = 0xFFFFFFFFull, cam.samples_per_pixel = 1, cam.width = cam.height = 1;
+    const rtz::DevCamera dc = to_dev_camera(cam, seed);
+    return run_probe(sp, n, recs, m, out, [&](rtz_context* c, const rtz_probe_bounce* din, rtz_ray_scatter* dout, unsigned blocks) {
+        rtz::probe_scatters_kernel<<<blocks, 128, 0, c->stream>>>(dc, c->geom.p, c->pairs.p, c->aux.p, c->albedo.p, din, m,
+                                                                 dout);
+    });
+}
+
+int32_t rtz_probe_hit(const rtz_sphere* sp, uint64_t n, const double o[3], const double d[3], double tmin, double tmax,
+                      rtz_hit* out) {
+    if (!sp || !n || !o || !d || !out) return RTZ_ERR_BAD_ARG;
+    const rtz_probe_ray r = {{(float)o[0], (float)o[1], (float)o[2]}, {(float)d[0], (float)d[1], (float)d[2]}, -1};
+    rtz_ray_hit h;
+    const int32_t rc = rtz_probe_hits(sp, n, &r, 1, tmin, tmax, &h);
+    if (rc != RTZ_OK) return rc;
     std::memset(out, 0, sizeof(*out));
-    out->hit = h.hit;
-    if (h.hit) {
-        out->index = h.index, out->front = h.front;
+    out->hit = h.best >= 0;
+    if (h.best >= 0) {
+        out->index = h.best, out->front = h.front;
         out->t = (double)h.t / (double)h.len;  // back to the reference's units of |dir|
-        for (int k = 0; k < 3; ++k) out->point[k] = h.p[k], out->normal[k] = h.n[k];
+        for (int k = 0; k < 3; ++k) out->point[k] = h.point[k], out->normal[k] = h.normal[k];
     }
     return RTZ_OK;
 }
@@ -1393,32 +1441,18 @@ int32_t rtz_probe_hit(const rtz_sphere* sp, uint64_t n, const double o[3], const
 int32_t rtz_probe_scatter(const rtz_sphere* sp, uint64_t n, int32_t index, const double o[3], const double d[3],
                           uint64_t seed, uint32_t pixel, uint32_t sample, uint32_t bounce, rtz_scatter* out) {
     if (!sp || !n || index < 0 || (uint64_t)index >= n || !o || !d || !out) return RTZ_ERR_BAD_ARG;
-    ScopedCtx sc;
-    int32_t rc = rtz_context_create(-1, nullptr, &sc.c);
+    const rtz_probe_bounce r = {index, {(float)o[0], (float)o[1], (float)o[2]}, {(float)d[0], (float)d[1], (float)d[2]},
+                                pixel, sample, bounce};
+    rtz_ray_scatter h;
+    const int32_t rc = rtz_probe_scatters(sp, n, &r, 1, seed, &h);
     if (rc != RTZ_OK) return rc;
-    rc = rtz_scene_upload(sc.c, sp, n);
-    if (rc != RTZ_OK) return rc;
-    rtz_camera cam;
-    std::memset(&cam, 0, sizeof(cam));
-    cam.t_min = 1e-3, cam.t_max = INFINITY, cam.bounce_max = 0xFFFFFFFFull, cam.samples_per_pixel = 1, cam.width = cam.height = 1;
-    const rtz::DevCamera dc = to_dev_camera(cam, seed);
-    rtz::ProbeScatterOut* dout;
-    RTZ_CUDA(cudaMalloc(&dout, sizeof(*dout)));
-    rtz::probe_scatter_kernel<<<1, 1, 0, sc.c->stream>>>(dc, sc.c->geom.p, sc.c->pairs.p, sc.c->aux.p, sc.c->albedo.p, index,
-                                                        (float)o[0], (float)o[1], (float)o[2], (float)d[0], (float)d[1],
-                                                        (float)d[2], pixel, sample, bounce, dout);
-    rtz::ProbeScatterOut h;
-    cudaError_t e = cudaMemcpyAsync(&h, dout, sizeof(h), cudaMemcpyDeviceToHost, sc.c->stream);
-    if (e == cudaSuccess) e = cudaStreamSynchronize(sc.c->stream);
-    cudaFree(dout);
-    RTZ_CUDA(e);
     std::memset(out, 0, sizeof(*out));
-    out->scattered = h.scattered;
-    if (h.scattered)
+    out->scattered = h.term == -1;
+    if (h.term == -1)
         for (int k = 0; k < 3; ++k) {
-            out->origin[k] = h.o[k];
-            out->direction[k] = (double)h.d[k] * (double)h.len;
-            out->attenuation[k] = h.att[k];
+            out->origin[k] = h.orig[k];
+            out->direction[k] = (double)h.dir[k] * (double)h.len;
+            out->attenuation[k] = h.attenuation[k];
         }
     return RTZ_OK;
 }

@@ -203,17 +203,23 @@ __device__ __forceinline__ void slow_path(float h, float disc, int i, int self, 
 // per-ray constants of the expanded discriminant
 struct RayK {
     float k1;             // -(d.o)
-    float nk2;            // -|o|^2
+    float nk2;            // -|o|^2 (1 - kGateSlack): the per-ray half of the gate's margin
     float tx, ty, tz;     // 2*o
 };
+// The expanded form rounds with an error that grows with eps (|o| + |c|)^2, the direct form that decides the root
+// with eps |c - o|^2.  Far from the world origin the expanded sign alone would reject spheres the direct form hits,
+// so the gate tests disc + kGateSlack (|o|^2 + |c|^2) >= 0 instead: the margin is split into the factor on -|o|^2
+// here and the term +kGateSlack |c|^2 that the host folds into cw.  kGateSlack = 64 eps covers both forms' rounding
+// with the margin's own rounding (derivation: DESIGN.md §4), so the gate never drops a sphere the direct form accepts.
+constexpr float kGateSlack = 0x1p-18f;  // 64 * 2^-24
 __device__ __forceinline__ RayK ray_constants(const Path& p) {
     RayK k;
     k.k1 = -fmaf(p.dz, p.oz, fmaf(p.dy, p.oy, p.dx * p.ox));
-    k.nk2 = -fmaf(p.oz, p.oz, fmaf(p.oy, p.oy, p.ox * p.ox));
+    k.nk2 = -fmaf(p.oz, p.oz, fmaf(p.oy, p.oy, p.ox * p.ox)) * (1.0f - kGateSlack);
     k.tx = 2.0f * p.ox, k.ty = 2.0f * p.oy, k.tz = 2.0f * p.oz;
     return k;
 }
-// candidate test: sign of the expanded discriminant; cw = -(|c|^2 - r^2) from the host
+// candidate test: sign of the expanded discriminant; cw = -(|c|^2 - r^2) + kGateSlack |c|^2 from the host
 __device__ __forceinline__ float expanded_disc(float cx, float cy, float cz, float cw, const Path& p, const RayK& k) {
     const float h = fmaf(p.dz, cz, fmaf(p.dy, cy, fmaf(p.dx, cx, k.k1)));
     const float w = fmaf(k.tz, cz, fmaf(k.ty, cy, fmaf(k.tx, cx, k.nk2))) + cw;

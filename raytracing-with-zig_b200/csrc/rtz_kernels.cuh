@@ -194,11 +194,13 @@ __device__ __forceinline__ void test_pair(const float4 p0, const float4 p1, cons
 //
 // Exactness contract of the block cull: a lane may report "no" only if the FP32 pipeline (sign of the expanded
 // discriminant, then the direct-form root in (t_min * |d|, closest)) would accept no sphere of the block.
-//  * An accepted root lies inside the padded box.  Both discriminant gates must pass, and each is off by at most
-//    about 12 eps |c - o|^2 (eps = 2^-24), so an accepted point p = o + t d — a self hit, o + 2 h d, included — has
-//    |p - c|^2 <= r^2 + 24 eps |c - o|^2: |p - c| <= r + 12 eps |c - o|^2 / r.  The host pads every sphere by
-//    1e-6 (R + |c|)^2 / r for |o| <= R (1e-6 > 16 eps) on top of the BVH builder's 1e-4 (1 + r + |c|_1); a ray
-//    starting farther out than R (|o|^2 > cull_r2) needs every block.
+//  * An accepted root lies inside the padded box.  Acceptance is decided by the direct form, whose disc is off by at
+//    most about 12 eps |c - o|^2 (eps = 2^-24); the expanded gate in front of it only filters and, with its margin
+//    (kGateSlack), never rejects what the direct form accepts.  So an accepted point p = o + t d — a self hit,
+//    o + 2 h d, included — has |p - c|^2 <= r^2 + 24 eps |c - o|^2: |p - c| <= r + 12 eps |c - o|^2 / r.  The host
+//    pads every sphere by 1e-6 (1.001 R + |c|)^2 / r for |o| <= R (1e-6 > 16 eps) on top of the BVH builder's
+//    1e-4 (1 + r + |c|_1); a ray starting farther out than R (|o|^2 > cull_r2) needs every block.  The origin test
+//    reads -nk2 = |o|^2 (1 - 2^-18), i.e. it admits |o| up to R (1 + 2e-6), well inside the 1.001 R of the padding.
 //  * The test itself errs towards "yes": the interval is [0, closest], a superset of (t_min |d|, closest), and
 //    compared with <=, never strictly; an accepted point sits at least the padding inside every face, far beyond
 //    the few ulps of (lo - o) * (1 / d); fminf / fmaxf drop the NaN of 0 * inf (an axis-parallel ray in the plane
@@ -1614,59 +1616,58 @@ __global__ void deinterleave_kernel(const uint8_t* __restrict__ gathered, uint64
 }
 
 // ---------------------------------------------------------------------------------------------
-// probes: one thread, the same device functions the render kernel inlines
+// probes: one thread per record, the same device functions the render kernel inlines
 // ---------------------------------------------------------------------------------------------
-struct ProbeHitOut {
-    int hit, index, front;
-    float t, len;
-    float p[3], n[3];
-};
-__global__ void probe_hit_kernel(const float4* geom, const float4* pairs, const float4* aux, int n_pad, float ox, float oy, float oz,
-                                 float dx, float dy, float dz, float tmin, float tmax, ProbeHitOut* out) {
+__global__ void probe_hits_kernel(const float4* geom, const float4* pairs, const float4* aux, int n_pad,
+                                  const rtz_probe_ray* rays, uint64_t m, float tmin, float tmax, rtz_ray_hit* out) {
+    const uint64_t k = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (k >= m) return;
+    const rtz_probe_ray r = rays[k];
     Path p;
-    p.ox = ox, p.oy = oy, p.oz = oz, p.self = -1, p.bounce = 0, p.tr = p.tg = p.tb = 1.f;
-    set_direction(p, dx, dy, dz);
+    p.ox = r.orig[0], p.oy = r.orig[1], p.oz = r.orig[2], p.self = r.self, p.bounce = 0, p.tr = p.tg = p.tb = 1.f;
+    set_direction(p, r.dir[0], r.dir[1], r.dir[2]);
     float t;
     int best;
     sweep_rows(geom, pairs, 0, n_pad, p, tmin, tmax, t, best);
-    out->hit = best >= 0, out->index = best, out->len = p.len, out->t = t;
+    rtz_ray_hit h = {best, 0, t, p.len, {0.f, 0.f, 0.f}, {0.f, 0.f, 0.f}};
     if (best >= 0) {
         const float gx = geom[best].x, gy = geom[best].y, gz = geom[best].z;
         const float px = fmaf(t, p.dx, p.ox), py = fmaf(t, p.dy, p.oy), pz = fmaf(t, p.dz, p.oz);
         float nx = (px - gx) * aux[best].y, ny = (py - gy) * aux[best].y, nz = (pz - gz) * aux[best].y;
         const bool front = fmaf(p.dz, nz, fmaf(p.dy, ny, p.dx * nx)) < 0.f;
         if (!front) nx = -nx, ny = -ny, nz = -nz;
-        out->front = front, out->p[0] = px, out->p[1] = py, out->p[2] = pz, out->n[0] = nx, out->n[1] = ny, out->n[2] = nz;
+        h.front = front, h.point[0] = px, h.point[1] = py, h.point[2] = pz, h.normal[0] = nx, h.normal[1] = ny, h.normal[2] = nz;
     }
+    out[k] = h;
 }
 
-struct ProbeScatterOut {
-    int scattered, term;
-    float o[3], d[3], att[3], len;
-};
-__global__ void probe_scatter_kernel(DevCamera cam, const float4* geom, const float4* pairs, const float4* aux,
-                                     const float4* albedo,
-                                     int index, float ox, float oy, float oz, float dx, float dy, float dz,
-                                     uint32_t pixel, uint32_t sample, uint32_t bounce, ProbeScatterOut* out) {
+__global__ void probe_scatters_kernel(DevCamera cam, const float4* geom, const float4* pairs, const float4* aux,
+                                      const float4* albedo, const rtz_probe_bounce* recs, uint64_t m,
+                                      rtz_ray_scatter* out) {
+    const uint64_t k = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (k >= m) return;
+    const rtz_probe_bounce r = recs[k];
     Path p;
-    p.ox = ox, p.oy = oy, p.oz = oz, p.self = -1, p.bounce = bounce, p.tr = p.tg = p.tb = 1.f;
-    set_direction(p, dx, dy, dz);
+    p.ox = r.orig[0], p.oy = r.orig[1], p.oz = r.orig[2], p.self = -1, p.bounce = r.bounce, p.tr = p.tg = p.tb = 1.f;
+    set_direction(p, r.dir[0], r.dir[1], r.dir[2]);
     float t;
     int best;
-    sweep_rows(geom, pairs, index, 1, p, cam.tmin, cam.tmax, t, best);  // Sphere.hit on that one sphere
-    out->scattered = 0, out->term = -1;
-    if (best < 0) return;
-    RngKey k{cam.key0, cam.key1, pixel, sample};
-    float sr, sg, sb;
-    int term = -1;
-    const bool done = shade(cam, k, geom, aux, albedo, p, t, index, sr, sg, sb, term);
-    out->term = term;
-    if (done) return;
-    out->scattered = 1;
-    out->o[0] = p.ox, out->o[1] = p.oy, out->o[2] = p.oz;
-    out->len = p.len;  // |direction| before normalisation
-    out->d[0] = p.dx, out->d[1] = p.dy, out->d[2] = p.dz;
-    out->att[0] = p.tr, out->att[1] = p.tg, out->att[2] = p.tb;
+    sweep_rows(geom, pairs, r.sphere, 1, p, cam.tmin, cam.tmax, t, best);  // Sphere.hit on that one sphere
+    rtz_ray_scatter s = {-2, {0.f, 0.f, 0.f}, {0.f, 0.f, 0.f}, 0.f, {0.f, 0.f, 0.f}};
+    if (best >= 0) {
+        const RngKey key{cam.key0, cam.key1, r.pixel, r.sample};
+        float sr, sg, sb;
+        int term = -1;
+        if (shade(cam, key, geom, aux, albedo, p, t, best, sr, sg, sb, term)) {
+            s.term = term;
+        } else {
+            s.term = -1;
+            s.orig[0] = p.ox, s.orig[1] = p.oy, s.orig[2] = p.oz;
+            s.dir[0] = p.dx, s.dir[1] = p.dy, s.dir[2] = p.dz, s.len = p.len;
+            s.attenuation[0] = p.tr, s.attenuation[1] = p.tg, s.attenuation[2] = p.tb;
+        }
+    }
+    out[k] = s;
 }
 
 __global__ void probe_camera_ray_kernel(DevCamera cam, uint32_t i, uint32_t j, uint32_t sample0, uint32_t n, float* o,

@@ -211,6 +211,14 @@ def oracle():
         lib.orc_mirror_camera_ray.restype = None
         lib.orc_mirror_camera_ray.argtypes = [P(Camera), u64, C.c_uint32, C.c_uint32, C.c_uint32, C.c_uint32,
                                               P(C.c_float), P(C.c_float), P(C.c_float)]
+    if hasattr(lib, "orc_mirror_hits"):   # twins of rtz_probe_hits / rtz_probe_scatters (records as raw pointers)
+        lib.orc_mirror_set_gate.restype, lib.orc_mirror_set_gate.argtypes = None, [C.c_int]
+        lib.orc_mirror_hits.restype = None
+        lib.orc_mirror_hits.argtypes = [P(Sphere), u64, vp, u64, f64, f64, vp]
+        lib.orc_mirror_scatters.restype = None
+        lib.orc_mirror_scatters.argtypes = [P(Sphere), u64, vp, u64, u64, vp]
+        lib.orc_mirror_cos_sin_all.restype = None
+        lib.orc_mirror_cos_sin_all.argtypes = [P(C.c_float), P(C.c_float)]
     _oracle = lib
     return lib
 

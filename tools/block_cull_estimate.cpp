@@ -40,7 +40,7 @@ struct Seg {
 // accept, or +inf.  With a finite running closest the loop accepts that same root iff it lies below closest.
 float accepted_root(const MSphere& s, int i, const Path& p, float tmin_d) {
     const float k1 = -std::fmaf(p.d.z, p.o.z, std::fmaf(p.d.y, p.o.y, p.d.x * p.o.x));
-    const float nk2 = -std::fmaf(p.o.z, p.o.z, std::fmaf(p.o.y, p.o.y, p.o.x * p.o.x));
+    const float nk2 = gate_nk2(p.o);
     const float he = std::fmaf(p.d.z, s.cz, std::fmaf(p.d.y, s.cy, std::fmaf(p.d.x, s.cx, k1)));
     const float w = std::fmaf(2.0f * p.o.z, s.cz, std::fmaf(2.0f * p.o.y, s.cy, std::fmaf(2.0f * p.o.x, s.cx, nk2))) + s.nq;
     if (std::signbit(std::fmaf(he, he, w))) return INFINITY;
@@ -229,18 +229,7 @@ int main(int argc, char** argv) {
     const int n = (int)sp.size(), n_pad = (n + 7) & ~7;
 
     std::vector<MSphere> ms(n);
-    for (int i = 0; i < n; ++i) {
-        const rtz_sphere& s = sp[i];
-        MSphere& m = ms[i];
-        const float r = (float)s.radius;
-        m.cx = (float)s.center[0], m.cy = (float)s.center[1], m.cz = (float)s.center[2], m.r2 = r * r;
-        m.nq = -(float)(((double)m.cx * m.cx + (double)m.cy * m.cy + (double)m.cz * m.cz) - (double)r * r);
-        m.r = r, m.inv_r = 1.0f / r;
-        m.param = s.mat_type == RTZ_MAT_METAL ? (float)s.fuzz : (float)s.refraction_index;
-        m.type = s.mat_type;
-        m.ar = (float)s.albedo[0], m.ag = (float)s.albedo[1], m.ab = (float)s.albedo[2];
-        m.inv_ior = 1.0f / (float)s.refraction_index;
-    }
+    for (int i = 0; i < n; ++i) ms[i] = mirror_sphere(sp[i]);
     MCamera c;
     c.p0 = f3(cam.pixel0), c.du = f3(cam.du), c.dv = f3(cam.dv), c.c = f3(cam.center);
     c.uu = f3(cam.defocus_disk_u), c.vv = f3(cam.defocus_disk_v);
