@@ -344,6 +344,11 @@ int32_t enqueue_path(rtz_context* ctx, const rtz_camera* cam, const rtz::ShardGe
             std::memcpy(C.pairs, ctx->h_rg_pairs.data(), (size_t)ctx->n_pad * sizeof(float4));
             std::memcpy(C.boxes, ctx->h_boxes.data(), ctx->h_boxes.size() * sizeof(float4));
             C.cull_r2 = ctx->cull_r2;
+            // culled blocks that at most this many of a warp's 64 paths reach are swept sphere-parallel (sweep2);
+            // RTZ_SPLIT overrides it for tests and A/B runs (0: the packed sweep alone, 64: every reached block
+            // sphere-parallel).  The image does not depend on it.
+            C.split_max = rtz::kSplitMax;
+            if (const char* e = std::getenv("RTZ_SPLIT")) C.split_max = std::atoi(e);
             rc = launch_trace(ctx, rtz::trace_kernel_const_cull<128, 6>, C, P.n_chunks, 128, 0);
         } else
             rc = launch_trace(ctx, rtz::trace_kernel_const<128, 6>, C, P.n_chunks, 128, 0);

@@ -66,7 +66,10 @@ struct TraceParamsConst {
     // distance from the world origin beyond which a ray origin was not accounted for in the padding
     float4 boxes[2 * (kMaxConstSpheres / 32)];
     float cull_r2;
+    // a culled block that at most this many of the warp's 64 paths reach is swept sphere-parallel (sweep2)
+    int split_max;
 };
+constexpr int kSplitMax = 16;
 
 // local (compact, padded) pixel index -> global pixel; false for tile padding
 __device__ __forceinline__ bool local_to_global(const ShardGeom& s, uint32_t W, uint32_t H, uint32_t lp, uint32_t& x,
@@ -205,6 +208,11 @@ __device__ __forceinline__ void test_pair(const float4 p0, const float4 p1, cons
 //    compared with <=, never strictly; an accepted point sits at least the padding inside every face, far beyond
 //    the few ulps of (lo - o) * (1 / d); fminf / fmaxf drop the NaN of 0 * inf (an axis-parallel ray in the plane
 //    of a face), which is then outside the box by the padding; an origin inside the box gives t_near = 0 <= t_far.
+// The contract is per path, so sweep2 may leave a path out of a block whose box it does not reach: the sphere-parallel
+// pass tests only the paths that reach the block, and the packed sweep tests every path of the warp, and both give
+// the same hits.  The two evaluate the same candidate gate (expanded_disc is test_pair's FMA sequence, one sphere at a
+// time) and resolve the candidates with resolve_candidates in ascending slot order, so the hit is still the
+// (t, original index) minimum whichever of the two swept a block.
 __device__ __forceinline__ bool box_reach(const float4 b0, const float4 b1, const Path& p, float ix, float iy, float iz,
                                           float closest) {
     const float2 tx = __fmul2_rn(__fadd2_rn(make_float2(b0.x, b0.y), make_float2(-p.ox, -p.ox)), make_float2(ix, ix));
@@ -213,6 +221,35 @@ __device__ __forceinline__ bool box_reach(const float4 b0, const float4 b1, cons
     const float tn = fmaxf(fmaxf(fminf(tx.x, tx.y), fminf(ty.x, ty.y)), fmaxf(fminf(tz.x, tz.y), 0.0f));
     const float tf = fminf(fminf(fmaxf(tx.x, tx.y), fmaxf(ty.x, ty.y)), fminf(fmaxf(tz.x, tz.y), closest));
     return tn <= tf;
+}
+
+// a shared-memory load the compiler cannot forward from an earlier store (so the stored value need not stay live)
+__device__ __forceinline__ float4 lds_opaque(const float4* p) {
+    float4 v;
+    asm volatile("ld.shared.v4.f32 {%0, %1, %2, %3}, [%4];" : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w) : "r"(smem_u32(p))
+                 : "memory");
+    return v;
+}
+
+// The sphere-parallel candidate test of one block: lane l holds sphere base + l ({cx, cy, cz} of `g`, and w), and
+// each path in `need` (bit l = the path of lane l) is read back from `stage` (its ray constants and direction, two
+// float4 at a uniform address) and tested against all of them at once.  The path's lane gets the ballot of the
+// spheres that pass the gate: bit l = sphere base + l.
+__device__ __forceinline__ unsigned split_candidates(const float4* __restrict__ stage, unsigned need, const float4 g,
+                                                     float w, unsigned lane) {
+    unsigned cand = 0u;
+    while (need) {
+        const unsigned src = __ffs(need) - 1;
+        need &= need - 1u;
+        const float4 s0 = stage[2 * src], s1 = stage[2 * src + 1];
+        Path q;
+        q.dx = s1.y, q.dy = s1.z, q.dz = s1.w;
+        const RayK k{s0.x, s0.y, s0.z, s0.w, s1.x};
+        const float d = expanded_disc(g.x, g.y, g.z, w, q, k);
+        const unsigned pass = __ballot_sync(0xFFFFFFFFu, !(__float_as_uint(d) >> 31));
+        if (lane == src) cand = pass;
+    }
+    return cand;
 }
 
 // HittableList.hit for the two paths of a thread.  `pairs` is warp-uniform storage (shared memory
@@ -226,11 +263,17 @@ __device__ __forceinline__ bool box_reach(const float4 b0, const float4 b1, cons
 // kCull (constant-bank lockstep kernel): a block of 32 spheres that no path of the warp can reach over (0, closest]
 // is skipped as a whole — a warp-uniform branch, so the loop stays on the uniform datapath.  Block 0 (the ground of
 // the book's scenes) is always swept first, which gives most paths a short closest hit before the bounds are tested.
+// The packed sweep costs the same whether 1 or 64 paths reach a block.  So a culled block that at most `split_max` of
+// the warp's 64 paths reach is swept sphere-parallel instead: lane l takes sphere base + l, and each reaching path's
+// ray constants are broadcast from the warp's staging rows (`stage`, written once per call) for one expanded_disc
+// and one ballot, which the path's lane keeps as its candidate mask.
 template <bool kConstBank, bool kSkipSelf = false, bool kCull = false>
 __device__ __forceinline__ void sweep2(const float4* __restrict__ pairs, const float4* __restrict__ gather, int n_pad,
                                        float tmin, float tmax, const Path& a, const Path& b, float& ta, int& ia,
                                        float& tb, int& ib, const float4* __restrict__ boxes = nullptr,
-                                       float cull_r2 = 0.0f, const int* __restrict__ orig = nullptr) {
+                                       float cull_r2 = 0.0f, const int* __restrict__ orig = nullptr,
+                                       const float* __restrict__ wexp = nullptr, int split_max = 0,
+                                       float4* __restrict__ stage = nullptr) {
     RayK ka = ray_constants(a), kb = ray_constants(b);
     // pin 2*o in registers: left alone, ptxas keeps o and re-adds it for every block of 32 spheres (not in the culled
     // sweep: its six reciprocals need those registers, and with the pin it spills under the 80-register cap)
@@ -247,25 +290,60 @@ __device__ __forceinline__ void sweep2(const float4* __restrict__ pairs, const f
         if (!(-ka.nk2 <= cull_r2)) iax = iay = iaz = __int_as_float(0x7fffffff);
         if (!(-kb.nk2 <= cull_r2)) ibx = iby = ibz = __int_as_float(0x7fffffff);
     }
+    if (kCull) {
+        // the warp's staging rows: path j (32 + lane for slot B) at stage[2j], stage[2j + 1], which the sphere-parallel
+        // pass broadcasts, and the lane's reciprocals at stage[128 + 2 lane], stage[129 + 2 lane]
+        const unsigned lane = threadIdx.x & 31u;
+        stage[2 * lane] = make_float4(ka.k1, ka.nk2, ka.tx, ka.ty);
+        stage[2 * lane + 1] = make_float4(ka.tz, a.dx, a.dy, a.dz);
+        stage[2 * lane + 64] = make_float4(kb.k1, kb.nk2, kb.tx, kb.ty);
+        stage[2 * lane + 65] = make_float4(kb.tz, b.dx, b.dy, b.dz);
+        stage[2 * lane + 128] = make_float4(iax, iay, iaz, 0.f);
+        stage[2 * lane + 129] = make_float4(ibx, iby, ibz, 0.f);
+        __syncwarp();
+    }
     for (int base = 0; base < n_pad; base += 32) {
+        unsigned canda, candb;
+        unsigned need_a = 0u, need_b = 0u;
         if (kCull && base > 0) {
             const float4 b0 = boxes[base >> 4], b1 = boxes[(base >> 4) + 1];
-            const bool need = box_reach(b0, b1, a, iax, iay, iaz, ca) | box_reach(b0, b1, b, ibx, iby, ibz, cb);
-            if (!__any_sync(0xFFFFFFFFu, need)) continue;
+            need_a = __ballot_sync(0xFFFFFFFFu, box_reach(b0, b1, a, iax, iay, iaz, ca));
+            need_b = __ballot_sync(0xFFFFFFFFu, box_reach(b0, b1, b, ibx, iby, ibz, cb));
+            if ((need_a | need_b) == 0u) continue;
         }
         const int cnt = min(32, n_pad - base);
-        unsigned ma = 0xFFFFFFFFu, mb = 0xFFFFFFFFu;  // 1 = miss
-        const float4* g = pairs + base;
+        if (kCull && base > 0 && __popc(need_a) + __popc(need_b) <= split_max) {
+            const unsigned lane = threadIdx.x & 31u;
+            // lanes >= cnt (the last block of a scene whose n_pad is not a multiple of 32) test a repeated sphere:
+            // their ballot bits are shifted out below
+            const int i = min(base + (int)lane, n_pad - 1);
+            const float4 g = gather[i];
+            const float w = __ldg(wexp + i);
+            canda = split_candidates(stage, need_a, g, w, lane);
+            candb = split_candidates(stage + 64, need_b, g, w, lane);
+            canda = __brev(canda) >> (32 - cnt);  // sphere base + i at bit cnt - 1 - i, as the packed sweep leaves it
+            candb = __brev(candb) >> (32 - cnt);
+            // the lane's own ray constants and reciprocals are read back instead of being held across this branch
+            // (the kernel runs at 80 registers)
+            const float4 a0 = lds_opaque(stage + 2 * lane), a1 = lds_opaque(stage + 2 * lane + 1);
+            const float4 b0 = lds_opaque(stage + 2 * lane + 64), b1 = lds_opaque(stage + 2 * lane + 65);
+            const float4 ra = lds_opaque(stage + 2 * lane + 128), rb = lds_opaque(stage + 2 * lane + 129);
+            ka = RayK{a0.x, a0.y, a0.z, a0.w, a1.x}, kb = RayK{b0.x, b0.y, b0.z, b0.w, b1.x};
+            iax = ra.x, iay = ra.y, iaz = ra.z, ibx = rb.x, iby = rb.y, ibz = rb.z;
+        } else {
+            unsigned ma = 0xFFFFFFFFu, mb = 0xFFFFFFFFu;  // 1 = miss
+            const float4* g = pairs + base;
 #pragma unroll 1
-        for (int k = 0; k < cnt; k += 8) {
+            for (int k = 0; k < cnt; k += 8) {
 #pragma unroll
-            for (int u = 0; u < 8; u += 2) {
-                const float4 p0 = g[k + u], p1 = g[k + u + 1];
-                test_pair(p0, p1, a, ka, ma);
-                test_pair(p0, p1, b, kb, mb);
+                for (int u = 0; u < 8; u += 2) {
+                    const float4 p0 = g[k + u], p1 = g[k + u + 1];
+                    test_pair(p0, p1, a, ka, ma);
+                    test_pair(p0, p1, b, kb, mb);
+                }
             }
+            canda = ~ma, candb = ~mb;
         }
-        unsigned canda = ~ma, candb = ~mb;
         if (kSkipSelf) {  // a ray that leaves its sphere outwards (shade<true> flagged it) cannot hit it: not a candidate
             const unsigned ra = (unsigned)(a.self & ~kSelfLeaves) - (unsigned)base, rb = (unsigned)(b.self & ~kSelfLeaves) - (unsigned)base;
             if ((a.self >> 30) == 1 && ra < (unsigned)cnt) canda &= ~(1u << (cnt - 1 - (int)ra));
@@ -414,15 +492,26 @@ __device__ __forceinline__ void take_camera_ray(const float* stage, uint32_t j, 
     p.bounce = 0;
 }
 constexpr int kStageFloats = 7 * 64;  // per warp: 7 rows (origin, unit direction, |direction|) of 64 rays (two slots per lane)
+// the culled kernel's rows also hold, during the sweep, the 8 ray constants of each of the 64 paths and the 6
+// reciprocals of each lane (sweep2)
+constexpr int kCullStageFloats = 12 * 64;
+
+// the warp's diagnostics row of P.timeline, formed where it is written: the opaque read of the block index keeps the
+// compiler from holding the 64-bit pointer in registers across the whole trace loop
+template <int kBlock>
+__device__ __forceinline__ unsigned long long* timeline_row(const TraceParams& P) {
+    unsigned cta;
+    asm volatile("mov.u32 %0, %%ctaid.x;" : "=r"(cta));
+    return P.timeline + 4ull * ((unsigned long long)cta * (kBlock / 32) + (threadIdx.x >> 5));
+}
 
 template <bool kConstBank, int kBlock, bool kCull = false>
 __device__ __forceinline__ void trace_body(const TraceParams& P, const float4* __restrict__ pairs,
                                            const float4* __restrict__ gather, float* __restrict__ stage_mem,
-                                           const float4* __restrict__ boxes = nullptr, float cull_r2 = 0.0f) {
-    float* const stage = stage_mem + (threadIdx.x >> 5) * kStageFloats;
-    unsigned long long* const tl =
-        P.timeline ? P.timeline + 4ull * ((unsigned long long)blockIdx.x * (kBlock / 32) + (threadIdx.x >> 5)) : nullptr;
-    if (tl && (threadIdx.x & 31u) == 0u) tl[0] = globaltimer_ns();
+                                           const float4* __restrict__ boxes = nullptr, float cull_r2 = 0.0f,
+                                           int split_max = 0) {
+    float* const stage = stage_mem + (threadIdx.x >> 5) * (kCull ? kCullStageFloats : kStageFloats);
+    if (P.timeline && (threadIdx.x & 31u) == 0u) timeline_row<kBlock>(P)[0] = globaltimer_ns();
     // material rows are touched once per HIT (not per test): they stay in global memory / L1
     const float4* s_aux = P.aux;
     const float4* s_alb = P.albedo;
@@ -462,7 +551,7 @@ __device__ __forceinline__ void trace_body(const TraceParams& P, const float4* _
                     // visible to ptxas (uniform branches keep the warp provably converged)
                     if (__any_sync(0xFFFFFFFFu, cid >= P.n_chunks)) {
                         exhausted = true;
-                        if (tl && lane == 0u) tl[1] = globaltimer_ns();
+                        if (P.timeline && lane == 0u) timeline_row<kBlock>(P)[1] = globaltimer_ns();
                         break;
                     }
                     // (the chunk is committed only behind the `continue`: written the other way round ptxas no
@@ -536,14 +625,16 @@ __device__ __forceinline__ void trace_body(const TraceParams& P, const float4* _
         float ta = 0.f, tb = 0.f;
         int ia = -1, ib = -1;
         sweep2<kConstBank, false, kCull>(pairs, gather, P.n_pad, cam.tmin, cam.tmax, A.path, B.path, ta, ia, tb, ib,
-                                         boxes, cull_r2, kCull ? P.orig : nullptr);
+                                         boxes, cull_r2, kCull ? P.orig : nullptr, P.wexp, split_max,
+                                         reinterpret_cast<float4*>(stage));
         if (A.alive) finish_or_continue(P, gather, s_aux, s_alb, A, ta, ia);
         if (B.alive) finish_or_continue(P, gather, s_aux, s_alb, B, tb, ib);
         // explicit reconvergence point: with it ptxas proves the loop top converged (no BRA.DIV before
         // the votes) and keeps the sweep's addressing / constant-bank operands on the uniform datapath
         __syncwarp();
     }
-    if (tl && lane == 0u) {
+    if (P.timeline && lane == 0u) {
+        unsigned long long* const tl = timeline_row<kBlock>(P);
         unsigned smid;
         asm volatile("mov.u32 %0, %smid;" : "=r"(smid));
         tl[2] = globaltimer_ns(), tl[3] = smid;
@@ -818,8 +909,8 @@ __global__ void __launch_bounds__(kBlock, kMinBlocks) trace_kernel_const(const _
 // can reach is skipped.  The host takes it for scenes whose blocks are compact against the scene's extent.
 template <int kBlock, int kMinBlocks>
 __global__ void __launch_bounds__(kBlock, kMinBlocks) trace_kernel_const_cull(const __grid_constant__ TraceParamsConst C) {
-    __shared__ float stage[(kBlock / 32) * kStageFloats];
-    trace_body<true, kBlock, true>(C.p, C.pairs, C.p.geom, stage, C.boxes, C.cull_r2);
+    __shared__ __align__(16) float stage[(kBlock / 32) * kCullStageFloats];
+    trace_body<true, kBlock, true>(C.p, C.pairs, C.p.geom, stage, C.boxes, C.cull_r2, C.split_max);
 }
 
 // K1b: geometry staged into shared memory by 1-D TMA bulk copies (cp.async.bulk + mbarrier): scenes

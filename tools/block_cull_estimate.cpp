@@ -7,7 +7,10 @@
 // executes when it skips every block whose padded bound none of its live paths can reach over (0, closest].
 // Three block orders (the reference's; the spatial regrouping the culled kernel sweeps, sweep_order in
 // csrc/rtz_api.cu; the same blocks swept near to far from the camera) times two bounds (axis-aligned boxes,
-// bounding spheres).
+// bounding spheres).  With boxes on the regrouped order it also reports what each path would execute if it swept
+// only the blocks its own bound admits, how many of the warp's paths reach each swept culled block, and the cost
+// of sweeping a block sphere-parallel over its k reaching paths (min(64, a k + 2) path-units against the packed
+// sweep's 64, for a = 1.5 / 2 / 3: sweep2's split branch).
 //
 // Build and run (a few seconds per 100 pixels on one core):
 //   g++ -O2 -std=c++17 -ffp-contract=off -mfma -pthread -o /tmp/bce tools/block_cull_estimate.cpp oracle/rtz_oracle.cpp
@@ -138,7 +141,13 @@ void kd_order(const std::vector<MSphere>& ms, std::vector<int>& idx, int first, 
 
 struct Result {
     double executed = 0, total = 0, bound_tests = 0, iters = 0;
+    double per_path = 0;             // tests if each live path swept only block 0 and the blocks its own bound admits
+    double split[3] = {0, 0, 0};     // tests-equivalent of the split sweep for kSplitCost[j] (see main)
+    double hist[65] = {};            // swept culled blocks by the number of paths of the warp that reach them
+    double always = 0;               // tests of the blocks swept without a bound test (block 0)
 };
+// cost of a sphere-parallel pass per reaching path, in units of one path of the packed sweep
+constexpr double kSplitCost[3] = {1.5, 2.0, 3.0};
 
 // one warp runs all chunks in sequence (each chunk = the samples of one pixel)
 // `seq`: the order in which the blocks are swept (block 0 first)
@@ -181,14 +190,26 @@ Result replay(const std::vector<std::vector<std::vector<Seg>>>& chunks, const st
             const int cnt = std::min(32, n_pad - 32 * b);
             R.total += cnt;
             bool need = bounds[b].all;
+            int reach = 0;  // paths whose own bound admits the block (every live path for block 0)
             if (!need) {
                 R.bound_tests += 1;
-                for (int s = 0; s < 64 && !need; ++s) {
+                for (int s = 0; s < 64; ++s) {
                     if (!slot[s].alive) continue;
                     const Path& p = chunks[slot[s].chunk][slot[s].sample][slot[s].seg].p;
-                    need = kind == 0 ? box_needed(bounds[b], p, closest[s]) : sphere_needed(bounds[b], p, closest[s]);
+                    reach += kind == 0 ? box_needed(bounds[b], p, closest[s]) : sphere_needed(bounds[b], p, closest[s]);
                 }
+                need = reach > 0;
+                if (need) R.hist[reach] += 1;
+                // split sweep: a sphere-parallel pass costs a * k + 2 path-units (k broadcast rays, the lane's sphere
+                // loads and the mask conversion), the packed sweep 64; the kernel takes the cheaper of the two
+                for (int j = 0; j < 3; ++j)
+                    if (need) R.split[j] += cnt * std::min(64.0, kSplitCost[j] * reach + 2.0) / 64.0;
+            } else {
+                reach = live;
+                R.always += cnt;
+                for (int j = 0; j < 3; ++j) R.split[j] += cnt;
             }
+            R.per_path += cnt * reach / 64.0;
             for (int s = 0; s < 64; ++s) {
                 if (!slot[s].alive) continue;
                 if (!need && rb[s][b] < closest[s]) {
@@ -298,6 +319,24 @@ int main(int argc, char** argv) {
                 std::printf("   c_b=%.1f: x%.3f (%.1f%% less time)", cb, 1.0 / rel, 100.0 * (1.0 - rel));
             }
             std::printf("\n");
+            if (kind != 0 || o == 0) continue;
+            // boxes on the regrouped order: what sweeping each path's own blocks would execute, how many paths reach
+            // the culled blocks that are swept, and the split sweep's cost model
+            std::printf("%-31s %9.1f%%\n", "  per path (own box_reach)", 100.0 * R.per_path / R.total);
+            double swept = 0;
+            for (int k = 1; k <= 64; ++k) swept += R.hist[k];
+            std::printf("  paths reaching a swept culled block, cumulative share:");
+            double acc = 0;
+            for (int k = 1, c = 0; k <= 64; ++k) {
+                acc += R.hist[k];
+                const int marks[6] = {4, 8, 16, 24, 32, 48};
+                if (c < 6 && k == marks[c]) std::printf("  <=%d: %.0f%%", k, 100.0 * acc / swept), ++c;
+            }
+            std::printf("\n");
+            for (int j = 0; j < 3; ++j)
+                std::printf("  split sweep, a = %.1f: %9.1f%% of brute force, culled blocks at %.2f of the packed sweep\n",
+                            kSplitCost[j], 100.0 * R.split[j] / R.total,
+                            (R.split[j] - R.always) / (R.executed - R.always));
         }
     }
     return 0;
