@@ -195,6 +195,27 @@ uint64_t rtz_shard_pixels(uint64_t width, uint64_t height, const rtz_shard* shar
 int32_t rtz_render_resident(rtz_context* ctx, const rtz_camera* camera, const rtz_shard* shard,
                             uint8_t* d_rgb_out, rtz_stats* stats_out);
 
+/* rtz_render_resident, plus the linear colour before gamma/quantisation as f32 (3 per pixel, same layout as
+ * d_rgb_out: compact tiles for a shard, row-major for the whole frame): (float) of rtz_render_linear's value.
+ * The bytes are rtz_render_resident's.  d_linear_out (DEVICE) is required; the legacy modes are refused. */
+int32_t rtz_render_resident_linear(rtz_context* ctx, const rtz_camera* camera, const rtz_shard* shard,
+                                   uint8_t* d_rgb_out, float* d_linear_out, rtz_stats* stats_out);
+
+/* First-hit guides of the frame's camera rays, samples 0 .. guide_samples-1 of every pixel (whole frame,
+ * row-major, top row first, 3 f32 per pixel each).  Either output may be NULL, not both.
+ * For each sample the ray is the frame's own camera ray (the counter-based RNG at (seed, pixel, sample, 0)) and
+ * its closest hit the render's first hit.  albedo: the sphere's albedo (lambertian, metal), (1,1,1) (dielectric),
+ * the sky colour the render returns for that ray on a miss; normal: the unit normal against the ray, (0,0,0) on a
+ * miss.  Per pixel, the samples' f32 values are added in ascending sample order from +0 and divided by
+ * guide_samples once; normals are not renormalised.  Guides do not depend on bounce_max, and RTZ_MODE_PATH_BVH
+ * gives the buffers of RTZ_MODE_PATH.  RTZ_ERR_BAD_ARG for a legacy mode, has_seed == 0 (an OS-drawn seed would
+ * give other rays than the frame's), guide_samples == 0 or > samples_per_pixel, both outputs NULL, or more than
+ * 2^31 - 1 work items (pixels for guide_samples >= 64).
+ * stats: samples = segments = width*height*guide_samples, sphere_tests, kernel_launches, trace_ms = total_ms
+ * (the guide kernel), seed_used; the rest 0.  Blocks like rtz_render_resident. */
+int32_t rtz_render_guides(rtz_context* ctx, const rtz_camera* camera, uint64_t guide_samples,
+                          float* d_albedo_out, float* d_normal_out, rtz_stats* stats_out);
+
 /* Rank-0 side of the tile gather: `d_gathered` holds `world` compact buffers of equal
  * size (rtz_shard_pixels of rank 0, the largest) back to back, as an all-gather /
  * gather leaves them; writes the plain row-major image to `d_rgb_out` (device). */

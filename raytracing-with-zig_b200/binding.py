@@ -75,6 +75,9 @@ SIGNATURES = {
     "rtz_scene_generate": (_i32, [_vp, _i32, _u64, _u64, C.POINTER(rtz_sphere), _u64, C.POINTER(_u64), C.POINTER(_u64)]),
     "rtz_shard_pixels": (_u64, [_u64, _u64, C.POINTER(rtz_shard)]),
     "rtz_render_resident": (_i32, [_vp, C.POINTER(rtz_camera), C.POINTER(rtz_shard), _vp, C.POINTER(rtz_stats)]),
+    "rtz_render_resident_linear": (_i32, [_vp, C.POINTER(rtz_camera), C.POINTER(rtz_shard), _vp, _vp,
+                                          C.POINTER(rtz_stats)]),
+    "rtz_render_guides": (_i32, [_vp, C.POINTER(rtz_camera), _u64, _vp, _vp, C.POINTER(rtz_stats)]),
     "rtz_deinterleave": (_i32, [_vp, _u64, _u64, _u32, _u32, _u32, _vp, _vp]),
     "rtz_multi_create": (_i32, [_i32, C.POINTER(_i32), _u32, _u32, _i32, C.POINTER(_vp)]),
     "rtz_multi_destroy": (_i32, [_vp]),

@@ -24,6 +24,7 @@
 
 #include "../../include/rtz.h"
 #include "rtz_kernels.cuh"
+#include "rtz_guides.cuh"
 #include "rtz_bvh.cuh"
 #include "rtz_scene.cuh"
 
@@ -231,6 +232,7 @@ int32_t ensure_bvh(rtz_context* c);
 struct FrameTarget {
     uint8_t* d_rgb = nullptr;
     double* d_linear = nullptr;
+    float* d_linear32 = nullptr;
     uint8_t* image = nullptr;
 };
 
@@ -393,7 +395,7 @@ int32_t enqueue_path(rtz_context* ctx, const rtz_camera* cam, const rtz::ShardGe
             ctx->accum.p, sg, (uint32_t)cam->width, (uint32_t)cam->height, cam->pixel_samples_scale, out.image);
     else
         rtz::resolve_kernel<<<(unsigned)((n3 + 255) / 256), 256, 0, ctx->stream>>>(
-            ctx->accum.p, n_local_pixels, cam->pixel_samples_scale, out.d_rgb, out.d_linear);
+            ctx->accum.p, n_local_pixels, cam->pixel_samples_scale, out.d_rgb, out.d_linear, out.d_linear32);
     RTZ_CUDA(cudaGetLastError());
     RTZ_CUDA(cudaEventRecord(ctx->ev[3], ctx->stream));
     RTZ_CUDA(cudaMemcpyAsync(ctx->h_counters, ctx->counters.p, 8 * sizeof(unsigned long long), cudaMemcpyDeviceToHost,
@@ -442,9 +444,9 @@ int32_t collect_path(rtz_context* ctx, const rtz_camera* cam, const rtz::ShardGe
 }
 
 int32_t render_path(rtz_context* ctx, const rtz_camera* cam, const rtz::ShardGeom& sg, uint8_t* d_rgb,
-                    double* d_linear, rtz_stats* st, uint64_t seed) {
+                    double* d_linear, rtz_stats* st, uint64_t seed, float* d_linear32 = nullptr) {
     FrameTarget out;
-    out.d_rgb = d_rgb, out.d_linear = d_linear;
+    out.d_rgb = d_rgb, out.d_linear = d_linear, out.d_linear32 = d_linear32;
     const int32_t rc = enqueue_path(ctx, cam, sg, out, seed);
     if (rc != RTZ_OK) return rc;
     return collect_path(ctx, cam, sg, st, seed);
@@ -888,7 +890,7 @@ uint64_t rtz_shard_pixels(uint64_t W, uint64_t H, const rtz_shard* s) {
 }
 
 static int32_t render_resident_impl(rtz_context* c, const rtz_camera* cam, const rtz_shard* shard, uint8_t* d_rgb,
-                                    double* d_linear, rtz_stats* st) {
+                                    double* d_linear, rtz_stats* st, float* d_linear32 = nullptr) {
     if (!c || !d_rgb) return RTZ_ERR_BAD_ARG;
     int32_t rc = check_camera(cam);
     if (rc != RTZ_OK) return rc;
@@ -896,18 +898,85 @@ static int32_t render_resident_impl(rtz_context* c, const rtz_camera* cam, const
     RTZ_CUDA(cudaSetDevice(c->device));
     if (cam->mode != RTZ_MODE_PATH && cam->mode != RTZ_MODE_PATH_BVH) {
         if (shard && shard->world != 1) return RTZ_ERR_BAD_ARG;  // the legacy modes are whole-frame only
+        if (d_linear32) return RTZ_ERR_BAD_ARG;                   // ... and report their linear colour in f64 only
         return render_legacy(c, cam, d_rgb, d_linear, st);
     }
     rtz::ShardGeom g;
     rc = shard_geom(cam->width, cam->height, shard, g);
     if (rc != RTZ_OK) return rc;
     const uint64_t seed = cam->has_seed ? cam->seed : os_seed();
-    return render_path(c, cam, g, d_rgb, d_linear, st, seed);
+    return render_path(c, cam, g, d_rgb, d_linear, st, seed, d_linear32);
 }
 
 int32_t rtz_render_resident(rtz_context* c, const rtz_camera* cam, const rtz_shard* shard, uint8_t* d_rgb,
                             rtz_stats* st) {
     return render_resident_impl(c, cam, shard, d_rgb, nullptr, st);
+}
+
+int32_t rtz_render_resident_linear(rtz_context* c, const rtz_camera* cam, const rtz_shard* shard, uint8_t* d_rgb,
+                                   float* d_linear, rtz_stats* st) {
+    if (!d_linear) return RTZ_ERR_BAD_ARG;
+    return render_resident_impl(c, cam, shard, d_rgb, nullptr, st, d_linear);
+}
+
+int32_t rtz_render_guides(rtz_context* c, const rtz_camera* cam, uint64_t guide_samples, float* d_albedo,
+                          float* d_normal, rtz_stats* st) {
+    if (!c) return RTZ_ERR_BAD_ARG;
+    int32_t rc = check_camera(cam);
+    if (rc != RTZ_OK) return rc;
+    if (cam->mode != RTZ_MODE_PATH && cam->mode != RTZ_MODE_PATH_BVH) return RTZ_ERR_BAD_ARG;
+    // the guides belong to a frame: its rays are keyed by the frame's seed, which an OS-drawn seed would not repeat
+    if (!cam->has_seed || guide_samples == 0 || guide_samples > cam->samples_per_pixel) return RTZ_ERR_BAD_ARG;
+    if (!d_albedo && !d_normal) return RTZ_ERR_BAD_ARG;
+    DeviceGuard guard;
+    RTZ_CUDA(cudaSetDevice(c->device));
+    const uint64_t n_pix = cam->width * cam->height;
+    rtz::GuideParams P{};
+    P.cam = to_dev_camera(*cam, cam->seed);
+    P.pairs = c->pairs.p, P.geom = c->geom.p, P.aux = c->aux.p, P.albedo = c->albedo.p, P.wexp = c->wexp.p;
+    P.orig = nullptr;
+    P.n_pad = c->n_pad;
+    P.g = (uint32_t)guide_samples;
+    P.pix_per_item = guide_samples >= 64 ? 1u : (uint32_t)(64 / guide_samples);
+    P.n_items = (uint32_t)((n_pix + P.pix_per_item - 1) / P.pix_per_item);
+    if (P.n_items > 0x7FFFFFFFu) return RTZ_ERR_BAD_ARG;  // one block (warp) per item: the grid's x limit
+    P.albedo_out = d_albedo, P.normal_out = d_normal;
+    const unsigned blocks = P.n_items;
+    // every mode sweeps by brute force here (the BVH finds the same hits), on the rows the render's sweep reads
+    RTZ_CUDA(cudaEventRecord(c->ev[0], c->stream));
+    if (c->n_pad <= rtz::kMaxConstSpheres && c->geo_const) {
+        static thread_local rtz::GuideParamsConst C;  // 8.5 KiB: keep it off the stack
+        if (c->cull) {
+            P.geom = c->rg_geom.p, P.aux = c->rg_aux.p, P.albedo = c->rg_albedo.p, P.wexp = c->rg_wexp.p;
+            P.orig = c->rg_orig.p, P.pairs = nullptr;
+            std::memcpy(C.pairs, c->h_rg_pairs.data(), (size_t)c->n_pad * sizeof(float4));
+            std::memcpy(C.boxes, c->h_boxes.data(), c->h_boxes.size() * sizeof(float4));
+            C.cull_r2 = c->cull_r2;
+            C.split_max = rtz::kSplitMax;
+        } else {
+            std::memcpy(C.pairs, c->h_pairs.data(), (size_t)c->n_pad * sizeof(float4));
+        }
+        C.p = P;
+        if (c->cull)
+            rtz::guide_kernel_const<true><<<blocks, 32, 0, c->stream>>>(C);
+        else
+            rtz::guide_kernel_const<false><<<blocks, 32, 0, c->stream>>>(C);
+    } else {
+        rtz::guide_kernel_global<<<blocks, 32, 0, c->stream>>>(P);
+    }
+    RTZ_CUDA(cudaGetLastError());
+    RTZ_CUDA(cudaEventRecord(c->ev[1], c->stream));
+    RTZ_CUDA(cudaStreamSynchronize(c->stream));
+    if (st) {
+        std::memset(st, 0, sizeof(*st));
+        st->samples = st->segments = n_pix * guide_samples;
+        st->sphere_tests = st->segments * (uint64_t)c->n_spheres;
+        st->kernel_launches = 1;
+        float ms = 0;
+        cudaEventElapsedTime(&ms, c->ev[0], c->ev[1]), st->trace_ms = st->total_ms = ms;
+        st->seed_used = cam->seed;
+    }
+    return RTZ_OK;
 }
 
 int32_t rtz_deinterleave(rtz_context* c, uint64_t W, uint64_t H, uint32_t world, uint32_t tw, uint32_t th,

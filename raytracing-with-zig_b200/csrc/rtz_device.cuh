@@ -256,6 +256,17 @@ __device__ __forceinline__ void sweep_rows(const float4* __restrict__ geo, const
     best_out = best;
 }
 
+// HitRecord (src/sphere.zig:44-53) of a hit at distance t on sphere g = {cx, cy, cz, -r^2} with inv_r = 1/r: the point
+// and the normal, flipped against the ray on a back face (shade forms the same expressions); returns HitRecord.front
+__device__ __forceinline__ bool hit_record(const float4 g, float inv_r, const Path& p, float t, float& px, float& py,
+                                           float& pz, float& nx, float& ny, float& nz) {
+    px = fmaf(t, p.dx, p.ox), py = fmaf(t, p.dy, p.oy), pz = fmaf(t, p.dz, p.oz);
+    nx = (px - g.x) * inv_r, ny = (py - g.y) * inv_r, nz = (pz - g.z) * inv_r;
+    const bool front = fmaf(p.dz, nz, fmaf(p.dy, ny, p.dx * nx)) < 0.0f;
+    if (!front) nx = -nx, ny = -ny, nz = -nz;
+    return front;
+}
+
 // ---------------------------------------------------------------------------------------------
 // Shading of one finished segment.  Returns true when the sample is finished; then (sr,sg,sb)
 // is its colour.  `term` reports why: 0 sky, 1 absorbed, 2 depth cap.

@@ -1,0 +1,154 @@
+// rtz_guides.cuh — first-hit guide buffers for a denoiser (sm_100a): the albedo and the normal that the camera rays
+// of a frame see at their closest hit.
+//
+// The guide kernel does not share a launch with the render.  It regenerates the frame's camera rays (camera_ray with
+// the key (seed, j*W + i, s), bounce 0: the render's first ray of sample s, bit for bit) and finds their closest hit
+// with the render's own sweep (sweep2, unchanged), so its hits are the ones the render's first world.hit returns:
+// the (t, original index) minimum over Scene.interval, with the same gate and roots.
+//
+// Per ray, six f32 values:
+//   albedo  hit: the sphere's albedo for lambertian and metal (the attenuation scatter applies), (1, 1, 1) for
+//                dielectric; miss: the sky colour of shade's miss branch at throughput 1, which is what the render
+//                returns for that ray (so colour / albedo = 1 on the sky);
+//   normal  hit: the HitRecord normal (p - c) * (1/r), flipped against the ray on a back face; miss: (0, 0, 0).
+// Per pixel and channel, the values of samples 0 .. g-1 are added in ascending sample order, each in f32 to a running
+// sum that starts at +0, and the sum is divided by (float)g once.  Normals are averaged, not renormalised.  A CPU
+// restatement of this order (tests/guide_mirror.cpp) must agree bit for bit.
+//
+// Work: a warp sweeps 64 camera rays at a time, two per lane, as the render does.  Its work item is whole pixels:
+// floor(64 / g) of them for g < 64 (so g = 1 still fills all 64 slots), one for g >= 64, swept in rounds of 64 of its
+// samples.  A pixel never spans two warps, so its sums keep their order: after each sweep the six values of every ray
+// are staged in shared memory and each (pixel, channel) is folded by one lane.
+#pragma once
+#include "rtz_kernels.cuh"
+
+namespace rtz {
+
+struct GuideParams {
+    DevCamera cam;
+    const float4* pairs;     // sweep layout in global memory (guide_kernel_global; the constant-bank kernel has its own)
+    const float4* geom;      // per-lane rows {cx, cy, cz, -r^2}: candidate roots, hit records
+    const float4* aux;       // {r, 1/r, fuzz|ior, type}
+    const float4* albedo;    // {r, g, b, 1/ior}
+    const float* wexp;       // w of the pair layout as a plain row
+    const int* orig;         // culled sweep: slot -> index in the caller's list (ties in t), else null
+    int n_pad;
+    uint32_t g;              // guide samples per pixel
+    uint32_t pix_per_item;   // whole pixels per warp: floor(64 / g), 1 for g >= 64
+    uint32_t n_items;
+    float* albedo_out;       // [W*H*3] or null
+    float* normal_out;       // [W*H*3] or null
+};
+
+// the constant-bank form: the rows the render's constant-bank kernels sweep (plain, or regrouped with their boxes)
+struct GuideParamsConst {
+    GuideParams p;
+    float4 pairs[kMaxConstSpheres];
+    float4 boxes[2 * (kMaxConstSpheres / 32)];
+    float cull_r2;
+    int split_max;
+};
+
+constexpr int kGuideStageFloats = 6 * 64;  // per warp: the six values of 64 rays
+
+// camera ray `r` of a work item (pixel pix0 + r / g, sample r % g); a slot past the item's last ray takes ray 0 of
+// the item and its result is not folded
+__device__ __forceinline__ void guide_ray(const DevCamera& cam, uint32_t g, uint32_t pix0, uint32_t r, uint32_t rays,
+                                          Path& p) {
+    if (r >= rays) r = 0;
+    const uint32_t pl = r / g, s = r - pl * g;
+    const uint32_t pixel = pix0 + pl;
+    const uint32_t y = pixel / cam.width, x = pixel - y * cam.width;
+    camera_ray(cam, RngKey{cam.key0, cam.key1, pixel, s}, x, y, p);
+}
+
+// the six values of one swept ray into its column `j` of the staging rows (row c = channel c: albedo rgb, normal xyz)
+__device__ __forceinline__ void guide_values(const GuideParams& P, const Path& p, float t, int best, float* stage,
+                                             uint32_t j) {
+    float v[6];
+    if (best < 0) {
+        // shade's sky (src/camera.zig:171-177) at throughput 1
+        const float a = 0.5f * (p.dy + 1.0f);
+        const float w = 1.0f - a;
+        v[0] = fmaf(a, 0.5f, w), v[1] = fmaf(a, 0.7f, w), v[2] = fmaf(a, 1.0f, w);
+        v[3] = v[4] = v[5] = 0.0f;
+    } else {
+        const float4 ax = __ldg(P.aux + best);
+        float px, py, pz;
+        hit_record(P.geom[best], ax.y, p, t, px, py, pz, v[3], v[4], v[5]);
+        if (__float_as_int(ax.w) == kDielectric) {
+            v[0] = v[1] = v[2] = 1.0f;
+        } else {
+            const float4 al = __ldg(P.albedo + best);
+            v[0] = al.x, v[1] = al.y, v[2] = al.z;
+        }
+    }
+#pragma unroll
+    for (int c = 0; c < 6; ++c) stage[c * 64 + j] = v[c];
+}
+
+__device__ __forceinline__ void guide_store(const GuideParams& P, uint32_t pixel, uint32_t c, float value) {
+    float* out = c < 3 ? P.albedo_out : P.normal_out;
+    if (out) out[3ull * pixel + (c < 3 ? c : c - 3)] = value;
+}
+
+template <bool kConstBank, bool kCull>
+__device__ __forceinline__ void guide_body(const GuideParams& P, const float4* __restrict__ pairs,
+                                           float* __restrict__ stage_mem, const float4* __restrict__ boxes = nullptr,
+                                           float cull_r2 = 0.0f, int split_max = 0) {
+    float* const stage = stage_mem;
+    // one warp per block, so that the work item is visibly warp-uniform to ptxas: with the item derived from the warp
+    // index inside a wider block, it guards the sweep's votes with divergent-branch checks (BRA.DIV)
+    const uint32_t item = blockIdx.x;
+    const unsigned lane = threadIdx.x & 31u;
+    const DevCamera& cam = P.cam;
+    const uint32_t g = P.g;
+    const uint32_t pix0 = item * P.pix_per_item;
+    const uint32_t n_here = min(P.pix_per_item, cam.width * cam.height - pix0);  // the last item may hold fewer
+    const uint32_t rays = n_here * g;
+    float acc = 0.0f;  // g >= 64: lane c < 6 holds the running sum of channel c of the item's one pixel
+    for (uint32_t r0 = 0; r0 < rays; r0 += 64) {
+        Path a, b;
+        guide_ray(cam, g, pix0, r0 + lane, rays, a);
+        guide_ray(cam, g, pix0, r0 + 32 + lane, rays, b);
+        __syncwarp();  // converged before the sweep's votes
+        float ta = 0.f, tb = 0.f;
+        int ia = -1, ib = -1;
+        sweep2<kConstBank, false, kCull>(pairs, P.geom, P.n_pad, cam.tmin, cam.tmax, a, b, ta, ia, tb, ib, boxes, cull_r2,
+                                         P.orig, P.wexp, split_max, reinterpret_cast<float4*>(stage));
+        __syncwarp();  // the culled sweep reads its staging rows (the same memory) until it returns
+        guide_values(P, a, ta, ia, stage, lane);
+        guide_values(P, b, tb, ib, stage, 32 + lane);
+        __syncwarp();
+        if (g < 64) {  // one round: fold every (pixel, channel) of the item, samples in ascending order
+            for (uint32_t q = lane; q < 6 * n_here; q += 32) {
+                const uint32_t pl = q / 6, c = q - 6 * pl;
+                const float* row = stage + c * 64 + pl * g;
+                float sum = 0.0f;
+                for (uint32_t s = 0; s < g; ++s) sum += row[s];
+                guide_store(P, pix0 + pl, c, sum / (float)g);
+            }
+        } else if (lane < 6) {
+            const uint32_t m = min(64u, rays - r0);
+            for (uint32_t s = 0; s < m; ++s) acc += stage[lane * 64 + s];
+        }
+        __syncwarp();  // the next round rewrites the rows
+    }
+    if (g >= 64 && lane < 6) guide_store(P, pix0, lane, acc / (float)g);
+}
+
+// Scenes the render sweeps from the constant bank (n_pad <= kMaxConstSpheres): the same rows, through the same
+// uniform loads; kCull = the culled kernel's regrouped rows, boxes and sphere-parallel split.
+template <bool kCull>
+__global__ void __launch_bounds__(32, 24) guide_kernel_const(const __grid_constant__ GuideParamsConst C) {
+    __shared__ __align__(16) float stage[kCull ? kCullStageFloats : kGuideStageFloats];
+    guide_body<true, kCull>(C.p, C.pairs, stage, C.boxes, C.cull_r2, C.split_max);
+}
+
+// Larger scenes: the plain pair rows from global memory (L1 / L2, warp-uniform addresses).
+__global__ void __launch_bounds__(32, 24) guide_kernel_global(const __grid_constant__ GuideParams P) {
+    __shared__ __align__(16) float stage[kGuideStageFloats];
+    guide_body<false, false>(P, P.pairs, stage);
+}
+
+}  // namespace rtz

@@ -1594,13 +1594,15 @@ __device__ __forceinline__ uint8_t to_byte(double lin) {
     return (uint8_t)(256.0 * g);
 }
 
+// `linear` / `linear32` (optional): the linear colour before gamma and quantisation, in f64 and rounded once to f32
 __global__ void resolve_kernel(const unsigned long long* __restrict__ accum, uint64_t n_pixels, double scale,
-                               uint8_t* __restrict__ rgb, double* __restrict__ linear) {
+                               uint8_t* __restrict__ rgb, double* __restrict__ linear, float* __restrict__ linear32) {
     const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;  // one thread per channel
     if (i >= 3 * n_pixels) return;
     const double lin = ((double)accum[i] * 0x1p-32) * scale;
     rgb[i] = to_byte(lin);
     if (linear) linear[i] = lin;
+    if (linear32) linear32[i] = (float)lin;
 }
 
 // K3 fused with the multi-GPU tile exchange (rtz_multi_*, RTZ_GATHER_P2P): the same resolve, but every channel
@@ -1722,12 +1724,9 @@ __global__ void probe_hits_kernel(const float4* geom, const float4* pairs, const
     sweep_rows(geom, pairs, 0, n_pad, p, tmin, tmax, t, best);
     rtz_ray_hit h = {best, 0, t, p.len, {0.f, 0.f, 0.f}, {0.f, 0.f, 0.f}};
     if (best >= 0) {
-        const float gx = geom[best].x, gy = geom[best].y, gz = geom[best].z;
-        const float px = fmaf(t, p.dx, p.ox), py = fmaf(t, p.dy, p.oy), pz = fmaf(t, p.dz, p.oz);
-        float nx = (px - gx) * aux[best].y, ny = (py - gy) * aux[best].y, nz = (pz - gz) * aux[best].y;
-        const bool front = fmaf(p.dz, nz, fmaf(p.dy, ny, p.dx * nx)) < 0.f;
-        if (!front) nx = -nx, ny = -ny, nz = -nz;
-        h.front = front, h.point[0] = px, h.point[1] = py, h.point[2] = pz, h.normal[0] = nx, h.normal[1] = ny, h.normal[2] = nz;
+        float px, py, pz, nx, ny, nz;
+        h.front = hit_record(geom[best], aux[best].y, p, t, px, py, pz, nx, ny, nz);
+        h.point[0] = px, h.point[1] = py, h.point[2] = pz, h.normal[0] = nx, h.normal[1] = ny, h.normal[2] = nz;
     }
     out[k] = h;
 }

@@ -108,6 +108,49 @@ class Renderer:
                                              C.c_void_p(out.data_ptr()), C.byref(st)))
         return out, st
 
+    def render_linear(self, camera, shard: B.rtz_shard | None = None, out=None, linear=None):
+        """`render`, plus the linear colour before gamma and quantisation (the noisy input of a denoiser) as a
+        float32 device tensor of the same shape; returns (uint8 tensor, float32 tensor, stats)."""
+        torch = self.torch
+        cam = _cast_camera(camera)
+        if shard is None:
+            shape = (int(cam.height), int(cam.width), 3)
+        else:
+            shape = (self.shard_pixels(cam.width, cam.height, shard), 3)
+        dev = f"cuda:{self.device}"
+        if out is None:
+            out = torch.empty(shape, dtype=torch.uint8, device=dev)
+        if linear is None:
+            linear = torch.empty(shape, dtype=torch.float32, device=dev)
+        for t, dt in ((out, torch.uint8), (linear, torch.float32)):
+            assert t.is_cuda and t.is_contiguous() and t.dtype == dt and tuple(t.shape) == shape, (t.shape, t.dtype)
+        st = B.rtz_stats()
+        self._order_after_torch()
+        B.check(self.lib.rtz_render_resident_linear(self._ctx, C.byref(cam),
+                                                    C.byref(shard) if shard is not None else None,
+                                                    C.c_void_p(out.data_ptr()), C.c_void_p(linear.data_ptr()),
+                                                    C.byref(st)))
+        return out, linear, st
+
+    def render_guides(self, camera, samples: int, albedo=None, normal=None):
+        """First-hit denoiser guides of the frame's camera rays, samples 0 .. samples-1 of every pixel (the camera
+        needs its seed): float32 [H, W, 3] device tensors (albedo, normal); returns (albedo, normal, stats)."""
+        torch = self.torch
+        cam = _cast_camera(camera)
+        shape = (int(cam.height), int(cam.width), 3)
+        dev = f"cuda:{self.device}"
+        if albedo is None:
+            albedo = torch.empty(shape, dtype=torch.float32, device=dev)
+        if normal is None:
+            normal = torch.empty(shape, dtype=torch.float32, device=dev)
+        for t in (albedo, normal):
+            assert t.is_cuda and t.is_contiguous() and t.dtype == torch.float32 and tuple(t.shape) == shape, (t.shape, t.dtype)
+        st = B.rtz_stats()
+        self._order_after_torch()
+        B.check(self.lib.rtz_render_guides(self._ctx, C.byref(cam), int(samples), C.c_void_p(albedo.data_ptr()),
+                                           C.c_void_p(normal.data_ptr()), C.byref(st)))
+        return albedo, normal, st
+
     def deinterleave(self, gathered, width: int, height: int, world: int, tile_w: int, tile_h: int, out=None):
         torch = self.torch
         if out is None:
