@@ -216,6 +216,47 @@ int32_t rtz_render_resident_linear(rtz_context* ctx, const rtz_camera* camera, c
 int32_t rtz_render_guides(rtz_context* ctx, const rtz_camera* camera, uint64_t guide_samples,
                           float* d_albedo_out, float* d_normal_out, rtz_stats* stats_out);
 
+/* ---- denoiser: edge-avoiding à-trous wavelet filter (Dammertz et al. 2010) over the linear colour, guided by the
+ * first-hit albedo and normal above ---------------------------------------------------------------------------
+ * Per pixel the colour is demodulated by the albedo (e = c / max(a, 2^-8)), filtered in `levels` passes of 5x5 taps
+ * at steps 1, 2, 4 ... with B3-spline weights times three edge-stopping factors E(x) = max(0, 1 - x/64)^64 of the
+ * squared differences of e (scaled by 4^k / sigma_color^2 at level k), of the normal (1 / sigma_normal^2) and of the
+ * albedo (1 / sigma_albedo^2), then remodulated; a tap at x >= 64 contributes nothing.  The bytes are Color.toRgb of
+ * the f32 result, as the resolve forms them.  IEEE f32 arithmetic in a fixed order (DESIGN.md §5 K7): the output is
+ * reproducible bit for bit.  The filter needs the whole frame: shards and multi-GPU frames are not supported. */
+typedef struct rtz_denoise_params {
+    uint32_t levels;       /* à-trous levels, step 2^k for k < levels; 0 = copy; <= 8                       */
+    uint32_t reserved;     /* must be 0                                                                     */
+    double sigma_color;    /* > 0, finite: edge scale of the demodulated colour at level 0                  */
+    double sigma_normal;   /* > 0, finite                                                                   */
+    double sigma_albedo;   /* > 0, finite                                                                   */
+} rtz_denoise_params;
+/* params NULL: levels 5, sigma_color 0.25, sigma_normal 0.25, sigma_albedo 0.25 */
+
+/* Whole frame, row-major, 3 f32 per pixel in each DEVICE buffer (d_color: rtz_render_resident_linear's linear
+ * colour; d_albedo / d_normal: rtz_render_guides' buffers); params NULL = the defaults above.  d_linear_out receives
+ * the denoised linear colour (3 f32 per pixel), d_rgb_out its bytes (3 per pixel); either may be NULL, not both.
+ * RTZ_ERR_BAD_ARG for a NULL context or input, both outputs NULL, an output that overlaps an input or the other
+ * output, a zero width or height or more than 2^31 - 1 pixels, levels > 8, reserved != 0, a sigma that is <= 0 or
+ * not finite, or a sigma_color so small that 4^(levels-1) / sigma_color^2 overflows f32.
+ * stats: kernel_launches and total_ms (CUDA events on the context's stream); the rest 0.  Blocks like
+ * rtz_render_resident. */
+int32_t rtz_denoise(rtz_context* ctx, uint64_t width, uint64_t height, const float* d_color, const float* d_albedo,
+                    const float* d_normal, const rtz_denoise_params* params, float* d_linear_out, uint8_t* d_rgb_out,
+                    rtz_stats* stats_out);
+
+/* rtz_render with host buffers, denoised: the linear colour of the frame (rtz_render_resident_linear), the guides of
+ * its samples 0 .. guide_samples-1 (rtz_render_guides) and rtz_denoise of the three, in the cached per-device context.
+ * guide_samples 0 = min(samples_per_pixel, 16).  has_seed == 0: ONE seed is drawn and keys both the render and the
+ * guides (stats_out->seed_used reports it).  rgb_out (3 bytes per pixel) and linear_out (3 f32 per pixel, the
+ * denoised linear colour) are HOST buffers; either may be NULL, not both.  RTZ_ERR_BAD_ARG as rtz_render and
+ * rtz_denoise, and for a legacy mode or guide_samples > samples_per_pixel.  The frame is whole: no shards, one GPU.
+ * stats: the render's counters as rtz_render reports them; kernel_launches counts every launch of the call and
+ * total_ms runs from the first launch to the denoised bytes. */
+int32_t rtz_render_denoised(const rtz_camera* camera, const rtz_sphere* spheres, uint64_t n_spheres,
+                            uint64_t guide_samples, const rtz_denoise_params* params, uint8_t* rgb_out,
+                            float* linear_out, rtz_stats* stats_out);
+
 /* Rank-0 side of the tile gather: `d_gathered` holds `world` compact buffers of equal
  * size (rtz_shard_pixels of rank 0, the largest) back to back, as an all-gather /
  * gather leaves them; writes the plain row-major image to `d_rgb_out` (device). */

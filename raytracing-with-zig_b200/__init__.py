@@ -5,9 +5,9 @@ Only what the hot path needs:
   host/            C++ mirror of the reference's Scene/Camera/Hittable/Material/PPM API above the ABI
   zig/             the Zig glue a reference maintainer would drop in (see INTEGRATION.md)
   binding.py       ctypes view of the ABI (raises when librtz.so is missing: no fallback)
-  renderer.py      resident renderer on torch device memory / streams; MultiRenderer = N GPUs in one process (rtz_multi)
+  renderer.py      resident renderer on torch device memory / streams (render, denoiser inputs, denoise); MultiRenderer = N GPUs in one process (rtz_multi)
   distributed.py   interleaved-tile sharding + NCCL gather (one process per GPU)
 """
-from .binding import RtzError, lib, rtz_camera, rtz_shard, rtz_sphere, rtz_stats  # noqa: F401
-from .renderer import MultiRenderer, Renderer, render_host, render_host_multi  # noqa: F401
+from .binding import RtzError, lib, rtz_camera, rtz_denoise_params, rtz_shard, rtz_sphere, rtz_stats  # noqa: F401
+from .renderer import MultiRenderer, Renderer, render_host, render_host_denoised, render_host_multi  # noqa: F401
 from .distributed import render_sharded, tile_index_map  # noqa: F401

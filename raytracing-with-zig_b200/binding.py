@@ -44,6 +44,12 @@ class rtz_stats(C.Structure):
                 ("gather_ms", C.c_double)]
 
 
+class rtz_denoise_params(C.Structure):
+    """à-trous levels and edge scales of rtz_denoise (include/rtz.h); NULL / None = the library's defaults."""
+    _fields_ = [("levels", C.c_uint32), ("reserved", C.c_uint32), ("sigma_color", C.c_double),
+                ("sigma_normal", C.c_double), ("sigma_albedo", C.c_double)]
+
+
 class rtz_hit(C.Structure):
     _fields_ = [("hit", C.c_int32), ("index", C.c_int32), ("front", C.c_int32), ("reserved", C.c_int32),
                 ("t", C.c_double), ("point", D3), ("normal", D3)]
@@ -78,6 +84,10 @@ SIGNATURES = {
     "rtz_render_resident_linear": (_i32, [_vp, C.POINTER(rtz_camera), C.POINTER(rtz_shard), _vp, _vp,
                                           C.POINTER(rtz_stats)]),
     "rtz_render_guides": (_i32, [_vp, C.POINTER(rtz_camera), _u64, _vp, _vp, C.POINTER(rtz_stats)]),
+    "rtz_denoise": (_i32, [_vp, _u64, _u64, _vp, _vp, _vp, C.POINTER(rtz_denoise_params), _vp, _vp,
+                           C.POINTER(rtz_stats)]),
+    "rtz_render_denoised": (_i32, [C.POINTER(rtz_camera), C.POINTER(rtz_sphere), _u64, _u64,
+                                   C.POINTER(rtz_denoise_params), _u8p, _f32p, C.POINTER(rtz_stats)]),
     "rtz_deinterleave": (_i32, [_vp, _u64, _u64, _u32, _u32, _u32, _vp, _vp]),
     "rtz_multi_create": (_i32, [_i32, C.POINTER(_i32), _u32, _u32, _i32, C.POINTER(_vp)]),
     "rtz_multi_destroy": (_i32, [_vp]),

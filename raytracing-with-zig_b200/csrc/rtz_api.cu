@@ -25,6 +25,7 @@
 #include "../../include/rtz.h"
 #include "rtz_kernels.cuh"
 #include "rtz_guides.cuh"
+#include "rtz_denoise.cuh"
 #include "rtz_bvh.cuh"
 #include "rtz_scene.cuh"
 
@@ -131,7 +132,12 @@ struct rtz_context {
     DevBuf<unsigned long long> timeline;  // RTZ_TIMELINE=1: per-warp {start, queue dry, done} stamps of the last frame
     DevBuf<uint8_t> rgb;                  // used by the host-buffer entry points
     DevBuf<double> linear;
-    cudaEvent_t ev[4] = {nullptr, nullptr, nullptr, nullptr};
+    // rtz_denoise: e (ping, pong), normal and albedo planes, one float4 per pixel each; rtz_render_denoised: its
+    // linear colour, albedo, normal and denoised linear colour (3 f32 per pixel each)
+    DevBuf<float4> denoise;
+    DevBuf<float> denoise_io;
+    // [0..3] a frame's phases, [4..5] the span of rtz_render_denoised
+    cudaEvent_t ev[6] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
     unsigned long long* h_counters = nullptr;  // pinned
 };
 
@@ -476,6 +482,72 @@ int32_t render_legacy(rtz_context* ctx, const rtz_camera* cam, uint8_t* d_rgb, d
     return RTZ_OK;
 }
 
+// rtz_denoise_params, checked, as the f32 words the kernels and a CPU restatement use
+struct DenoiseConsts {
+    uint32_t levels;
+    float ic0, in, ia;  // 1 / sigma^2 of the colour (level 0), the normal, the albedo
+};
+
+int32_t denoise_consts(const rtz_denoise_params* prm, DenoiseConsts& k) {
+    rtz_denoise_params d{5, 0, 0.25, 0.25, 0.25};  // the defaults of include/rtz.h (DESIGN.md §5 K7)
+    if (prm) d = *prm;
+    if (d.levels > (uint32_t)rtz::kDenoiseMaxLevels || d.reserved != 0) return RTZ_ERR_BAD_ARG;
+    for (const double s : {d.sigma_color, d.sigma_normal, d.sigma_albedo})
+        if (!(s > 0.0) || !std::isfinite(s)) return RTZ_ERR_BAD_ARG;
+    k.levels = d.levels;
+    k.ic0 = (float)(1.0 / (d.sigma_color * d.sigma_color));
+    k.in = (float)(1.0 / (d.sigma_normal * d.sigma_normal));
+    k.ia = (float)(1.0 / (d.sigma_albedo * d.sigma_albedo));
+    float deepest = k.ic0;  // 4^(levels-1) / sigma_color^2: an infinite scale would make the centre tap's 0 * inf NaN
+    for (uint32_t l = 1; l < k.levels; ++l) deepest *= 4.0f;
+    if (!std::isfinite(deepest) || !std::isfinite(k.in) || !std::isfinite(k.ia)) return RTZ_ERR_BAD_ARG;
+    return RTZ_OK;
+}
+
+bool overlaps(const void* a, size_t na, const void* b, size_t nb) {
+    const uintptr_t x = (uintptr_t)a, y = (uintptr_t)b;
+    return a && b && x < y + nb && y < x + na;
+}
+
+// Enqueue the denoise of a whole W x H frame on the context's stream (K7): prepare, `levels` level passes ping-ponging
+// between the e planes, finish; `launches` receives the kernel count.  No host wait.
+int32_t enqueue_denoise(rtz_context* c, uint32_t W, uint32_t H, const float* color, const float* albedo,
+                        const float* normal, const DenoiseConsts& k, float* linear_out, uint8_t* rgb_out,
+                        uint64_t& launches) {
+    const uint64_t n_pix = (uint64_t)W * H;
+    const uint32_t tiles_x = (W + rtz::kDenoiseBlockX - 1) / rtz::kDenoiseBlockX;
+    const uint64_t tiles = (uint64_t)tiles_x * ((H + rtz::kDenoiseBlockY - 1) / rtz::kDenoiseBlockY);
+    const dim3 block(rtz::kDenoiseBlockX, rtz::kDenoiseBlockY);
+    const float4* e = nullptr;
+    launches = 1;
+    if (k.levels > 0) {
+        RTZ_CUDA(c->denoise.reserve(4 * n_pix));
+        float4* const planes[2] = {c->denoise.p, c->denoise.p + n_pix};
+        float4* const nrm = c->denoise.p + 2 * n_pix;
+        float4* const alb = c->denoise.p + 3 * n_pix;
+        rtz::denoise_prepare_kernel<<<(unsigned)tiles, block, 0, c->stream>>>(color, albedo, normal, planes[0], nrm, alb,
+                                                                              W, H, tiles_x);
+        RTZ_CUDA(cudaGetLastError());
+        rtz::DenoiseLevelParams P{};
+        P.nrm = nrm, P.alb = alb;
+        P.width = W, P.height = H, P.tiles_x = tiles_x;
+        P.ic = k.ic0, P.in = k.in, P.ia = k.ia;
+        for (uint32_t l = 0; l < k.levels; ++l) {
+            P.e_in = planes[l & 1], P.e_out = planes[(l + 1) & 1];
+            P.step = 1u << l;
+            rtz::denoise_level_kernel<<<(unsigned)tiles, block, 0, c->stream>>>(P);
+            RTZ_CUDA(cudaGetLastError());
+            P.ic *= 4.0f;  // sigma_color halves at each level; exact
+        }
+        e = planes[k.levels & 1];
+        launches += 1 + k.levels;
+    }
+    rtz::denoise_finish_kernel<<<(unsigned)tiles, block, 0, c->stream>>>(e, color, albedo, linear_out, rgb_out, W, H,
+                                                                         tiles_x);
+    RTZ_CUDA(cudaGetLastError());
+    return RTZ_OK;
+}
+
 struct ScopedCtx {  // context for the one-shot entry points
     rtz_context* c = nullptr;
     ~ScopedCtx() {
@@ -571,6 +643,7 @@ int32_t rtz_context_destroy(rtz_context* c) {
     c->accum.release(), c->counters.release(), c->rgb.release(), c->linear.release(), c->timeline.release(), c->pool.release();
     c->bvh_nodes.release(), c->bvh_order.release(), c->wexp.release();
     c->rg_geom.release(), c->rg_aux.release(), c->rg_albedo.release(), c->rg_wexp.release(), c->rg_orig.release();
+    c->denoise.release(), c->denoise_io.release();
     for (auto& e : c->ev)
         if (e) cudaEventDestroy(e);
     if (c->h_counters) cudaFreeHost(c->h_counters);
@@ -979,6 +1052,35 @@ int32_t rtz_render_guides(rtz_context* c, const rtz_camera* cam, uint64_t guide_
     return RTZ_OK;
 }
 
+int32_t rtz_denoise(rtz_context* c, uint64_t W, uint64_t H, const float* d_color, const float* d_albedo,
+                    const float* d_normal, const rtz_denoise_params* prm, float* d_linear, uint8_t* d_rgb,
+                    rtz_stats* st) {
+    if (!c || !d_color || !d_albedo || !d_normal || (!d_linear && !d_rgb)) return RTZ_ERR_BAD_ARG;
+    if (W == 0 || H == 0 || W > 0x7FFFFFFFull || H > 0x7FFFFFFFull || W * H > 0x7FFFFFFFull) return RTZ_ERR_BAD_ARG;
+    DenoiseConsts k;
+    int32_t rc = denoise_consts(prm, k);
+    if (rc != RTZ_OK) return rc;
+    const size_t nf = 3 * W * H * sizeof(float), nb = 3 * W * H;
+    for (const void* in : {(const void*)d_color, (const void*)d_albedo, (const void*)d_normal})
+        if (overlaps(d_linear, nf, in, nf) || overlaps(d_rgb, nb, in, nf)) return RTZ_ERR_BAD_ARG;
+    if (overlaps(d_linear, nf, d_rgb, nb)) return RTZ_ERR_BAD_ARG;
+    DeviceGuard guard;
+    RTZ_CUDA(cudaSetDevice(c->device));
+    uint64_t launches = 0;
+    RTZ_CUDA(cudaEventRecord(c->ev[0], c->stream));
+    rc = enqueue_denoise(c, (uint32_t)W, (uint32_t)H, d_color, d_albedo, d_normal, k, d_linear, d_rgb, launches);
+    if (rc != RTZ_OK) return rc;
+    RTZ_CUDA(cudaEventRecord(c->ev[1], c->stream));
+    RTZ_CUDA(cudaStreamSynchronize(c->stream));
+    if (st) {
+        std::memset(st, 0, sizeof(*st));
+        st->kernel_launches = launches;
+        float ms = 0;
+        cudaEventElapsedTime(&ms, c->ev[0], c->ev[1]), st->total_ms = ms;
+    }
+    return RTZ_OK;
+}
+
 int32_t rtz_deinterleave(rtz_context* c, uint64_t W, uint64_t H, uint32_t world, uint32_t tw, uint32_t th,
                          const uint8_t* d_gathered, uint8_t* d_rgb) {
     if (!c || !d_gathered || !d_rgb || !W || !H) return RTZ_ERR_BAD_ARG;
@@ -1002,6 +1104,19 @@ int32_t rtz_deinterleave(rtz_context* c, uint64_t W, uint64_t H, uint32_t world,
 static std::mutex g_default_mu;
 static std::map<int, rtz_context*> g_default_ctx;
 
+// the cached context of the caller's current device, created on first use; call with g_default_mu held
+static int32_t default_context(rtz_context** out) {
+    int dev = 0;
+    RTZ_CUDA(cudaGetDevice(&dev));
+    rtz_context*& slot = g_default_ctx[dev];
+    if (!slot) {
+        const int32_t rc = rtz_context_create(dev, nullptr, &slot);
+        if (rc != RTZ_OK) return rc;
+    }
+    *out = slot;
+    return RTZ_OK;
+}
+
 int32_t rtz_render_linear(const rtz_camera* cam, const rtz_sphere* sp, uint64_t n, uint8_t* rgb_out,
                           double* linear_out, rtz_stats* st) {
     if (!rgb_out || (!sp && n)) return RTZ_ERR_BAD_ARG;
@@ -1012,14 +1127,9 @@ int32_t rtz_render_linear(const rtz_camera* cam, const rtz_sphere* sp, uint64_t 
     if (rc != RTZ_OK) return rc;
     std::lock_guard<std::mutex> lock(g_default_mu);
     DeviceGuard guard;
-    int dev = 0;
-    RTZ_CUDA(cudaGetDevice(&dev));
-    rtz_context*& slot = g_default_ctx[dev];
-    if (!slot) {
-        rc = rtz_context_create(dev, nullptr, &slot);
-        if (rc != RTZ_OK) return rc;
-    }
-    rtz_context* c = slot;
+    rtz_context* c = nullptr;
+    rc = default_context(&c);
+    if (rc != RTZ_OK) return rc;
     rc = rtz_scene_upload(c, sp, n);
     if (rc != RTZ_OK) return rc;
     RTZ_CUDA(cudaSetDevice(c->device));
@@ -1038,6 +1148,62 @@ int32_t rtz_render_linear(const rtz_camera* cam, const rtz_sphere* sp, uint64_t 
 
 int32_t rtz_render(const rtz_camera* cam, const rtz_sphere* sp, uint64_t n, uint8_t* rgb_out, rtz_stats* st) {
     return rtz_render_linear(cam, sp, n, rgb_out, nullptr, st);
+}
+
+int32_t rtz_render_denoised(const rtz_camera* cam, const rtz_sphere* sp, uint64_t n, uint64_t guide_samples,
+                            const rtz_denoise_params* prm, uint8_t* rgb_out, float* linear_out, rtz_stats* st) {
+    if ((!rgb_out && !linear_out) || (!sp && n)) return RTZ_ERR_BAD_ARG;
+    int32_t rc = check_camera(cam);
+    if (rc != RTZ_OK) return rc;
+    if (cam->mode != RTZ_MODE_PATH && cam->mode != RTZ_MODE_PATH_BVH) return RTZ_ERR_BAD_ARG;
+    if (guide_samples > cam->samples_per_pixel) return RTZ_ERR_BAD_ARG;
+    const uint64_t px = cam->width * cam->height;
+    if (px > 0x7FFFFFFFull) return RTZ_ERR_BAD_ARG;
+    DenoiseConsts k;
+    rc = denoise_consts(prm, k);
+    if (rc != RTZ_OK) return rc;
+    const uint64_t g = guide_samples ? guide_samples : std::min<uint64_t>(cam->samples_per_pixel, 16);
+    rtz_camera fc = *cam;  // the guides need the frame's seed: draw it once, here
+    if (!fc.has_seed) fc.seed = os_seed(), fc.has_seed = 1;
+    int cnt = 0;
+    rc = rtz_device_count(&cnt);
+    if (rc != RTZ_OK) return rc;
+    std::lock_guard<std::mutex> lock(g_default_mu);
+    DeviceGuard guard;
+    rtz_context* c = nullptr;
+    rc = default_context(&c);
+    if (rc != RTZ_OK) return rc;
+    rc = rtz_scene_upload(c, sp, n);
+    if (rc != RTZ_OK) return rc;
+    RTZ_CUDA(cudaSetDevice(c->device));
+    RTZ_CUDA(c->rgb.reserve(3 * px));
+    RTZ_CUDA(c->denoise_io.reserve(12 * px));
+    float* const lin = c->denoise_io.p;
+    float* const alb = lin + 3 * px;
+    float* const nrm = alb + 3 * px;
+    float* const out = nrm + 3 * px;
+    RTZ_CUDA(cudaEventRecord(c->ev[4], c->stream));
+    rtz_stats rs, gs;
+    rc = render_resident_impl(c, &fc, nullptr, c->rgb.p, nullptr, &rs, lin);
+    if (rc != RTZ_OK) return rc;
+    rc = rtz_render_guides(c, &fc, g, alb, nrm, &gs);
+    if (rc != RTZ_OK) return rc;
+    uint64_t launches = 0;
+    rc = enqueue_denoise(c, (uint32_t)cam->width, (uint32_t)cam->height, lin, alb, nrm, k, linear_out ? out : nullptr,
+                         rgb_out ? c->rgb.p : nullptr, launches);
+    if (rc != RTZ_OK) return rc;
+    RTZ_CUDA(cudaEventRecord(c->ev[5], c->stream));
+    if (rgb_out) RTZ_CUDA(cudaMemcpyAsync(rgb_out, c->rgb.p, 3 * px, cudaMemcpyDeviceToHost, c->stream));
+    if (linear_out)
+        RTZ_CUDA(cudaMemcpyAsync(linear_out, out, 3 * px * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
+    RTZ_CUDA(cudaStreamSynchronize(c->stream));
+    if (st) {
+        *st = rs;
+        st->kernel_launches = rs.kernel_launches + gs.kernel_launches + launches;
+        float ms = 0;
+        cudaEventElapsedTime(&ms, c->ev[4], c->ev[5]), st->total_ms = ms;
+    }
+    return RTZ_OK;
 }
 
 int32_t rtz_write_ppm(const char* path, uint64_t w, uint64_t h, const uint8_t* rgb) {

@@ -151,6 +151,29 @@ class Renderer:
                                            C.c_void_p(normal.data_ptr()), C.byref(st)))
         return albedo, normal, st
 
+    def denoise(self, linear, albedo, normal, params: B.rtz_denoise_params | None = None, out_linear=None,
+                out_rgb=None):
+        """Denoise a whole frame (`rtz_denoise`): the float32 [H, W, 3] device tensors of `render_linear` and
+        `render_guides`; returns (uint8 tensor, float32 tensor, stats) of the denoised frame."""
+        torch = self.torch
+        shape = tuple(linear.shape)
+        assert len(shape) == 3 and shape[2] == 3, shape
+        dev = f"cuda:{self.device}"
+        if out_linear is None:
+            out_linear = torch.empty(shape, dtype=torch.float32, device=dev)
+        if out_rgb is None:
+            out_rgb = torch.empty(shape, dtype=torch.uint8, device=dev)
+        for t, dt in ((linear, torch.float32), (albedo, torch.float32), (normal, torch.float32),
+                      (out_linear, torch.float32), (out_rgb, torch.uint8)):
+            assert t.is_cuda and t.is_contiguous() and t.dtype == dt and tuple(t.shape) == shape, (t.shape, t.dtype)
+        st = B.rtz_stats()
+        self._order_after_torch()
+        B.check(self.lib.rtz_denoise(self._ctx, shape[1], shape[0], C.c_void_p(linear.data_ptr()),
+                                     C.c_void_p(albedo.data_ptr()), C.c_void_p(normal.data_ptr()),
+                                     C.byref(params) if params is not None else None,
+                                     C.c_void_p(out_linear.data_ptr()), C.c_void_p(out_rgb.data_ptr()), C.byref(st)))
+        return out_rgb, out_linear, st
+
     def deinterleave(self, gathered, width: int, height: int, world: int, tile_w: int, tile_h: int, out=None):
         torch = self.torch
         if out is None:
@@ -218,6 +241,27 @@ def render_host_multi(camera, spheres, n: int | None = None, num_gpus: int = 0):
     B.check(l.rtz_render_multi(C.byref(cam), C.cast(arr, C.POINTER(B.rtz_sphere)), n, int(num_gpus),
                                rgb.ctypes.data_as(C.POINTER(C.c_uint8)), C.byref(st)))
     return rgb, st
+
+
+def render_host_denoised(camera, spheres, n: int | None = None, guide_samples: int = 0,
+                         params: B.rtz_denoise_params | None = None):
+    """`rtz_render_denoised`: the one-shot C-ABI call with HOST buffers, render + guides + denoise.
+    Returns (numpy uint8 [H,W,3], numpy float32 [H,W,3] denoised linear colour, stats)."""
+    import numpy as np
+
+    l = B.lib()
+    cam = _cast_camera(camera)
+    arr, cnt = _as_sphere_array(spheres)
+    n = cnt if n is None else int(n)
+    H, W = int(cam.height), int(cam.width)
+    rgb = np.empty((H, W, 3), dtype=np.uint8)
+    lin = np.empty((H, W, 3), dtype=np.float32)
+    st = B.rtz_stats()
+    B.check(l.rtz_render_denoised(C.byref(cam), C.cast(arr, C.POINTER(B.rtz_sphere)), n, int(guide_samples),
+                                  C.byref(params) if params is not None else None,
+                                  rgb.ctypes.data_as(C.POINTER(C.c_uint8)), lin.ctypes.data_as(C.POINTER(C.c_float)),
+                                  C.byref(st)))
+    return rgb, lin, st
 
 
 def render_host(camera, spheres, n: int | None = None, want_linear: bool = False):
