@@ -79,7 +79,13 @@ typedef struct rtz_sphere {
                               /* it (and any non-finite field) with RTZ_ERR_BAD_ARG at upload      */
     int32_t mat_type;         /* RTZ_MAT_*                                                    */
     int32_t reserved;         /* must be 0                                                    */
-    double albedo[3];         /* lambertian, metal                                            */
+    double albedo[3];         /* lambertian, metal: every component in [0, 1] (-0.0 included), */
+                              /* else RTZ_ERR_BAD_ARG at upload.  Samples then lie in [0, 1].   */
+                              /* Each is clamped at 0 and added to an unsigned 32.32 fixed-     */
+                              /* point pixel sum, which agrees with the reference (it sums      */
+                              /* signed samples and clamps the mean) only for samples >= 0, and */
+                              /* a sum stays <= spp * 2^32 < 2^63: exact for every accepted     */
+                              /* spp.  Unchecked for a dielectric: its scatter never reads it.  */
     double fuzz;              /* metal; NOT clamped to <= 1 (reference does not clamp)        */
     double refraction_index;  /* dielectric                                                   */
 } rtz_sphere;

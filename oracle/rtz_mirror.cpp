@@ -264,7 +264,9 @@ inline bool shade(const MCamera& cam, const Rng& g, const std::vector<MSphere>& 
 
 inline uint64_t toFixed(float c) {
     c = (c >= 0.0f) ? c : 0.0f;
-    return (uint64_t)std::llrint((double)(c * 4294967296.0f));  // value is an exact integer < 2^33
+    // samples lie in [0, 1] (rtz_scene_upload refuses albedos outside it): c * 2^32 is exact and at most 2^32, and
+    // llrint rounds it half to even as __float2ull_rn does
+    return (uint64_t)std::llrint((double)(c * 4294967296.0f));
 }
 
 inline uint8_t toByte(double lin) {

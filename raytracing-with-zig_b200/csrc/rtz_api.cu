@@ -779,6 +779,18 @@ int32_t rtz_scene_upload(rtz_context* c, const rtz_sphere* sp, uint64_t n) {
             g_last_error = "sphere " + std::to_string(i) + ": radius must be > 0 and every field of its material finite";
             return RTZ_ERR_BAD_ARG;
         }
+        // The pixel sums are unsigned 32.32 fixed point and every sample is clamped at 0 before it is added
+        // (to_fixed): exact only while samples lie in [0, 1], i.e. while every albedo a path multiplies does.
+        // Dielectric scatter never reads the albedo.
+        if (s.mat_type != RTZ_MAT_DIELECTRIC)
+            for (int k = 0; k < 3; ++k)
+                if (!(s.albedo[k] >= 0.0 && s.albedo[k] <= 1.0)) {
+                    char v[32];
+                    std::snprintf(v, sizeof v, "%.17g", s.albedo[k]);
+                    g_last_error = "sphere " + std::to_string(i) + ": albedo[" + std::to_string(k) + "] = " + v +
+                                   " is outside [0, 1]";
+                    return RTZ_ERR_BAD_ARG;
+                }
         const float cx = (float)s.center[0], cy = (float)s.center[1], cz = (float)s.center[2];
         // q = |c|^2 - r^2 of the FP32-rounded sphere less the per-sphere half of the gate's margin (kGateSlack at
         // ray_constants), evaluated in f64 and rounded once

@@ -564,7 +564,7 @@ def _sweep_scene(orc, n, T):
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize("n_spheres", [16, 200, 485, 513, 4096, 8192])
+@pytest.mark.parametrize("n_spheres", [4, 9, 16, 32, 33, 64, 65, 200, 256, 257, 485, 513, 4096, 8192])
 def test_translated_scene_equals_mirror_in_every_kernel(pkg, gpu, orc, monkeypatch, n_spheres):
     """A sweep scene moved to (1000, 1000, 1000) (and the final scene, at 485, so that the culled kernel runs)
     through every trace kernel that serves its size: bytes, fixed-point sums and counters equal the mirror's."""
