@@ -386,6 +386,44 @@ int32_t rtz_probe_scatters(const rtz_sphere* spheres, uint64_t n_spheres, const 
  * regrouped by median splits of their centres into compact blocks of 32 slots. */
 int32_t rtz_probe_sweep_order(const rtz_sphere* spheres, uint64_t n_spheres, int32_t* order_out);
 
+/* The culled sweep's block bounds (host only, no device needed), on the regrouped order of rtz_probe_sweep_order:
+ * for each of the ceil(n_pad / 32) blocks (n_pad = n rounded up to a multiple of 8), the padded box as the kernel
+ * receives it, 6 floats {lo.x, hi.x, lo.y, hi.y, lo.z, hi.z} (block 0, always swept, has none: zeros); cull_r2, the
+ * squared origin radius the padding covers; and whether a render culls this scene (1) or sweeps it plainly (0).
+ * RTZ_ERR_BAD_ARG for null outputs and for the spheres rtz_scene_upload refuses. */
+int32_t rtz_probe_cull_bounds(const rtz_sphere* spheres, uint64_t n_spheres, float* boxes_out, float* cull_r2_out,
+                              int32_t* host_culls_out);
+
+/* The production sweeps of the render kernels, for chosen rays: each kind runs the device function the named
+ * kernel runs, with the same template arguments, and fills rtz_ray_hit as rtz_probe_hits does (best in the
+ * caller's sphere indices, point and normal from the caller's rows), so one comparison against the f32 mirror
+ * covers it.
+ *   RTZ_SWEEP_CONST            packed sweep over the constant bank (the lockstep kernel, up to 512 spheres)
+ *   RTZ_SWEEP_CULL             the culled constant-bank sweep on the regrouped rows, boxes and cull_r2 of the
+ *                              upload, whether or not a render would cull the scene; split_max (0 .. 64) is the
+ *                              sphere-parallel threshold a frame takes from RTZ_SPLIT
+ *   RTZ_SWEEP_SKIP_SELF        the wavefront kernel's sweep, which drops the sphere a ray leaves outwards (the
+ *                              flag is set from the ray's self as the shader sets it)
+ *   RTZ_SWEEP_SMEM             the rows staged into shared memory (refused where they do not fit)
+ *   RTZ_SWEEP_GLOBAL           the rows read from global memory
+ *   RTZ_SWEEP_COOP             the drain's warp-cooperative sweep, one ray by the whole warp at a time
+ *   RTZ_SWEEP_COOP_REGROUPED   the same on the regrouped rows, ties by original index
+ *   RTZ_SWEEP_BVH              the RTZ_MODE_PATH_BVH traversal, one ray per thread
+ * The two-path kinds (CONST .. GLOBAL) take warps of 64 rays: warp w holds ray 64 w + l in lane l's first slot and
+ * 64 w + 32 + l in its second, so m must be a multiple of 64.  RTZ_ERR_BAD_ARG (with rtz_last_error) for null
+ * pointers, m > 2^31, an unknown kind, split_max outside 0 .. 64, such an m, a constant-bank kind above 512 spheres,
+ * a ray whose self is not -1 or a sphere index, and the spheres rtz_scene_upload refuses. */
+#define RTZ_SWEEP_CONST 0
+#define RTZ_SWEEP_CULL 1
+#define RTZ_SWEEP_SKIP_SELF 2
+#define RTZ_SWEEP_SMEM 3
+#define RTZ_SWEEP_GLOBAL 4
+#define RTZ_SWEEP_COOP 5
+#define RTZ_SWEEP_COOP_REGROUPED 6
+#define RTZ_SWEEP_BVH 7
+int32_t rtz_probe_sweeps(const rtz_sphere* spheres, uint64_t n_spheres, const rtz_probe_ray* rays, uint64_t m,
+                         double t_min, double t_max, int32_t kind, int32_t split_max, rtz_ray_hit* out);
+
 /* Color.toRgb (src/color.zig:63-80) on the device for `n` colours (3 f64 each). */
 int32_t rtz_probe_to_rgb(const double* linear, uint64_t n, uint8_t* rgb_out);
 

@@ -67,6 +67,9 @@ ERR_NAMES = {1: "RTZ_ERR_BAD_ARG", 2: "RTZ_ERR_NO_DEVICE", 3: "RTZ_ERR_CUDA", 4:
              5: "RTZ_ERR_TOO_MANY_SPHERES", 6: "RTZ_ERR_ARCH", 7: "RTZ_ERR_NCCL"}
 GATHER_AUTO, GATHER_P2P, GATHER_NCCL = 0, 1, 2
 ABI_VERSION = 2
+# rtz_probe_sweeps kinds (include/rtz.h)
+(SWEEP_CONST, SWEEP_CULL, SWEEP_SKIP_SELF, SWEEP_SMEM, SWEEP_GLOBAL, SWEEP_COOP, SWEEP_COOP_REGROUPED,
+ SWEEP_BVH) = range(8)
 
 # every symbol include/rtz.h declares, with its signature
 _u8p, _f64p, _f32p = C.POINTER(C.c_uint8), C.POINTER(C.c_double), C.POINTER(C.c_float)
@@ -103,6 +106,8 @@ SIGNATURES = {
     "rtz_probe_scatters": (_i32, [C.POINTER(rtz_sphere), _u64, _vp, _u64, _u64, _vp]),
     "rtz_probe_to_rgb": (_i32, [_f64p, _u64, _u8p]),
     "rtz_probe_sweep_order": (_i32, [C.POINTER(rtz_sphere), _u64, C.POINTER(_i32)]),
+    "rtz_probe_cull_bounds": (_i32, [C.POINTER(rtz_sphere), _u64, _f32p, _f32p, C.POINTER(_i32)]),
+    "rtz_probe_sweeps": (_i32, [C.POINTER(rtz_sphere), _u64, _vp, _u64, _f64, _f64, _i32, _i32, _vp]),
     "rtz_probe_uniform": (_i32, [_u64, _u32, _u32, _u32, _u64, _f32p]),
     "rtz_probe_camera_ray": (_i32, [C.POINTER(rtz_camera), _u64, _u64, _u64, _u64, _f32p, _f32p, _f32p]),
     "rtz_strerror": (C.c_char_p, [_i32]),

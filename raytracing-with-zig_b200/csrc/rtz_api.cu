@@ -122,6 +122,7 @@ struct rtz_context {
     DevBuf<int> bvh_order;
     std::vector<float4> h_geom;
     std::vector<float> h_w;
+    float bvh_r2 = 0.0f;  // BvhParams::r2
     bool bvh_ready = false;
     int n_spheres = 0, n_pad = 0;
     // frame state
@@ -229,6 +230,15 @@ int32_t launch_trace(rtz_context* ctx, Kern kern, const Params& P, uint64_t n_ch
     return RTZ_OK;
 }
 
+// Can the shared-memory kernel stage the scene's rows (pair layout + per-lane rows, 32 B per sphere) next to its own
+// static shared memory (ray staging rows)?  Beyond, the scene is read from L1/L2 (trace_kernel_global).
+cudaError_t smem_rows_fit(const rtz_context* ctx, bool& fits) {
+    cudaFuncAttributes fa{};
+    const cudaError_t e = cudaFuncGetAttributes(&fa, rtz::trace_kernel_smem<512, 1>);
+    fits = (size_t)ctx->n_pad * 32 + fa.sharedSizeBytes + 1024 <= ctx->smem_optin;
+    return e;
+}
+
 // RTZ_MODE_PATH_BVH (extension) needs the hierarchy: built on the host from the FP32 spheres the first time a
 // render asks for it, so that plain uploads (and every brute-force frame) never pay for it.
 int32_t ensure_bvh(rtz_context* c);
@@ -294,10 +304,9 @@ int32_t enqueue_path(rtz_context* ctx, const rtz_camera* cam, const rtz::ShardGe
     }
     const bool use_const = ctx->n_pad <= rtz::kMaxConstSpheres && ctx->geo_const;
     const size_t smem = use_const ? 0 : (size_t)ctx->n_pad * 32;  // pair layout + per-lane rows
-    // too large to stage next to the kernel's own static shared memory (ray staging rows): read it from L1/L2
-    cudaFuncAttributes fa{};
-    RTZ_CUDA(cudaFuncGetAttributes(&fa, rtz::trace_kernel_smem<512, 1>));
-    const bool use_global = !use_const && smem + fa.sharedSizeBytes + 1024 > ctx->smem_optin;
+    bool smem_fits = false;
+    RTZ_CUDA(smem_rows_fit(ctx, smem_fits));
+    const bool use_global = !use_const && !smem_fits;
     RTZ_CUDA(cudaEventRecord(ctx->ev[0], ctx->stream));
     RTZ_CUDA(cudaMemsetAsync(ctx->accum.p, 0, 3 * n_local_pixels * sizeof(unsigned long long), ctx->stream));
     RTZ_CUDA(cudaMemsetAsync(ctx->counters.p, 0, 16 * sizeof(unsigned long long), ctx->stream));
@@ -308,7 +317,7 @@ int32_t enqueue_path(rtz_context* ctx, const rtz_camera* cam, const rtz::ShardGe
         // `while (bounces < bounceMax)` never runs (src/camera.zig:153): every sample is black and no
         // world.hit is made.  Nothing to trace; the zeroed sums resolve to zeros.
     } else if (cam->mode == RTZ_MODE_PATH_BVH) {
-        rtz::BvhParams B{P, ctx->bvh_nodes.p, ctx->bvh_order.p, ctx->wexp.p};
+        rtz::BvhParams B{P, ctx->bvh_nodes.p, ctx->bvh_order.p, ctx->wexp.p, ctx->bvh_r2};
         rc = launch_trace(ctx, rtz::trace_kernel_bvh<128, 6>, B, P.n_chunks, 128, 0);
     } else if (use_const) {
         static thread_local rtz::TraceParamsConst C;  // 8 KiB: keep it off the stack
@@ -704,16 +713,29 @@ struct BvhBuilder {
     const std::vector<float4>& g;
     std::vector<rtz::BvhNode> nodes;
     std::vector<int> order;
+    double R = 0.0;  // the origin radius the padding covers (BvhParams::r2)
     explicit BvhBuilder(const std::vector<float4>& geom, int n) : g(geom), order(n) {
         for (int i = 0; i < n; ++i) order[i] = i;
+        // twice the farthest point of a sphere other than sphere 0 (the ground of the book's scenes, whose far side
+        // would make every pad large); a ray from beyond R widens the boxes it tests instead (hit_box)
+        double reach = 0.0;
+        for (int i = n > 1 ? 1 : 0; i < n; ++i) {
+            const float4 s = g[i];
+            reach = std::max(reach, std::sqrt((double)s.x * s.x + (double)s.y * s.y + (double)s.z * s.z) + std::sqrt(-(double)s.w));
+        }
+        R = 2.0 * reach;
     }
-    void bounds(int first, int cnt, float lo[3], float hi[3]) const {
+    void bounds(int first, int cnt, float lo[3], float hi[3], float& inv_r) const {
         for (int a = 0; a < 3; ++a) lo[a] = INFINITY, hi[a] = -INFINITY;
+        inv_r = 0.0f;
         for (int q = first; q < first + cnt; ++q) {
             const float4 s = g[order[q]];
             const float c[3] = {s.x, s.y, s.z};
             const float r = std::sqrt(-s.w);
-            const float pad = 1e-4f * (1.0f + r + std::fabs(s.x) + std::fabs(s.y) + std::fabs(s.z));
+            inv_r = std::max(inv_r, 1.0f / r);
+            const double cn = std::sqrt((double)s.x * s.x + (double)s.y * s.y + (double)s.z * s.z);
+            const float pad = 1e-4f * (1.0f + r + std::fabs(s.x) + std::fabs(s.y) + std::fabs(s.z)) +
+                              (float)(1e-6 * (1.001 * R + cn) * (1.001 * R + cn) / r);
             for (int a = 0; a < 3; ++a) lo[a] = std::min(lo[a], c[a] - r - pad), hi[a] = std::max(hi[a], c[a] + r + pad);
         }
     }
@@ -739,9 +761,9 @@ struct BvhBuilder {
         nodes.emplace_back();
         const int c0 = build(first, half), c1 = build(first + half, cnt - half);
         rtz::BvhNode& nd = nodes[me];
-        bounds(first, half, nd.lo0, nd.hi0);
-        bounds(first + half, cnt - half, nd.lo1, nd.hi1);
-        nd.child0 = c0, nd.child1 = c1, nd.pad0 = nd.pad1 = 0;
+        bounds(first, half, nd.lo0, nd.hi0, nd.inv_r0);
+        bounds(first + half, cnt - half, nd.lo1, nd.hi1, nd.inv_r1);
+        nd.child0 = c0, nd.child1 = c1;
         return me;
     }
     void run() {
@@ -750,59 +772,71 @@ struct BvhBuilder {
         const int root = n > 0 ? build(0, n) : rtz::kBvhEmpty;
         if (root != 0) {  // fewer than five spheres (or none): a root whose first child is the only leaf
             rtz::BvhNode nd{};
-            if (n > 0) bounds(0, n, nd.lo0, nd.hi0);
+            if (n > 0) bounds(0, n, nd.lo0, nd.hi0, nd.inv_r0);
             nd.child0 = root, nd.child1 = rtz::kBvhEmpty;
             nodes.insert(nodes.begin(), nd);
         }
     }
 };
-}  // namespace
 
-int32_t rtz_scene_upload(rtz_context* c, const rtz_sphere* sp, uint64_t n) {
-    if (!c || (!sp && n) || n > (1u << 20)) return RTZ_ERR_BAD_ARG;
-    DeviceGuard guard;
-    RTZ_CUDA(cudaSetDevice(c->device));
+// The host rows of a scene, before any of them reaches a device: the sweep rows, and the regrouped order, block
+// boxes and cull_r2 of the culled kernel with the host's choice of whether to cull.  RTZ_ERR_BAD_ARG (and
+// g_last_error) for a sphere the renderer refuses.
+struct HostScene {
+    int n_pad = 0;
+    std::vector<float4> g, a, al, pairs;
+    std::vector<float> w;
+    std::vector<rtz::DSphere> ds;
+    std::vector<int> order;
+    std::vector<float4> boxes;
+    double R = 0.0;
+    bool cull = false;
+};
+int32_t host_scene(const rtz_sphere* sp, uint64_t n, HostScene& s) {
     const int n_pad = (int)((n + 7) & ~7ull);
-    std::vector<float4> g(n_pad ? n_pad : 1), a(n_pad ? n_pad : 1), al(n_pad ? n_pad : 1);
-    std::vector<float> w(n_pad ? n_pad : 1);
-    std::vector<rtz::DSphere> ds(n ? n : 1);
+    s.n_pad = n_pad;
+    std::vector<float4>&g = s.g, &a = s.a, &al = s.al;
+    std::vector<float>& w = s.w;
+    g.assign(n_pad ? n_pad : 1, float4{}), a.assign(n_pad ? n_pad : 1, float4{}), al.assign(n_pad ? n_pad : 1, float4{});
+    w.assign(n_pad ? n_pad : 1, 0.f);
+    s.ds.assign(n ? n : 1, rtz::DSphere{});
     for (uint64_t i = 0; i < n; ++i) {
-        const rtz_sphere& s = sp[i];
-        if (s.mat_type < RTZ_MAT_LAMBERTIAN || s.mat_type > RTZ_MAT_DIELECTRIC) return RTZ_ERR_BAD_ARG;
-        const float r = (float)(s.radius < 0 ? 0.0 : s.radius);  // Sphere.init clamp (src/sphere.zig:21)
+        const rtz_sphere& sph = sp[i];
+        if (sph.mat_type < RTZ_MAT_LAMBERTIAN || sph.mat_type > RTZ_MAT_DIELECTRIC) return RTZ_ERR_BAD_ARG;
+        const float r = (float)(sph.radius < 0 ? 0.0 : sph.radius);  // Sphere.init clamp (src/sphere.zig:21)
         // A radius-0 sphere makes the reference panic in Vec.divScalar (src/vec.zig:39-45) when it is hit, and
         // NaN / infinite geometry only yields NaN samples: both are refused here instead of rendered wrongly.
-        const bool mat_ok = s.mat_type == RTZ_MAT_DIELECTRIC
-                                ? (std::isfinite(s.refraction_index) && (float)s.refraction_index != 0.0f)
-                                : (finite3(s.albedo) && (s.mat_type != RTZ_MAT_METAL || std::isfinite(s.fuzz)));
-        if (!finite3(s.center) || !std::isfinite(s.radius) || !(r > 0.0f) || !mat_ok) {
+        const bool mat_ok = sph.mat_type == RTZ_MAT_DIELECTRIC
+                                ? (std::isfinite(sph.refraction_index) && (float)sph.refraction_index != 0.0f)
+                                : (finite3(sph.albedo) && (sph.mat_type != RTZ_MAT_METAL || std::isfinite(sph.fuzz)));
+        if (!finite3(sph.center) || !std::isfinite(sph.radius) || !(r > 0.0f) || !mat_ok) {
             g_last_error = "sphere " + std::to_string(i) + ": radius must be > 0 and every field of its material finite";
             return RTZ_ERR_BAD_ARG;
         }
         // The pixel sums are unsigned 32.32 fixed point and every sample is clamped at 0 before it is added
         // (to_fixed): exact only while samples lie in [0, 1], i.e. while every albedo a path multiplies does.
         // Dielectric scatter never reads the albedo.
-        if (s.mat_type != RTZ_MAT_DIELECTRIC)
+        if (sph.mat_type != RTZ_MAT_DIELECTRIC)
             for (int k = 0; k < 3; ++k)
-                if (!(s.albedo[k] >= 0.0 && s.albedo[k] <= 1.0)) {
+                if (!(sph.albedo[k] >= 0.0 && sph.albedo[k] <= 1.0)) {
                     char v[32];
-                    std::snprintf(v, sizeof v, "%.17g", s.albedo[k]);
+                    std::snprintf(v, sizeof v, "%.17g", sph.albedo[k]);
                     g_last_error = "sphere " + std::to_string(i) + ": albedo[" + std::to_string(k) + "] = " + v +
                                    " is outside [0, 1]";
                     return RTZ_ERR_BAD_ARG;
                 }
-        const float cx = (float)s.center[0], cy = (float)s.center[1], cz = (float)s.center[2];
+        const float cx = (float)sph.center[0], cy = (float)sph.center[1], cz = (float)sph.center[2];
         // q = |c|^2 - r^2 of the FP32-rounded sphere less the per-sphere half of the gate's margin (kGateSlack at
         // ray_constants), evaluated in f64 and rounded once
         const double c2 = (double)cx * cx + (double)cy * cy + (double)cz * cz;
         const double q = (c2 - (double)r * r) - (double)rtz::kGateSlack * c2;
         g[i] = make_float4(cx, cy, cz, -(r * r));
         w[i] = -(float)q;
-        const float param = s.mat_type == RTZ_MAT_METAL ? (float)s.fuzz : (float)s.refraction_index;
-        a[i] = make_float4(r, 1.0f / r, param, bits_to_float(s.mat_type));
-        al[i] = make_float4((float)s.albedo[0], (float)s.albedo[1], (float)s.albedo[2],
-                            1.0f / (float)s.refraction_index);
-        ds[i] = rtz::DSphere{s.center[0], s.center[1], s.center[2], s.radius < 0 ? 0.0 : s.radius};
+        const float param = sph.mat_type == RTZ_MAT_METAL ? (float)sph.fuzz : (float)sph.refraction_index;
+        a[i] = make_float4(r, 1.0f / r, param, bits_to_float(sph.mat_type));
+        al[i] = make_float4((float)sph.albedo[0], (float)sph.albedo[1], (float)sph.albedo[2],
+                            1.0f / (float)sph.refraction_index);
+        s.ds[i] = rtz::DSphere{sph.center[0], sph.center[1], sph.center[2], sph.radius < 0 ? 0.0 : sph.radius};
     }
     for (int i = (int)n; i < n_pad; ++i) {  // padding: w = -inf  ->  disc = -inf (never a candidate)
         g[i] = make_float4(0.f, 0.f, 0.f, -0.f);
@@ -810,17 +844,19 @@ int32_t rtz_scene_upload(rtz_context* c, const rtz_sphere* sp, uint64_t n) {
         a[i] = make_float4(0.f, 0.f, 0.f, bits_to_float(0));
         al[i] = make_float4(0.f, 0.f, 0.f, 0.f);
     }
-    std::vector<float4> pr = pair_rows(g, w, n_pad);
+    s.pairs = pair_rows(g, w, n_pad);
     // Bounds of the culled kernel's 32-sphere blocks, on its regrouped order (box_reach in rtz_kernels.cuh states
     // the exactness contract these paddings serve).  R covers every ray origin within twice the farthest point of
     // a sphere outside block 0; block 0 (the ground of the book's scenes) has no box: it is always swept.
-    const std::vector<int> order = sweep_order(g, (int)n);
+    s.order = sweep_order(g, (int)n);
+    const std::vector<int>& order = s.order;
     const int n_blocks = (n_pad + 31) / 32;
-    std::vector<float4> bx(2 * (size_t)std::max(n_blocks, 1), make_float4(0.f, 0.f, 0.f, 0.f));
+    std::vector<float4>& bx = s.boxes;
+    bx.assign(2 * (size_t)std::max(n_blocks, 1), make_float4(0.f, 0.f, 0.f, 0.f));
     double reach = 0.0;
     for (uint64_t q = 32; q < n; ++q) {
-        const float4 s = g[order[q]];
-        reach = std::max(reach, std::sqrt((double)s.x * s.x + (double)s.y * s.y + (double)s.z * s.z) + std::sqrt(-(double)s.w));
+        const float4 c = g[order[q]];
+        reach = std::max(reach, std::sqrt((double)c.x * c.x + (double)c.y * c.y + (double)c.z * c.z) + std::sqrt(-(double)c.w));
     }
     const double R = 2.0 * reach;
     double lo_all[3] = {INFINITY, INFINITY, INFINITY}, hi_all[3] = {-INFINITY, -INFINITY, -INFINITY}, vol_sum = 0.0;
@@ -828,17 +864,17 @@ int32_t rtz_scene_upload(rtz_context* c, const rtz_sphere* sp, uint64_t n) {
     for (int b = 1; b < n_blocks; ++b) {
         double lo[3] = {INFINITY, INFINITY, INFINITY}, hi[3] = {-INFINITY, -INFINITY, -INFINITY};
         for (uint64_t q = 32ull * b; q < std::min<uint64_t>(n, 32ull * b + 32); ++q) {
-            const float4 s = g[order[q]];
-            const double c[3] = {s.x, s.y, s.z}, r = std::sqrt(-(double)s.w);
+            const float4 sq = g[order[q]];
+            const double c[3] = {sq.x, sq.y, sq.z}, r = std::sqrt(-(double)sq.w);
             const double cn = std::sqrt(c[0] * c[0] + c[1] * c[1] + c[2] * c[2]);
             const double pad = 1e-4 * (1.0 + r + std::fabs(c[0]) + std::fabs(c[1]) + std::fabs(c[2])) +
                                1e-6 * (1.001 * R + cn) * (1.001 * R + cn) / r;
-            for (int a = 0; a < 3; ++a) lo[a] = std::min(lo[a], c[a] - r - pad), hi[a] = std::max(hi[a], c[a] + r + pad);
+            for (int k = 0; k < 3; ++k) lo[k] = std::min(lo[k], c[k] - r - pad), hi[k] = std::max(hi[k], c[k] + r + pad);
         }
         float fl[3], fh[3];  // rounded outwards
-        for (int a = 0; a < 3; ++a) {
-            fl[a] = std::nextafter((float)lo[a], -INFINITY), fh[a] = std::nextafter((float)hi[a], INFINITY);
-            lo_all[a] = std::min(lo_all[a], lo[a]), hi_all[a] = std::max(hi_all[a], hi[a]);
+        for (int k = 0; k < 3; ++k) {
+            fl[k] = std::nextafter((float)lo[k], -INFINITY), fh[k] = std::nextafter((float)hi[k], INFINITY);
+            lo_all[k] = std::min(lo_all[k], lo[k]), hi_all[k] = std::max(hi_all[k], hi[k]);
         }
         bx[2 * b] = make_float4(fl[0], fh[0], fl[1], fh[1]);
         bx[2 * b + 1] = make_float4(fl[2], fh[2], 0.f, 0.f);
@@ -849,16 +885,30 @@ int32_t rtz_scene_upload(rtz_context* c, const rtz_sphere* sp, uint64_t n) {
     // compact blocks (485 in a cube: about 7 % each), and it is faster culled (DESIGN.md §5).
     for (double v : vols) vol_sum += v;
     const double vol_all = (hi_all[0] - lo_all[0]) * (hi_all[1] - lo_all[1]) * (hi_all[2] - lo_all[2]);
-    const bool cull = n_pad <= rtz::kMaxConstSpheres && !vols.empty() && std::isfinite(R) &&
-                      vol_sum < 0.25 * vols.size() * vol_all;
+    s.R = R;
+    s.cull = n_pad <= rtz::kMaxConstSpheres && !vols.empty() && std::isfinite(R) && vol_sum < 0.25 * vols.size() * vol_all;
+    return RTZ_OK;
+}
+
+// rtz_scene_upload; `regrouped` also uploads the culled kernel's rows for a scene the host does not cull (the
+// sweep probes: the exactness of the cull must not depend on the host's choice)
+int32_t scene_upload(rtz_context* c, const rtz_sphere* sp, uint64_t n, bool regrouped) {
+    if (!c || (!sp && n) || n > (1u << 20)) return RTZ_ERR_BAD_ARG;
+    DeviceGuard guard;
+    RTZ_CUDA(cudaSetDevice(c->device));
+    HostScene s;
+    const int32_t rc = host_scene(sp, n, s);
+    if (rc != RTZ_OK) return rc;
+    const int n_pad = s.n_pad;
+    const bool rows = s.cull || (regrouped && n_pad);
     // the rows of the culled kernel in its order; padding stays in slots n .. n_pad-1
-    std::vector<float4> rg(cull ? n_pad : 0), ra(cull ? n_pad : 0), ral(cull ? n_pad : 0), rpr;
-    std::vector<float> rw(cull ? n_pad : 0);
-    std::vector<int> ro(cull ? n_pad : 0);
-    if (cull) {
+    std::vector<float4> rg(rows ? n_pad : 0), ra(rows ? n_pad : 0), ral(rows ? n_pad : 0), rpr;
+    std::vector<float> rw(rows ? n_pad : 0);
+    std::vector<int> ro(rows ? n_pad : 0);
+    if (rows) {
         for (int q = 0; q < n_pad; ++q) {
-            const int i = q < (int)n ? order[q] : q;
-            rg[q] = g[i], ra[q] = a[i], ral[q] = al[i], rw[q] = w[i], ro[q] = i;
+            const int i = q < (int)n ? s.order[q] : q;
+            rg[q] = s.g[i], ra[q] = s.a[i], ral[q] = s.al[i], rw[q] = s.w[i], ro[q] = i;
         }
         rpr = pair_rows(rg, rw, n_pad);
     }
@@ -874,14 +924,14 @@ int32_t rtz_scene_upload(rtz_context* c, const rtz_sphere* sp, uint64_t n) {
         RTZ_CUDA(c->aux.reserve(n_pad));
         RTZ_CUDA(c->albedo.reserve(n_pad));
         RTZ_CUDA(c->wexp.reserve(n_pad));
-        RTZ_CUDA(cudaMemcpyAsync(c->wexp.p, w.data(), n_pad * sizeof(float), cudaMemcpyHostToDevice, c->stream));
+        RTZ_CUDA(cudaMemcpyAsync(c->wexp.p, s.w.data(), n_pad * sizeof(float), cudaMemcpyHostToDevice, c->stream));
         // pageable sources: cudaMemcpyAsync returns once the bytes are staged, so the vectors may die at return
-        RTZ_CUDA(cudaMemcpyAsync(c->geom.p, g.data(), n_pad * sizeof(float4), cudaMemcpyHostToDevice, c->stream));
-        RTZ_CUDA(cudaMemcpyAsync(c->pairs.p, pr.data(), n_pad * sizeof(float4), cudaMemcpyHostToDevice, c->stream));
-        RTZ_CUDA(cudaMemcpyAsync(c->aux.p, a.data(), n_pad * sizeof(float4), cudaMemcpyHostToDevice, c->stream));
-        RTZ_CUDA(cudaMemcpyAsync(c->albedo.p, al.data(), n_pad * sizeof(float4), cudaMemcpyHostToDevice, c->stream));
+        RTZ_CUDA(cudaMemcpyAsync(c->geom.p, s.g.data(), n_pad * sizeof(float4), cudaMemcpyHostToDevice, c->stream));
+        RTZ_CUDA(cudaMemcpyAsync(c->pairs.p, s.pairs.data(), n_pad * sizeof(float4), cudaMemcpyHostToDevice, c->stream));
+        RTZ_CUDA(cudaMemcpyAsync(c->aux.p, s.a.data(), n_pad * sizeof(float4), cudaMemcpyHostToDevice, c->stream));
+        RTZ_CUDA(cudaMemcpyAsync(c->albedo.p, s.al.data(), n_pad * sizeof(float4), cudaMemcpyHostToDevice, c->stream));
     }
-    if (cull) {
+    if (rows) {
         RTZ_CUDA(c->rg_geom.reserve(n_pad));
         RTZ_CUDA(c->rg_aux.reserve(n_pad));
         RTZ_CUDA(c->rg_albedo.reserve(n_pad));
@@ -893,19 +943,22 @@ int32_t rtz_scene_upload(rtz_context* c, const rtz_sphere* sp, uint64_t n) {
         RTZ_CUDA(cudaMemcpyAsync(c->rg_wexp.p, rw.data(), n_pad * sizeof(float), cudaMemcpyHostToDevice, c->stream));
         RTZ_CUDA(cudaMemcpyAsync(c->rg_orig.p, ro.data(), n_pad * sizeof(int), cudaMemcpyHostToDevice, c->stream));
     }
-    RTZ_CUDA(c->dspheres.reserve(ds.size()));
-    RTZ_CUDA(cudaMemcpyAsync(c->dspheres.p, ds.data(), ds.size() * sizeof(rtz::DSphere), cudaMemcpyHostToDevice,
+    RTZ_CUDA(c->dspheres.reserve(s.ds.size()));
+    RTZ_CUDA(cudaMemcpyAsync(c->dspheres.p, s.ds.data(), s.ds.size() * sizeof(rtz::DSphere), cudaMemcpyHostToDevice,
                              c->stream));
-    c->h_pairs.swap(pr);  // host copy: small scenes travel to the kernel as a __grid_constant__ parameter
+    c->h_pairs.swap(s.pairs);  // host copy: small scenes travel to the kernel as a __grid_constant__ parameter
     c->h_rg_pairs.swap(rpr);
-    c->h_boxes.swap(bx);
-    c->cull_r2 = (float)(R * R);
-    c->cull = cull;
-    g.resize(n), w.resize(n);
-    c->h_geom.swap(g), c->h_w.swap(w);  // what the BVH extension is built from, if it is ever asked for
+    c->h_boxes.swap(s.boxes);
+    c->cull_r2 = (float)(s.R * s.R);
+    c->cull = s.cull;
+    s.g.resize(n), s.w.resize(n);
+    c->h_geom.swap(s.g), c->h_w.swap(s.w);  // what the BVH extension is built from, if it is ever asked for
     c->n_spheres = (int)n, c->n_pad = n_pad;
     return RTZ_OK;
 }
+}  // namespace
+
+int32_t rtz_scene_upload(rtz_context* c, const rtz_sphere* sp, uint64_t n) { return scene_upload(c, sp, n, false); }
 
 }  // extern "C"
 
@@ -922,6 +975,7 @@ int32_t ensure_bvh(rtz_context* c) {
         RTZ_CUDA(cudaMemcpyAsync(c->bvh_order.p, bvh.order.data(), n * sizeof(int), cudaMemcpyHostToDevice, c->stream));
     }
     RTZ_CUDA(cudaStreamSynchronize(c->stream));
+    c->bvh_r2 = (float)(bvh.R * bvh.R);
     c->bvh_ready = true;
     return RTZ_OK;
 }
@@ -1620,12 +1674,14 @@ extern "C" {
 
 namespace {
 // Upload the scene to a fresh context, copy the m records in, run `launch(ctx, in, out)` and copy the m results out.
+// `launch` returns RTZ_OK or refuses the call before it launches anything.
 template <class In, class Out, class Launch>
-int32_t run_probe(const rtz_sphere* sp, uint64_t n, const In* in, uint64_t m, Out* out, Launch launch) {
+int32_t run_probe(const rtz_sphere* sp, uint64_t n, const In* in, uint64_t m, Out* out, Launch launch,
+                  bool regrouped = false) {
     ScopedCtx sc;
     int32_t rc = rtz_context_create(-1, nullptr, &sc.c);
     if (rc != RTZ_OK) return rc;
-    rc = rtz_scene_upload(sc.c, sp, n);
+    rc = scene_upload(sc.c, sp, n, regrouped);
     if (rc != RTZ_OK) return rc;
     In* din = nullptr;
     Out* dout = nullptr;
@@ -1633,13 +1689,14 @@ int32_t run_probe(const rtz_sphere* sp, uint64_t n, const In* in, uint64_t m, Ou
     if (e == cudaSuccess) e = cudaMalloc(&dout, m * sizeof(Out));
     if (e == cudaSuccess) e = cudaMemcpyAsync(din, in, m * sizeof(In), cudaMemcpyHostToDevice, sc.c->stream);
     if (e == cudaSuccess) {
-        launch(sc.c, din, dout, (unsigned)((m + 127) / 128));
+        rc = launch(sc.c, din, dout, (unsigned)((m + 127) / 128));
         e = cudaGetLastError();
     }
-    if (e == cudaSuccess) e = cudaMemcpyAsync(out, dout, m * sizeof(Out), cudaMemcpyDeviceToHost, sc.c->stream);
+    if (e == cudaSuccess && rc == RTZ_OK) e = cudaMemcpyAsync(out, dout, m * sizeof(Out), cudaMemcpyDeviceToHost, sc.c->stream);
     if (e == cudaSuccess) e = cudaStreamSynchronize(sc.c->stream);
     cudaFree(din);
     cudaFree(dout);
+    if (rc != RTZ_OK) return rc;
     RTZ_CUDA(e);
     return RTZ_OK;
 }
@@ -1654,6 +1711,7 @@ int32_t rtz_probe_hits(const rtz_sphere* sp, uint64_t n, const rtz_probe_ray* ra
     return run_probe(sp, n, rays, m, out, [&](rtz_context* c, const rtz_probe_ray* din, rtz_ray_hit* dout, unsigned blocks) {
         rtz::probe_hits_kernel<<<blocks, 128, 0, c->stream>>>(c->geom.p, c->pairs.p, c->aux.p, c->n_pad, din, m,
                                                              (float)tmin, (float)tmax, dout);
+        return RTZ_OK;
     });
 }
 
@@ -1670,6 +1728,7 @@ int32_t rtz_probe_scatters(const rtz_sphere* sp, uint64_t n, const rtz_probe_bou
     return run_probe(sp, n, recs, m, out, [&](rtz_context* c, const rtz_probe_bounce* din, rtz_ray_scatter* dout, unsigned blocks) {
         rtz::probe_scatters_kernel<<<blocks, 128, 0, c->stream>>>(dc, c->geom.p, c->pairs.p, c->aux.p, c->albedo.p, din, m,
                                                                  dout);
+        return RTZ_OK;
     });
 }
 
@@ -1720,6 +1779,101 @@ int32_t rtz_probe_sweep_order(const rtz_sphere* sp, uint64_t n, int32_t* order_o
     const std::vector<int> order = sweep_order(g, (int)n);
     std::copy(order.begin(), order.end(), order_out);
     return RTZ_OK;
+}
+
+int32_t rtz_probe_cull_bounds(const rtz_sphere* sp, uint64_t n, float* boxes_out, float* cull_r2_out,
+                              int32_t* host_culls_out) {
+    if ((!sp && n) || (!boxes_out && n) || !cull_r2_out || !host_culls_out || n > (1u << 20)) return RTZ_ERR_BAD_ARG;
+    HostScene s;
+    const int32_t rc = host_scene(sp, n, s);
+    if (rc != RTZ_OK) return rc;
+    for (int b = 0; b < (s.n_pad + 31) / 32; ++b) {
+        const float4 b0 = s.boxes[2 * b], b1 = s.boxes[2 * b + 1];
+        const float v[6] = {b0.x, b0.y, b0.z, b0.w, b1.x, b1.y};
+        std::copy(v, v + 6, boxes_out + 6 * b);
+    }
+    *cull_r2_out = (float)(s.R * s.R);
+    *host_culls_out = s.cull ? 1 : 0;
+    return RTZ_OK;
+}
+
+int32_t rtz_probe_sweeps(const rtz_sphere* sp, uint64_t n, const rtz_probe_ray* rays, uint64_t m, double tmin,
+                         double tmax, int32_t kind, int32_t split_max, rtz_ray_hit* out) {
+    auto refuse = [](const std::string& why) {
+        g_last_error = "rtz_probe_sweeps: " + why;
+        return RTZ_ERR_BAD_ARG;
+    };
+    if (!sp || !n || (!rays && m) || (!out && m)) return refuse("null spheres, rays or output, or no spheres");
+    if (n > (1u << 20) || m > (1ull << 31)) return refuse("too many spheres or rays");
+    if (kind < RTZ_SWEEP_CONST || kind > RTZ_SWEEP_BVH) return refuse("unknown sweep kind " + std::to_string(kind));
+    if (split_max < 0 || split_max > 64) return refuse("split_max must lie in 0 .. 64");
+    const bool two_path = kind <= RTZ_SWEEP_GLOBAL, const_bank = kind <= RTZ_SWEEP_SKIP_SELF;
+    if (two_path && m % 64) return refuse("a two-path sweep takes its rays in warps of 64: m must be a multiple of 64");
+    if (const_bank && n > (uint64_t)rtz::kMaxConstSpheres) return refuse("the constant bank holds at most 512 spheres");
+    const bool regrouped = kind == RTZ_SWEEP_CULL || kind == RTZ_SWEEP_COOP_REGROUPED;
+    // `self` in the sweep's slots
+    std::vector<rtz_probe_ray> in(rays, rays + m);
+    std::vector<int32_t> slot(regrouped ? n : 0);
+    if (regrouped) {
+        std::vector<int32_t> order(n);
+        const int32_t rc = rtz_probe_sweep_order(sp, n, order.data());
+        if (rc != RTZ_OK) return rc;
+        for (uint64_t q = 0; q < n; ++q) slot[order[q]] = (int32_t)q;
+    }
+    for (rtz_probe_ray& r : in) {
+        if (r.self < -1 || (int64_t)r.self >= (int64_t)n) return refuse("a ray's self is not -1 or a sphere index");
+        if (regrouped && r.self >= 0) r.self = slot[r.self];
+    }
+    if (!m) return RTZ_OK;
+    auto launch = [&](rtz_context* c, const rtz_probe_ray* din, rtz_ray_hit* dout, unsigned blocks) -> int32_t {
+        const rtz::SweepProbeIO io{din, m, (float)tmin, (float)tmax, c->geom.p, c->aux.p,
+                                   regrouped ? c->rg_orig.p : nullptr, dout};
+        rtz::TraceParams P{};
+        P.geom = c->geom.p, P.pairs = c->pairs.p, P.aux = c->aux.p, P.albedo = c->albedo.p, P.wexp = c->wexp.p;
+        P.orig = nullptr;
+        P.n_spheres = c->n_spheres, P.n_pad = c->n_pad;
+        const unsigned pair_blocks = (unsigned)((m / 64 + 3) / 4);  // four warps of 64 rays per block
+        if (const_bank) {
+            static thread_local rtz::TraceParamsConst C;
+            if (kind == RTZ_SWEEP_CULL) {  // trace_kernel_const_cull's parameters
+                P.geom = c->rg_geom.p, P.aux = c->rg_aux.p, P.albedo = c->rg_albedo.p, P.wexp = c->rg_wexp.p;
+                P.orig = c->rg_orig.p, P.pairs = nullptr;
+                std::memcpy(C.pairs, c->h_rg_pairs.data(), (size_t)c->n_pad * sizeof(float4));
+                std::memcpy(C.boxes, c->h_boxes.data(), c->h_boxes.size() * sizeof(float4));
+                C.cull_r2 = c->cull_r2;
+                C.split_max = split_max;
+            } else {
+                std::memcpy(C.pairs, c->h_pairs.data(), (size_t)c->n_pad * sizeof(float4));
+            }
+            C.p = P;
+            if (kind == RTZ_SWEEP_CONST)
+                rtz::probe_sweep_const_kernel<false, false><<<pair_blocks, 128, 0, c->stream>>>(C, io);
+            else if (kind == RTZ_SWEEP_SKIP_SELF)
+                rtz::probe_sweep_const_kernel<true, false><<<pair_blocks, 128, 0, c->stream>>>(C, io);
+            else
+                rtz::probe_sweep_const_kernel<false, true><<<pair_blocks, 128, 0, c->stream>>>(C, io);
+        } else if (kind == RTZ_SWEEP_SMEM) {
+            bool fits = false;
+            RTZ_CUDA(smem_rows_fit(c, fits));
+            if (!fits) return refuse("the scene's rows do not fit in shared memory");
+            const size_t smem = (size_t)c->n_pad * 32;
+            RTZ_CUDA(cudaFuncSetAttribute(rtz::probe_sweep_smem_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+            rtz::probe_sweep_smem_kernel<<<pair_blocks, 128, smem, c->stream>>>(P, io);
+        } else if (kind == RTZ_SWEEP_GLOBAL) {
+            rtz::probe_sweep_global_kernel<<<pair_blocks, 128, 0, c->stream>>>(P, io);
+        } else if (kind == RTZ_SWEEP_COOP) {
+            rtz::probe_coop_kernel<<<blocks, 128, 0, c->stream>>>(c->geom.p, c->wexp.p, nullptr, c->n_spheres, io);
+        } else if (kind == RTZ_SWEEP_COOP_REGROUPED) {
+            rtz::probe_coop_kernel<<<blocks, 128, 0, c->stream>>>(c->rg_geom.p, c->rg_wexp.p, c->rg_orig.p, c->n_spheres, io);
+        } else {
+            const int32_t rc = ensure_bvh(c);
+            if (rc != RTZ_OK) return rc;
+            const rtz::BvhParams B{P, c->bvh_nodes.p, c->bvh_order.p, c->wexp.p, c->bvh_r2};
+            rtz::probe_bvh_kernel<<<blocks, 128, 0, c->stream>>>(B, io);
+        }
+        return RTZ_OK;
+    };
+    return run_probe(sp, n, in.data(), m, out, launch, regrouped);
 }
 
 int32_t rtz_probe_to_rgb(const double* lin, uint64_t n, uint8_t* rgb_out) {

@@ -18,7 +18,7 @@ namespace rtz {
 struct BvhNode {
     float lo0[3], hi0[3], lo1[3], hi1[3];
     int child0, child1;
-    int pad0, pad1;
+    float inv_r0, inv_r1;  // the largest 1 / r among each child's spheres (hit_box's slack)
 };
 static_assert(sizeof(BvhNode) == 64, "BvhNode is four float4");
 constexpr int kBvhEmpty = 0x7fffffff;
@@ -29,6 +29,7 @@ struct BvhParams {
     const BvhNode* nodes;
     const int* order;     // leaf ranges: original sphere indices
     const float* wexp;    // [n] w = -(|c|^2 - r^2) of the expanded discriminant, as in the sweep layout
+    float r2;             // the squared origin radius the boxes' padding covers (hit_box)
 };
 
 // Sphere.hit for one sphere through the brute-force arithmetic, closest hit kept as min over (t, index).
@@ -52,29 +53,34 @@ __device__ __forceinline__ void test_sphere_lex(const float4 g, float w, int i, 
     if (t < closest || (t == closest && i < best)) closest = t, best = i;
 }
 
-// slab test of one box against the ray segment (t_lo, t_hi); fminf/fmaxf drop the NaN of 0 * inf
-__device__ __forceinline__ bool hit_box(const float* lo, const float* hi, const Path& p, float ix, float iy, float iz,
-                                        float t_lo, float t_hi, float& t_near) {
-    const float ax = (lo[0] - p.ox) * ix, bx = (hi[0] - p.ox) * ix;
-    const float ay = (lo[1] - p.oy) * iy, by = (hi[1] - p.oy) * iy;
-    const float az = (lo[2] - p.oz) * iz, bz = (hi[2] - p.oz) * iz;
+// slab test of one box against the ray segment (t_lo, t_hi); fminf/fmaxf drop the NaN of 0 * inf.
+// The direct form accepts a root of sphere (c, r) at a point up to 12 eps |c - o|^2 / r outside the sphere (box_reach
+// in rtz_kernels.cuh).  The builder pads every sphere by 1e-6 (1.001 R + |c|)^2 / r, which covers origins with
+// |o|^2 <= r2 = R^2 (the origin test reads |o|^2 (1 - 2^-18)).  A ray from farther out (kFar) widens each box by
+// s = 1e-6 (|m - o| + |h|)^2 max(1/r) instead (m the box's centre, h its half diagonal: |c - o| <= |m - o| + |h|).
+template <bool kFar>
+__device__ __forceinline__ bool hit_box(const float* lo, const float* hi, float inv_r, const Path& p, float ix, float iy,
+                                        float iz, float t_lo, float t_hi, float& t_near) {
+    float s = 0.0f;
+    if (kFar) {
+        const float mx = 0.5f * (lo[0] + hi[0]) - p.ox, my = 0.5f * (lo[1] + hi[1]) - p.oy, mz = 0.5f * (lo[2] + hi[2]) - p.oz;
+        const float hx = 0.5f * (hi[0] - lo[0]), hy = 0.5f * (hi[1] - lo[1]), hz = 0.5f * (hi[2] - lo[2]);
+        const float dist = sqrtf(fmaf(mz, mz, fmaf(my, my, mx * mx))) + sqrtf(fmaf(hz, hz, fmaf(hy, hy, hx * hx)));
+        s = 1e-6f * (dist * dist) * inv_r;
+    }
+    const float ax = (lo[0] - s - p.ox) * ix, bx = (hi[0] + s - p.ox) * ix;
+    const float ay = (lo[1] - s - p.oy) * iy, by = (hi[1] + s - p.oy) * iy;
+    const float az = (lo[2] - s - p.oz) * iz, bz = (hi[2] + s - p.oz) * iz;
     const float tn = fmaxf(fmaxf(fminf(ax, bx), fminf(ay, by)), fmaxf(fminf(az, bz), t_lo));
     const float tf = fminf(fminf(fmaxf(ax, bx), fmaxf(ay, by)), fminf(fmaxf(az, bz), t_hi));
     t_near = tn;
     return tn <= tf;
 }
 
-// Closest hit through the hierarchy.  "While-while" traversal: a warp first walks inner nodes until every lane
-// holds a leaf (or is done), then all lanes test their leaves together, so that box tests and sphere tests
-// are not interleaved lane by lane.  A popped entry whose box lies beyond the current closest hit is skipped.
 constexpr int kBvhDone = (int)0x80000000;
-template <int kBlock>
-__device__ __forceinline__ void bvh_closest_hit(const BvhParams& B, const Path& p, float tmin, float tmax, int* stack,
-                                                float* tstack, float& t_out, int& best_out, unsigned long long& n_tests) {
-    const RayK k = ray_constants(p);
-    const float tmin_d = tmin * p.len;
-    float closest = tmax * p.len;
-    int best = -1;
+template <int kBlock, bool kFar>
+__device__ __forceinline__ void bvh_walk(const BvhParams& B, const Path& p, const RayK& k, float tmin_d, float& closest,
+                                         int& best, int* stack, float* tstack, unsigned long long& n_tests) {
     const float ix = 1.0f / p.dx, iy = 1.0f / p.dy, iz = 1.0f / p.dz;
     const float4* geom = B.p.geom;
     int sp = 0;
@@ -94,8 +100,8 @@ __device__ __forceinline__ void bvh_closest_hit(const BvhParams& B, const Path& 
             const float lo1[3] = {n1.z, n1.w, n2.x}, hi1[3] = {n2.y, n2.z, n2.w};
             const int c0 = __float_as_int(n3.x), c1 = __float_as_int(n3.y);
             float t0, t1;
-            const bool h0 = c0 != kBvhEmpty && hit_box(lo0, hi0, p, ix, iy, iz, tmin_d, closest, t0);
-            const bool h1 = c1 != kBvhEmpty && hit_box(lo1, hi1, p, ix, iy, iz, tmin_d, closest, t1);
+            const bool h0 = c0 != kBvhEmpty && hit_box<kFar>(lo0, hi0, n3.z, p, ix, iy, iz, tmin_d, closest, t0);
+            const bool h1 = c1 != kBvhEmpty && hit_box<kFar>(lo1, hi1, n3.w, p, ix, iy, iz, tmin_d, closest, t1);
             if (h0 && h1) {  // nearer child first, the other on the stack with its entry distance
                 const bool swap = t1 < t0;
                 stack[sp * kBlock] = swap ? c0 : c1;
@@ -117,6 +123,22 @@ __device__ __forceinline__ void bvh_closest_hit(const BvhParams& B, const Path& 
         n_tests += (unsigned)cnt;
         node = pop();
     }
+}
+
+// Closest hit through the hierarchy.  "While-while" traversal: a warp first walks inner nodes until every lane
+// holds a leaf (or is done), then all lanes test their leaves together, so that box tests and sphere tests
+// are not interleaved lane by lane.  A popped entry whose box lies beyond the current closest hit is skipped.
+template <int kBlock>
+__device__ __forceinline__ void bvh_closest_hit(const BvhParams& B, const Path& p, float tmin, float tmax, int* stack,
+                                                float* tstack, float& t_out, int& best_out, unsigned long long& n_tests) {
+    const RayK k = ray_constants(p);
+    const float tmin_d = tmin * p.len;
+    float closest = tmax * p.len;
+    int best = -1;
+    if (-k.nk2 <= B.r2)
+        bvh_walk<kBlock, false>(B, p, k, tmin_d, closest, best, stack, tstack, n_tests);
+    else
+        bvh_walk<kBlock, true>(B, p, k, tmin_d, closest, best, stack, tstack, n_tests);
     t_out = closest, best_out = best;
 }
 
@@ -195,6 +217,21 @@ __global__ void __launch_bounds__(kBlock, kMinBlocks) trace_kernel_bvh(const __g
         atomicAdd(P.stats + 3, v3);
         atomicAdd(P.stats + 4, v4);
     }
+}
+
+// RTZ_SWEEP_BVH (rtz_probe_sweeps): one ray per thread through bvh_closest_hit, with trace_kernel_bvh's stacks
+__global__ void __launch_bounds__(128) probe_bvh_kernel(const __grid_constant__ BvhParams B, const SweepProbeIO io) {
+    __shared__ int s_stack[kBvhMaxDepth * 128];
+    __shared__ float s_tstack[kBvhMaxDepth * 128];
+    const uint64_t k = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (k >= io.m) return;
+    Path p;
+    probe_path(io.rays[k], p);
+    float t;
+    int best;
+    unsigned long long n_tests = 0;
+    bvh_closest_hit<128>(B, p, io.tmin, io.tmax, s_stack + threadIdx.x, s_tstack + threadIdx.x, t, best, n_tests);
+    probe_store(io, k, p, t, best);
 }
 
 }  // namespace rtz

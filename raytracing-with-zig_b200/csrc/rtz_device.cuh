@@ -277,6 +277,12 @@ __device__ __forceinline__ bool hit_record(const float4 g, float inv_r, const Pa
 // exact c = 0 its roots are h - |h| and h + |h|, both <= 0 when h = d.(centre - origin) <= 0 — so the sweep may drop
 // that sphere from its candidates.  The flag (bit 30 of `self`) is set from the very h candidate_root would form.
 constexpr int kSelfLeaves = 0x40000000;
+// h = d.(c - o) of a ray from (px, py, pz) on the sphere of centre g: the ray leaves the sphere when h <= 0 (shade<true>
+// flags it with kSelfLeaves)
+__device__ __forceinline__ float leaving_h(float gx, float gy, float gz, float px, float py, float pz, const Path& p) {
+    const float ocx = gx - px, ocy = gy - py, ocz = gz - pz;
+    return fmaf(p.dz, ocz, fmaf(p.dy, ocy, p.dx * ocx));
+}
 template <bool kFlagSelf = false>
 __device__ __forceinline__ bool shade(const DevCamera& cam, const RngKey& k, const float4* __restrict__ geo,
                                       const float4* __restrict__ aux, const float4* __restrict__ albedo, Path& p,
@@ -356,9 +362,7 @@ __device__ __forceinline__ bool shade(const DevCamera& cam, const RngKey& k, con
     set_direction(p, ndx, ndy, ndz);
     p.self = best;
     if (kFlagSelf) {
-        const float ocx = gx - px, ocy = gy - py, ocz = gz - pz;
-        const float h = fmaf(p.dz, ocz, fmaf(p.dy, ocy, p.dx * ocx));
-        if (!(h > 0.0f)) p.self = best | kSelfLeaves;
+        if (!(leaving_h(gx, gy, gz, px, py, pz, p) > 0.0f)) p.self = best | kSelfLeaves;
     }
     return false;
 }

@@ -1711,24 +1711,140 @@ __global__ void deinterleave_kernel(const uint8_t* __restrict__ gathered, uint64
 // ---------------------------------------------------------------------------------------------
 // probes: one thread per record, the same device functions the render kernel inlines
 // ---------------------------------------------------------------------------------------------
-__global__ void probe_hits_kernel(const float4* geom, const float4* pairs, const float4* aux, int n_pad,
-                                  const rtz_probe_ray* rays, uint64_t m, float tmin, float tmax, rtz_ray_hit* out) {
-    const uint64_t k = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (k >= m) return;
-    const rtz_probe_ray r = rays[k];
-    Path p;
+__device__ __forceinline__ void probe_path(const rtz_probe_ray& r, Path& p) {
     p.ox = r.orig[0], p.oy = r.orig[1], p.oz = r.orig[2], p.self = r.self, p.bounce = 0, p.tr = p.tg = p.tb = 1.f;
     set_direction(p, r.dir[0], r.dir[1], r.dir[2]);
-    float t;
-    int best;
-    sweep_rows(geom, pairs, 0, n_pad, p, tmin, tmax, t, best);
+}
+// the record of closest hit (t, best) of a probe ray; geom / aux are the caller's rows, best the caller's index
+__device__ __forceinline__ rtz_ray_hit probe_record(const float4* geom, const float4* aux, const Path& p, float t,
+                                                    int best) {
     rtz_ray_hit h = {best, 0, t, p.len, {0.f, 0.f, 0.f}, {0.f, 0.f, 0.f}};
     if (best >= 0) {
         float px, py, pz, nx, ny, nz;
         h.front = hit_record(geom[best], aux[best].y, p, t, px, py, pz, nx, ny, nz);
         h.point[0] = px, h.point[1] = py, h.point[2] = pz, h.normal[0] = nx, h.normal[1] = ny, h.normal[2] = nz;
     }
-    out[k] = h;
+    return h;
+}
+
+__global__ void probe_hits_kernel(const float4* geom, const float4* pairs, const float4* aux, int n_pad,
+                                  const rtz_probe_ray* rays, uint64_t m, float tmin, float tmax, rtz_ray_hit* out) {
+    const uint64_t k = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (k >= m) return;
+    Path p;
+    probe_path(rays[k], p);
+    float t;
+    int best;
+    sweep_rows(geom, pairs, 0, n_pad, p, tmin, tmax, t, best);
+    out[k] = probe_record(geom, aux, p, t, best);
+}
+
+// rtz_probe_sweeps: chosen rays through one production sweep, with the template arguments of the kernel that runs
+// it.  Ray `self` arrives in the sweep's slots; hits leave in the caller's indices (through `orig`).
+struct SweepProbeIO {
+    const rtz_probe_ray* rays;
+    uint64_t m;
+    float tmin, tmax;
+    const float4* geom;  // the caller's rows, for the hit records
+    const float4* aux;
+    const int* orig;     // slot -> caller's index (regrouped rows), null = identity
+    rtz_ray_hit* out;
+};
+__device__ __forceinline__ void probe_store(const SweepProbeIO& io, uint64_t k, const Path& p, float t, int slot) {
+    io.out[k] = probe_record(io.geom, io.aux, p, t, slot >= 0 && io.orig ? io.orig[slot] : slot);
+}
+
+// The two-path sweeps (trace_body and trace_body_wave): warp w holds rays 64 w + lane in slot A and
+// 64 w + 32 + lane in slot B; m is a multiple of 64.  Returns false for a warp past the end.
+__device__ __forceinline__ bool probe_pair(const SweepProbeIO& io, Path& a, Path& b, uint64_t& ka) {
+    const uint64_t w = (uint64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+    if (64 * w >= io.m) return false;
+    ka = 64 * w + (threadIdx.x & 31u);
+    probe_path(io.rays[ka], a);
+    probe_path(io.rays[ka + 32], b);
+    return true;
+}
+
+// RTZ_SWEEP_CONST (trace_kernel_const), RTZ_SWEEP_SKIP_SELF (trace_kernel_wave: the flag from shade<true>'s
+// expression) and RTZ_SWEEP_CULL (trace_kernel_const_cull, on the regrouped rows)
+template <bool kSkipSelf, bool kCull>
+__global__ void __launch_bounds__(128) probe_sweep_const_kernel(const __grid_constant__ TraceParamsConst C, const SweepProbeIO io) {
+    __shared__ __align__(16) float stage[4 * kCullStageFloats];
+    Path a, b;
+    uint64_t k;
+    if (!probe_pair(io, a, b, k)) return;
+    if (kSkipSelf) {
+        const float4 ga = C.p.geom[max(a.self, 0)], gb = C.p.geom[max(b.self, 0)];
+        if (a.self >= 0 && !(leaving_h(ga.x, ga.y, ga.z, a.ox, a.oy, a.oz, a) > 0.0f)) a.self |= kSelfLeaves;
+        if (b.self >= 0 && !(leaving_h(gb.x, gb.y, gb.z, b.ox, b.oy, b.oz, b) > 0.0f)) b.self |= kSelfLeaves;
+    }
+    float ta, tb;
+    int ia, ib;
+    if (kCull)
+        sweep2<true, false, true>(C.pairs, C.p.geom, C.p.n_pad, io.tmin, io.tmax, a, b, ta, ia, tb, ib, C.boxes, C.cull_r2,
+                                  C.p.orig, C.p.wexp, C.split_max,
+                                  reinterpret_cast<float4*>(stage + (threadIdx.x >> 5) * kCullStageFloats));
+    else
+        sweep2<true, kSkipSelf>(C.pairs, C.p.geom, C.p.n_pad, io.tmin, io.tmax, a, b, ta, ia, tb, ib);
+    probe_store(io, k, a, ta, ia);
+    probe_store(io, k + 32, b, tb, ib);
+}
+
+// RTZ_SWEEP_SMEM: the rows staged as trace_kernel_smem stages them
+__global__ void __launch_bounds__(128) probe_sweep_smem_kernel(const __grid_constant__ TraceParams P, const SweepProbeIO io) {
+    extern __shared__ __align__(128) unsigned char smem_raw[];
+    float4* s_pairs = reinterpret_cast<float4*>(smem_raw);
+    float4* s_geom = s_pairs + P.n_pad;
+    __shared__ __align__(8) uint64_t s_bar;
+    if (threadIdx.x == 0) {
+        mbar_init(&s_bar, 1);
+        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    }
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        const uint32_t bytes = (uint32_t)P.n_pad * 16u;
+        mbar_expect_tx(&s_bar, 2u * bytes);
+        bulk_g2s(s_pairs, P.pairs, bytes, &s_bar);
+        bulk_g2s(s_geom, P.geom, bytes, &s_bar);
+    }
+    mbar_wait(&s_bar, 0);
+    Path a, b;
+    uint64_t k;
+    if (!probe_pair(io, a, b, k)) return;
+    float ta, tb;
+    int ia, ib;
+    sweep2<false>(s_pairs, s_geom, P.n_pad, io.tmin, io.tmax, a, b, ta, ia, tb, ib);
+    probe_store(io, k, a, ta, ia);
+    probe_store(io, k + 32, b, tb, ib);
+}
+
+// RTZ_SWEEP_GLOBAL: trace_kernel_global's sweep over the rows in global memory
+__global__ void __launch_bounds__(128) probe_sweep_global_kernel(const __grid_constant__ TraceParams P, const SweepProbeIO io) {
+    Path a, b;
+    uint64_t k;
+    if (!probe_pair(io, a, b, k)) return;
+    float ta, tb;
+    int ia, ib;
+    sweep2<false>(P.pairs, P.geom, P.n_pad, io.tmin, io.tmax, a, b, ta, ia, tb, ib);
+    probe_store(io, k, a, ta, ia);
+    probe_store(io, k + 32, b, tb, ib);
+}
+
+// RTZ_SWEEP_COOP / RTZ_SWEEP_COOP_REGROUPED: drain_kernel<true>'s loop, one warp per 32 rays, each ray swept by the
+// whole warp in turn (geom / wexp / orig are the plain or the regrouped rows)
+__global__ void __launch_bounds__(128) probe_coop_kernel(const float4* geom, const float* wexp, const int* orig, int n,
+                                                         const SweepProbeIO io) {
+    const uint64_t k = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    const unsigned lane = threadIdx.x & 31u;
+    Path p;
+    p.ox = p.oy = p.oz = 0.f, p.dx = p.dy = 0.f, p.dz = 1.f, p.len = 1.f, p.self = -1;
+    if (k < io.m) probe_path(io.rays[k], p);
+    const unsigned live = __ballot_sync(0xFFFFFFFFu, k < io.m);
+    float t = 0.f;
+    int best = -1;
+    for (unsigned mm = live; mm; mm &= mm - 1u)
+        coop_hit<false>(geom, wexp, orig, n, io.tmin, io.tmax, p, __ffs(mm) - 1, lane, t, best);
+    if (k < io.m) probe_store(io, k, p, t, best);
 }
 
 __global__ void probe_scatters_kernel(DevCamera cam, const float4* geom, const float4* pairs, const float4* aux,
