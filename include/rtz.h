@@ -104,7 +104,9 @@ typedef struct rtz_camera {
     uint64_t samples_per_pixel;       /* (:88)                                                */
     uint64_t bounce_max;              /* (:90), reference default 50 (:221)                   */
     double pixel_samples_scale;       /* 1/spp (:89), applied as a multiply (:137)            */
-    double t_min, t_max;              /* Scene.interval, (1e-3, +inf)  (src/Scene.zig:21)     */
+    double t_min, t_max;              /* Scene.interval, (1e-3, +inf)  (src/Scene.zig:21);    */
+                                      /* t_min < 0 is refused by the renders (RTZ_ERR_BAD_ARG;*/
+                                      /* -0.0 renders as 0), t_max may be anything but NaN     */
     uint64_t seed;                    /* Scene.seed: key of the counter-based RNG             */
     int32_t has_seed;                 /* 0: the library draws a key from the OS, like         */
                                       /*    Scene.init does with getrandom (src/Scene.zig:33) */
@@ -358,7 +360,10 @@ typedef struct rtz_ray_hit {
     float normal[3];       /* unit, against the ray                                                   */
 } rtz_ray_hit;
 
-/* HittableList.hit(ray, Interval(t_min, t_max)) for m rays (set_direction, then the sweep's gate and root). */
+/* HittableList.hit(ray, Interval(t_min, t_max)) for m rays (set_direction, then the sweep's gate and root).
+ * Any interval is taken, a negative t_min included, as the reference's HittableList.hit takes it (its unit test
+ * uses Interval(-6, 6)): this scalar sweep tests every sphere and both roots against the interval.  The render
+ * calls and rtz_probe_sweeps, whose sweeps rely on t_min >= 0, refuse a negative t_min. */
 int32_t rtz_probe_hits(const rtz_sphere* spheres, uint64_t n_spheres, const rtz_probe_ray* rays, uint64_t m,
                        double t_min, double t_max, rtz_ray_hit* out);
 
@@ -409,10 +414,13 @@ int32_t rtz_probe_cull_bounds(const rtz_sphere* spheres, uint64_t n_spheres, flo
  *   RTZ_SWEEP_COOP             the drain's warp-cooperative sweep, one ray by the whole warp at a time
  *   RTZ_SWEEP_COOP_REGROUPED   the same on the regrouped rows, ties by original index
  *   RTZ_SWEEP_BVH              the RTZ_MODE_PATH_BVH traversal, one ray per thread
+ *   RTZ_SWEEP_WAVE4            the four-path wavefront kernel's sweep over the constant bank (128 paths per warp,
+ *                              up to 512 spheres), which drops the sphere a ray leaves outwards as SKIP_SELF does
  * The two-path kinds (CONST .. GLOBAL) take warps of 64 rays: warp w holds ray 64 w + l in lane l's first slot and
- * 64 w + 32 + l in its second, so m must be a multiple of 64.  RTZ_ERR_BAD_ARG (with rtz_last_error) for null
- * pointers, m > 2^31, an unknown kind, split_max outside 0 .. 64, such an m, a constant-bank kind above 512 spheres,
- * a ray whose self is not -1 or a sphere index, and the spheres rtz_scene_upload refuses. */
+ * 64 w + 32 + l in its second, so m must be a multiple of 64.  RTZ_SWEEP_WAVE4 takes warps of 128 rays, ray
+ * 128 w + l + 32 h in lane l's slot h, so m must be a multiple of 128.  RTZ_ERR_BAD_ARG (with rtz_last_error) for
+ * null pointers, m > 2^31, an unknown kind, split_max outside 0 .. 64, such an m, a constant-bank kind above 512
+ * spheres, t_min < 0, a ray whose self is not -1 or a sphere index, and the spheres rtz_scene_upload refuses. */
 #define RTZ_SWEEP_CONST 0
 #define RTZ_SWEEP_CULL 1
 #define RTZ_SWEEP_SKIP_SELF 2
@@ -421,6 +429,7 @@ int32_t rtz_probe_cull_bounds(const rtz_sphere* spheres, uint64_t n_spheres, flo
 #define RTZ_SWEEP_COOP 5
 #define RTZ_SWEEP_COOP_REGROUPED 6
 #define RTZ_SWEEP_BVH 7
+#define RTZ_SWEEP_WAVE4 8
 int32_t rtz_probe_sweeps(const rtz_sphere* spheres, uint64_t n_spheres, const rtz_probe_ray* rays, uint64_t m,
                          double t_min, double t_max, int32_t kind, int32_t split_max, rtz_ray_hit* out);
 

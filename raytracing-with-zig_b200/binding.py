@@ -69,7 +69,7 @@ GATHER_AUTO, GATHER_P2P, GATHER_NCCL = 0, 1, 2
 ABI_VERSION = 2
 # rtz_probe_sweeps kinds (include/rtz.h)
 (SWEEP_CONST, SWEEP_CULL, SWEEP_SKIP_SELF, SWEEP_SMEM, SWEEP_GLOBAL, SWEEP_COOP, SWEEP_COOP_REGROUPED,
- SWEEP_BVH) = range(8)
+ SWEEP_BVH, SWEEP_WAVE4) = range(9)
 
 # every symbol include/rtz.h declares, with its signature
 _u8p, _f64p, _f32p = C.POINTER(C.c_uint8), C.POINTER(C.c_double), C.POINTER(C.c_float)

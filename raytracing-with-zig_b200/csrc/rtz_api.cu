@@ -170,6 +170,12 @@ int32_t check_camera(const rtz_camera* c) {
         g_last_error = "camera has a non-finite field";
         return RTZ_ERR_BAD_ARG;
     }
+    // the sweeps' exactness rests on t_min >= 0 (DESIGN.md §4): the culled sweep's boxes are tested over [0, closest],
+    // and the sphere a ray leaves has roots h -/+ |h| <= 0; -0.0 compares equal to 0 and is accepted
+    if (c->t_min < 0.0) {
+        g_last_error = "camera t_min is negative";
+        return RTZ_ERR_BAD_ARG;
+    }
     if (c->mode < RTZ_MODE_PATH || c->mode > RTZ_MODE_PATH_BVH) return RTZ_ERR_BAD_ARG;
     if (c->samples_per_pixel == 0 || c->samples_per_pixel > 0x7FFFFFFFull) return RTZ_ERR_BAD_ARG;
     if (c->mode != RTZ_MODE_PATH && c->mode != RTZ_MODE_PATH_BVH && c->samples_per_pixel != 1) return RTZ_ERR_BAD_ARG;
@@ -1706,6 +1712,8 @@ extern "C" {
 
 int32_t rtz_probe_hits(const rtz_sphere* sp, uint64_t n, const rtz_probe_ray* rays, uint64_t m, double tmin,
                        double tmax, rtz_ray_hit* out) {
+    // any interval, a negative t_min included (the reference's HittableList KAT takes Interval(-6, 6)): the scalar
+    // sweep tests every sphere and both roots against it, with none of the render sweeps' t_min >= 0 shortcuts
     if (!sp || !n || (!rays && m) || (!out && m) || m > (1ull << 31)) return RTZ_ERR_BAD_ARG;
     if (!m) return RTZ_OK;
     return run_probe(sp, n, rays, m, out, [&](rtz_context* c, const rtz_probe_ray* din, rtz_ray_hit* dout, unsigned blocks) {
@@ -1805,10 +1813,14 @@ int32_t rtz_probe_sweeps(const rtz_sphere* sp, uint64_t n, const rtz_probe_ray* 
     };
     if (!sp || !n || (!rays && m) || (!out && m)) return refuse("null spheres, rays or output, or no spheres");
     if (n > (1u << 20) || m > (1ull << 31)) return refuse("too many spheres or rays");
-    if (kind < RTZ_SWEEP_CONST || kind > RTZ_SWEEP_BVH) return refuse("unknown sweep kind " + std::to_string(kind));
+    if (kind < RTZ_SWEEP_CONST || kind > RTZ_SWEEP_WAVE4) return refuse("unknown sweep kind " + std::to_string(kind));
     if (split_max < 0 || split_max > 64) return refuse("split_max must lie in 0 .. 64");
-    const bool two_path = kind <= RTZ_SWEEP_GLOBAL, const_bank = kind <= RTZ_SWEEP_SKIP_SELF;
+    if (tmin < 0.0) return refuse("t_min is negative");
+    const bool two_path = kind <= RTZ_SWEEP_GLOBAL;
+    const bool const_bank = kind <= RTZ_SWEEP_SKIP_SELF || kind == RTZ_SWEEP_WAVE4;
     if (two_path && m % 64) return refuse("a two-path sweep takes its rays in warps of 64: m must be a multiple of 64");
+    if (kind == RTZ_SWEEP_WAVE4 && m % 128)
+        return refuse("the four-path sweep takes its rays in warps of 128: m must be a multiple of 128");
     if (const_bank && n > (uint64_t)rtz::kMaxConstSpheres) return refuse("the constant bank holds at most 512 spheres");
     const bool regrouped = kind == RTZ_SWEEP_CULL || kind == RTZ_SWEEP_COOP_REGROUPED;
     // `self` in the sweep's slots
@@ -1846,7 +1858,9 @@ int32_t rtz_probe_sweeps(const rtz_sphere* sp, uint64_t n, const rtz_probe_ray* 
                 std::memcpy(C.pairs, c->h_pairs.data(), (size_t)c->n_pad * sizeof(float4));
             }
             C.p = P;
-            if (kind == RTZ_SWEEP_CONST)
+            if (kind == RTZ_SWEEP_WAVE4)
+                rtz::probe_sweep_wave4_kernel<<<(unsigned)((m / 128 + 3) / 4), 128, 0, c->stream>>>(C, io);
+            else if (kind == RTZ_SWEEP_CONST)
                 rtz::probe_sweep_const_kernel<false, false><<<pair_blocks, 128, 0, c->stream>>>(C, io);
             else if (kind == RTZ_SWEEP_SKIP_SELF)
                 rtz::probe_sweep_const_kernel<true, false><<<pair_blocks, 128, 0, c->stream>>>(C, io);

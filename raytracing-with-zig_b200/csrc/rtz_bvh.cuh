@@ -40,10 +40,9 @@ __device__ __forceinline__ void test_sphere_lex(const float4 g, float w, int i, 
     const float ocx = g.x - p.ox, ocy = g.y - p.oy, ocz = g.z - p.oz;
     const float h = fmaf(p.dz, ocz, fmaf(p.dy, ocy, p.dx * ocx));
     const float c = fmaf(ocz, ocz, fmaf(ocy, ocy, fmaf(ocx, ocx, g.w)));
-    float disc = fmaf(h, h, -c);
+    const float disc = fmaf(h, h, -c);
     if (!(disc >= 0.0f)) return;
-    if (i == p.self) disc = h * h;
-    const float sq = sqrtf(disc);
+    const float sq = (i == p.self) ? fabsf(h) : sqrtf(disc);  // slow_path's exact roots h -/+ |h| on the self sphere
     // the root the ascending loop would accept: the near one if it lies beyond t_min, else the far one
     float t = h - sq;
     if (!(t > tmin_d)) {

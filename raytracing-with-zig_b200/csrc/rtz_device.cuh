@@ -189,8 +189,10 @@ __device__ __forceinline__ bool nearer(float t, int i, float closest, int best, 
 }
 __device__ __forceinline__ void slow_path(float h, float disc, int i, int self, float tmin_d, float& closest,
                                           int& best, const int* __restrict__ orig = nullptr) {
-    if (i == self) disc = h * h;  // exact c = 0 for the sphere we stand on
-    const float sq = sqrtf(disc);
+    // exact c = 0 for the sphere we stand on: roots h -/+ |h| (sqrtf(h * h) exceeds |h| where h * h underflows, and
+    // would put a root of a ray leaving the sphere at h + sqrtf(h * h) > 0)
+    float sq = sqrtf(disc);
+    if (i == self) sq = fabsf(h);
     float t = h - sq;  // (h - sqrtd)/a with a = 1
     if (!(t > tmin_d && nearer(t, i, closest, best, orig))) {  // Interval.surrounds is strict (src/interval.zig:36-38)
         t = h + sq;

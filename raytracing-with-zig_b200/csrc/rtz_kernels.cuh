@@ -1231,6 +1231,72 @@ __device__ __forceinline__ void wave_add_sky_n(const TraceParams& P, const float
     if (sr != sr || sg != sg || sb != sb) atomicAdd(P.stats + 5, 1ULL);
 }
 
+// The sweep of trace_body_wave_n (and of its probe, RTZ_SWEEP_WAVE4): HittableList.hit for the S paths of the lane,
+// path lane + 32 h read from the warp's field rows `w`, over the hit interval (tmin, tmax) in units of |d|.  A path
+// flagged kSelfLeaves does not test the sphere it leaves, as in sweep2<.., true>.  closest[h] / best[h] receive the
+// closest hit in distance units and its sphere (best -1 and closest tmax |d| for none).
+template <int S>
+__device__ __forceinline__ void wave_sweep_n(const float4* __restrict__ pairs, const float4* __restrict__ gather, int n_pad,
+                                             float tmin, float tmax, const float* w, unsigned lane, float (&closest)[S],
+                                             int (&best)[S]) {
+    constexpr int N = WaveN<S>::kPaths;
+    const uint32_t* const wu = reinterpret_cast<const uint32_t*>(w);
+    float dx[S], dy[S], dz[S];
+    RayK k[S];
+#pragma unroll
+    for (int h = 0; h < S; ++h) {
+        const uint32_t s = lane + 32u * h;
+        Path q;
+        q.ox = w[wOx * N + s], q.oy = w[wOy * N + s], q.oz = w[wOz * N + s];
+        q.dx = dx[h] = w[wDx * N + s], q.dy = dy[h] = w[wDy * N + s], q.dz = dz[h] = w[wDz * N + s];
+        k[h] = ray_constants(q);
+        asm volatile("" : "+f"(k[h].tx), "+f"(k[h].ty), "+f"(k[h].tz));
+        closest[h] = tmax * w[wLen * N + s];
+        best[h] = -1;
+    }
+    for (int base = 0; base < n_pad; base += 32) {
+        const int cnt = min(32, n_pad - base);
+        unsigned m[S];
+#pragma unroll
+        for (int h = 0; h < S; ++h) m[h] = 0xFFFFFFFFu;  // 1 = miss
+        const float4* g = pairs + base;
+#pragma unroll 1
+        for (int q0 = 0; q0 < cnt; q0 += 8) {
+#pragma unroll
+            for (int u = 0; u < 8; u += 2) {
+                const float4 p0 = g[q0 + u], p1 = g[q0 + u + 1];
+#pragma unroll
+                for (int h = 0; h < S; ++h) {
+                    Path q;
+                    q.dx = dx[h], q.dy = dy[h], q.dz = dz[h];
+                    test_pair(p0, p1, q, k[h], m[h]);
+                }
+            }
+        }
+        unsigned any = 0;
+#pragma unroll
+        for (int h = 0; h < S; ++h) m[h] = ~m[h], any |= m[h];
+        if (any) {
+#pragma unroll
+            for (int h = 0; h < S; ++h) {
+                if (m[h]) {
+                    const uint32_t s = lane + 32u * h;
+                    const volatile float* wv = w;  // re-read here, not held in registers across the packed loop
+                    const volatile uint32_t* wuv = wu;
+                    Path q;
+                    q.ox = wv[wOx * N + s], q.oy = wv[wOy * N + s], q.oz = wv[wOz * N + s];
+                    q.dx = dx[h], q.dy = dy[h], q.dz = dz[h];
+                    q.self = (int)wuv[wSelf * N + s];
+                    unsigned c = m[h];
+                    const unsigned rel = (unsigned)(q.self & ~kSelfLeaves) - (unsigned)base;
+                    if ((q.self >> 30) == 1 && rel < (unsigned)cnt) c &= ~(1u << (cnt - 1 - (int)rel));
+                    resolve_candidates(gather, c, base, cnt, q, tmin * wv[wLen * N + s], closest[h], best[h]);
+                }
+            }
+        }
+    }
+}
+
 template <int S, int kBlock>
 __device__ __forceinline__ void trace_body_wave_n(const TraceParams& P, const float4* __restrict__ pairs,
                                                   const float4* __restrict__ gather, float* __restrict__ wave_mem) {
@@ -1371,61 +1437,9 @@ __device__ __forceinline__ void trace_body_wave_n(const TraceParams& P, const fl
         if (any_live == 0u) break;
 
         // ---- sweep ----
-        float dx[S], dy[S], dz[S], closest[S];
-        RayK k[S];
+        float closest[S];
         int best[S];
-#pragma unroll
-        for (int h = 0; h < S; ++h) {
-            const uint32_t s = lane + 32u * h;
-            Path q;
-            q.ox = w[wOx * N + s], q.oy = w[wOy * N + s], q.oz = w[wOz * N + s];
-            q.dx = dx[h] = w[wDx * N + s], q.dy = dy[h] = w[wDy * N + s], q.dz = dz[h] = w[wDz * N + s];
-            k[h] = ray_constants(q);
-            asm volatile("" : "+f"(k[h].tx), "+f"(k[h].ty), "+f"(k[h].tz));
-            closest[h] = cam.tmax * w[wLen * N + s];
-            best[h] = -1;
-        }
-        for (int base = 0; base < P.n_pad; base += 32) {
-            const int cnt = min(32, P.n_pad - base);
-            unsigned m[S];
-#pragma unroll
-            for (int h = 0; h < S; ++h) m[h] = 0xFFFFFFFFu;  // 1 = miss
-            const float4* g = pairs + base;
-#pragma unroll 1
-            for (int q0 = 0; q0 < cnt; q0 += 8) {
-#pragma unroll
-                for (int u = 0; u < 8; u += 2) {
-                    const float4 p0 = g[q0 + u], p1 = g[q0 + u + 1];
-#pragma unroll
-                    for (int h = 0; h < S; ++h) {
-                        Path q;
-                        q.dx = dx[h], q.dy = dy[h], q.dz = dz[h];
-                        test_pair(p0, p1, q, k[h], m[h]);
-                    }
-                }
-            }
-            unsigned any = 0;
-#pragma unroll
-            for (int h = 0; h < S; ++h) m[h] = ~m[h], any |= m[h];
-            if (any) {
-#pragma unroll
-                for (int h = 0; h < S; ++h) {
-                    if (m[h]) {
-                        const uint32_t s = lane + 32u * h;
-                        const volatile float* wv = w;  // re-read here, not held in registers across the packed loop
-                        const volatile uint32_t* wuv = wu;
-                        Path q;
-                        q.ox = wv[wOx * N + s], q.oy = wv[wOy * N + s], q.oz = wv[wOz * N + s];
-                        q.dx = dx[h], q.dy = dy[h], q.dz = dz[h];
-                        q.self = (int)wuv[wSelf * N + s];
-                        unsigned c = m[h];
-                        const unsigned rel = (unsigned)(q.self & ~kSelfLeaves) - (unsigned)base;
-                        if ((q.self >> 30) == 1 && rel < (unsigned)cnt) c &= ~(1u << (cnt - 1 - (int)rel));
-                        resolve_candidates(gather, c, base, cnt, q, cam.tmin * wv[wLen * N + s], closest[h], best[h]);
-                    }
-                }
-            }
-        }
+        wave_sweep_n<S>(pairs, gather, P.n_pad, cam.tmin, cam.tmax, w, lane, closest, best);
         unsigned hit = 0u;
 #pragma unroll
         for (int h = 0; h < S; ++h) {
@@ -1788,6 +1802,38 @@ __global__ void __launch_bounds__(128) probe_sweep_const_kernel(const __grid_con
         sweep2<true, kSkipSelf>(C.pairs, C.p.geom, C.p.n_pad, io.tmin, io.tmax, a, b, ta, ia, tb, ib);
     probe_store(io, k, a, ta, ia);
     probe_store(io, k + 32, b, tb, ib);
+}
+
+// RTZ_SWEEP_WAVE4: trace_kernel_wave_n<4, ..>'s sweep.  Warp w writes ray 128 w + lane + 32 h into slot h of its field
+// rows, flagged as shade<true> flags it (as RTZ_SWEEP_SKIP_SELF does); m is a multiple of 128.
+__global__ void __launch_bounds__(128) probe_sweep_wave4_kernel(const __grid_constant__ TraceParamsConst C, const SweepProbeIO io) {
+    constexpr int S = 4, N = WaveN<S>::kPaths;
+    __shared__ float wave_mem[4 * WaveN<S>::kWords];
+    float* const w = wave_mem + (threadIdx.x >> 5) * WaveN<S>::kWords;
+    uint32_t* const wu = reinterpret_cast<uint32_t*>(w);
+    const unsigned lane = threadIdx.x & 31u;
+    const uint64_t k0 = N * ((uint64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5)) + lane;
+    if (k0 >= io.m) return;  // the whole warp: m is a multiple of 128
+    Path p[S];
+#pragma unroll
+    for (int h = 0; h < S; ++h) {
+        const uint32_t s = lane + 32u * h;
+        probe_path(io.rays[k0 + 32 * h], p[h]);
+        int self = p[h].self;
+        if (self >= 0) {
+            const float4 g = C.p.geom[self];
+            if (!(leaving_h(g.x, g.y, g.z, p[h].ox, p[h].oy, p[h].oz, p[h]) > 0.0f)) self |= kSelfLeaves;
+        }
+        w[wOx * N + s] = p[h].ox, w[wOy * N + s] = p[h].oy, w[wOz * N + s] = p[h].oz;
+        w[wDx * N + s] = p[h].dx, w[wDy * N + s] = p[h].dy, w[wDz * N + s] = p[h].dz;
+        w[wLen * N + s] = p[h].len, wu[wSelf * N + s] = (uint32_t)self;
+    }
+    __syncwarp();
+    float closest[S];
+    int best[S];
+    wave_sweep_n<S>(C.pairs, C.p.geom, C.p.n_pad, io.tmin, io.tmax, w, lane, closest, best);
+#pragma unroll
+    for (int h = 0; h < S; ++h) probe_store(io, k0 + 32 * h, p[h], closest[h], best[h]);
 }
 
 // RTZ_SWEEP_SMEM: the rows staged as trace_kernel_smem stages them

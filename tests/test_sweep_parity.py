@@ -3,7 +3,8 @@
 test_ray_parity.py ties the mirror to the f64 reference ray by ray, and the device's scalar probe sweep to the
 mirror.  The render kernels find their closest hits with other code: the packed two-path sweep over the constant
 bank, shared memory or global memory; its culled form (padded block boxes, regrouped rows, the sphere-parallel
-pass); the wavefront kernel's sweep that drops the sphere a ray leaves; the drain's warp-cooperative sweep; the BVH
+pass); the wavefront kernels' sweeps that drop the sphere a ray leaves (two paths per lane, and the four-path kernel's
+own sweep over 128 paths per warp); the drain's warp-cooperative sweep; the BVH
 traversal.  rtz_probe_sweeps runs each of them, with the render kernel's template arguments, on rays the tests
 choose, and every result must equal the mirror's bit for bit.
 
@@ -16,6 +17,8 @@ check that each new family stays within the f64 error model on the mirror, so th
 "within the error model", and that rtz_probe_cull_bounds gives the documented block boxes.
 """
 import ctypes as C
+import re
+import subprocess
 
 import numpy as np
 import pytest
@@ -25,8 +28,8 @@ from test_block_regroup import _scene as _tie_scene
 from test_ray_parity import (HIT, RAY, TMIN, TRANSLATIONS, _camera_rays, _check, _families, _mirror_hits,
                              _moved_camera, _ptr, _rays, _secondary, _sweep_scene, _translated, _unit)
 
-CONST, CULL, SKIP_SELF, SMEM, GLOBAL, COOP, COOP_REGROUPED, BVH = range(8)
-NAMES = ["CONST", "CULL", "SKIP_SELF", "SMEM", "GLOBAL", "COOP", "COOP_REGROUPED", "BVH"]
+CONST, CULL, SKIP_SELF, SMEM, GLOBAL, COOP, COOP_REGROUPED, BVH, WAVE4 = range(9)
+NAMES = ["CONST", "CULL", "SKIP_SELF", "SMEM", "GLOBAL", "COOP", "COOP_REGROUPED", "BVH", "WAVE4"]
 CULL_SIZES = [65, 200, 257, 485, 511, 512]  # 485 is the book's final scene; the rest sweep scenes
 F32 = np.float32
 
@@ -381,15 +384,16 @@ def _probe(pkg, sp, n, rays, kind, tmin=TMIN, tmax=np.inf, split=16):
     return out
 
 
-def _pad64(rays):
-    k = (-len(rays)) % 64
+def _pad128(rays):
+    """Whole warps for every kind: 64 rays for the two-path sweeps, 128 for WAVE4."""
+    k = (-len(rays)) % 128
     return np.concatenate([rays, np.resize(rays, k)]) if k else rays
 
 
 def _kinds(n):
     k = [GLOBAL, COOP, COOP_REGROUPED, BVH]
     if n <= 512:
-        k = [CONST, CULL, SKIP_SELF] + k
+        k = [CONST, CULL, SKIP_SELF, WAVE4] + k
     if n <= 6000:
         k.append(SMEM)
     return k
@@ -397,7 +401,7 @@ def _kinds(n):
 
 def _same(pkg, orc, sp, n, rays, label, kinds=None, tmin=TMIN, tmax=np.inf, splits=(16,)):
     """Every kind equals the mirror bit for bit; returns the list of disagreements."""
-    rays = _pad64(rays)
+    rays = _pad128(rays)
     want = _mirror_hits(orc, sp, n, rays, tmin, tmax)
     bad = []
     for kind in kinds if kinds is not None else _kinds(n):
@@ -501,7 +505,8 @@ def test_ties_and_self_with_a_finite_t_max(pkg, gpu, orc):
 
 SIZES = {CONST: [65, 200, 257, 485, 511, 512], SKIP_SELF: [65, 200, 257, 485, 511, 512],
          CULL: [65, 200, 257, 485, 511, 512], SMEM: [513, 4096, 6000], GLOBAL: [8192, 16384],
-         COOP: [1, 31, 33, 64, 485], COOP_REGROUPED: [1, 31, 33, 64, 485]}
+         COOP: [1, 31, 33, 64, 485], COOP_REGROUPED: [1, 31, 33, 64, 485],
+         WAVE4: [33, 64, 65, 128, 200, 256, 257, 512]}
 
 
 @pytest.mark.gpu
@@ -543,7 +548,7 @@ def test_malformed_calls_are_refused(pkg, gpu, orc):
     P = C.POINTER(pkg.rtz_sphere)
     sp, n = _scene(orc, 485), 485
     rng = np.random.default_rng(3)
-    rays = _pad64(_c3_rays(orc, (0.0, 0.0, 0.0), rng, pixels=16))
+    rays = _pad128(_c3_rays(orc, (0.0, 0.0, 0.0), rng, pixels=16))
     out = np.zeros(len(rays), HIT)
     ok = (C.cast(sp, P), n, _ptr(rays), len(rays), TMIN, np.inf, CONST, 16, _ptr(out))
 
@@ -555,15 +560,16 @@ def test_malformed_calls_are_refused(pkg, gpu, orc):
 
     assert call() == 0
     refused = [dict(sp=None), dict(n=0), dict(rays=None), dict(out=None), dict(m=(1 << 31) + 64), dict(kind=-1),
-               dict(kind=8), dict(split=-1), dict(split=65), dict(m=63), dict(m=32, kind=GLOBAL)]
+               dict(kind=9), dict(split=-1), dict(split=65), dict(m=63), dict(m=32, kind=GLOBAL),
+               dict(m=64, kind=WAVE4)]
     big = _scene(orc, 513)
-    refused += [dict(sp=C.cast(big, P), n=513, kind=k) for k in (CONST, CULL, SKIP_SELF)]
+    refused += [dict(sp=C.cast(big, P), n=513, kind=k) for k in (CONST, CULL, SKIP_SELF, WAVE4)]
     for r in refused:
         assert call(**r) == 1, r
     selfish = rays.copy()
     for s in (-2, n):
         selfish["self"][5] = s
-        for kind in (SKIP_SELF, CULL, COOP_REGROUPED):
+        for kind in (SKIP_SELF, CULL, COOP_REGROUPED, WAVE4):
             assert call(rays=_ptr(selfish), kind=kind) == 1, (s, kind)
     assert b"self" in l.rtz_last_error()
     bad = R.sphere_array([R.make_sphere((0, 0, 0), 0.0, R.MAT_LAMBERTIAN)])
@@ -600,3 +606,21 @@ def test_malformed_calls_are_refused(pkg, gpu, orc):
         l.rtz_context_destroy(c)
     assert held > 0
     assert min(drop(refuse) for _ in range(3)) < held / 2
+
+
+def test_four_path_wavefront_kernel_keeps_its_registers_and_the_uniform_sweep(pkg):
+    """Codegen guard (no GPU needed): the four-path wavefront kernel, whose sweep RTZ_SWEEP_WAVE4 probes through the
+    same inlined function, must not spill, must keep its sphere operands in uniform registers and must not diverge."""
+    out = subprocess.run(["cuobjdump", "-sass", str(pkg.binding.LIB_PATH)], capture_output=True, text=True).stdout
+    body, name = {}, None
+    for line in out.splitlines():
+        if "Function :" in line:
+            name = line.split("Function :")[1].strip()
+        elif name:
+            body.setdefault(name, []).append(line)
+    wave = [k for k in body if "trace_kernel_wave_nILi4ELi128ELi6" in k]
+    assert len(wave) == 1, wave
+    sass = "\n".join(body[wave[0]])
+    assert not re.search(r"\b(STL|LDL)\b", sass), "the four-path wavefront kernel spills to local memory"
+    assert len(re.findall(r"FFMA2 [^;]*UR\d+\.F32x2", sass)) >= 48
+    assert "BRA.DIV" not in sass

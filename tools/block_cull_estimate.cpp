@@ -50,10 +50,9 @@ float accepted_root(const MSphere& s, int i, const Path& p, float tmin_d) {
     const float ocx = s.cx - p.o.x, ocy = s.cy - p.o.y, ocz = s.cz - p.o.z;
     const float h = std::fmaf(p.d.z, ocz, std::fmaf(p.d.y, ocy, p.d.x * ocx));
     const float c = std::fmaf(ocz, ocz, std::fmaf(ocy, ocy, std::fmaf(ocx, ocx, -s.r2)));
-    float disc = std::fmaf(h, h, -c);
+    const float disc = std::fmaf(h, h, -c);
     if (!(disc >= 0.0f)) return INFINITY;
-    if (i == p.self) disc = h * h;
-    const float sq = std::sqrt(disc);
+    const float sq = i == p.self ? std::fabs(h) : std::sqrt(disc);
     float t = h - sq;
     if (t > tmin_d) return t;
     t = h + sq;
