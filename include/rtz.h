@@ -224,6 +224,16 @@ int32_t rtz_render_resident_linear(rtz_context* ctx, const rtz_camera* camera, c
 int32_t rtz_render_guides(rtz_context* ctx, const rtz_camera* camera, uint64_t guide_samples,
                           float* d_albedo_out, float* d_normal_out, rtz_stats* stats_out);
 
+/* rtz_render_guides for this rank's tiles (rtz_shard): the outputs are DEVICE buffers of 3 f32 per pixel for
+ * rtz_shard_pixels(...) pixels in the compact tile layout of rtz_render_resident, tile-padding pixels 0.  Every pixel's
+ * values are the whole frame's (its rays are keyed by its global index y*width + x), so the shards' buffers, gathered
+ * and passed through rtz_deinterleave_f32, equal rtz_render_guides bit for bit.  shard == NULL is rtz_render_guides.
+ * RTZ_ERR_BAD_ARG as rtz_render_guides (the 2^31 - 1 work items count the shard's padded pixels), and for a shard
+ * with rank >= world or a zero tile size.  stats as rtz_render_guides, samples = segments = the shard's pixels
+ * (padding excluded) * guide_samples. */
+int32_t rtz_render_guides_sharded(rtz_context* ctx, const rtz_camera* camera, const rtz_shard* shard,
+                                  uint64_t guide_samples, float* d_albedo_out, float* d_normal_out, rtz_stats* stats_out);
+
 /* ---- denoiser: edge-avoiding à-trous wavelet filter (Dammertz et al. 2010) over the linear colour, guided by the
  * first-hit albedo and normal above ---------------------------------------------------------------------------
  * Per pixel the colour is demodulated by the albedo (e = c / max(a, 2^-8)), filtered in `levels` passes of 5x5 taps
@@ -231,7 +241,8 @@ int32_t rtz_render_guides(rtz_context* ctx, const rtz_camera* camera, uint64_t g
  * squared differences of e (scaled by 4^k / sigma_color^2 at level k), of the normal (1 / sigma_normal^2) and of the
  * albedo (1 / sigma_albedo^2), then remodulated; a tap at x >= 64 contributes nothing.  The bytes are Color.toRgb of
  * the f32 result, as the resolve forms them.  IEEE f32 arithmetic in a fixed order (DESIGN.md §5 K7): the output is
- * reproducible bit for bit.  The filter needs the whole frame: shards and multi-GPU frames are not supported. */
+ * reproducible bit for bit.  The filter runs on one device over the whole frame; a sharded or multi-GPU frame brings
+ * its linear colour and guides to that device first (rtz_deinterleave_f32, rtz_multi_render_denoised). */
 typedef struct rtz_denoise_params {
     uint32_t levels;       /* à-trous levels, step 2^k for k < levels; 0 = copy; <= 8                       */
     uint32_t reserved;     /* must be 0                                                                     */
@@ -258,7 +269,8 @@ int32_t rtz_denoise(rtz_context* ctx, uint64_t width, uint64_t height, const flo
  * guide_samples 0 = min(samples_per_pixel, 16).  has_seed == 0: ONE seed is drawn and keys both the render and the
  * guides (stats_out->seed_used reports it).  rgb_out (3 bytes per pixel) and linear_out (3 f32 per pixel, the
  * denoised linear colour) are HOST buffers; either may be NULL, not both.  RTZ_ERR_BAD_ARG as rtz_render and
- * rtz_denoise, and for a legacy mode or guide_samples > samples_per_pixel.  The frame is whole: no shards, one GPU.
+ * rtz_denoise, and for a legacy mode or guide_samples > samples_per_pixel.  One GPU; rtz_render_multi_denoised is
+ * the same frame on N.
  * stats: the render's counters as rtz_render reports them; kernel_launches counts every launch of the call and
  * total_ms runs from the first launch to the denoised bytes. */
 int32_t rtz_render_denoised(const rtz_camera* camera, const rtz_sphere* spheres, uint64_t n_spheres,
@@ -271,6 +283,12 @@ int32_t rtz_render_denoised(const rtz_camera* camera, const rtz_sphere* spheres,
 int32_t rtz_deinterleave(rtz_context* ctx, uint64_t width, uint64_t height, uint32_t world,
                          uint32_t tile_w, uint32_t tile_h, const uint8_t* d_gathered,
                          uint8_t* d_rgb_out);
+
+/* The same for 3 f32 per pixel (the linear colour of rtz_render_resident_linear, the guides of
+ * rtz_render_guides_sharded): `d_gathered` holds `world` compact buffers back to back, `d_out` (device) receives
+ * width*height*3 f32, row-major.  Arguments and refusals as rtz_deinterleave. */
+int32_t rtz_deinterleave_f32(rtz_context* ctx, uint64_t width, uint64_t height, uint32_t world,
+                             uint32_t tile_w, uint32_t tile_h, const float* d_gathered, float* d_out);
 
 /* ---- N GPUs of ONE box behind the same call (north_star: "rendered on 8xB200" as a drop-in for
  * Camera.render; SURVEY.md 8b `num_gpus`, 8e "single process ... no host MPI").  ONE host process, no
@@ -309,6 +327,25 @@ int32_t rtz_multi_render(rtz_multi* multi, const rtz_camera* camera, uint8_t* rg
  * created rtz_multi per device count, like rtz_render keeps one context. */
 int32_t rtz_render_multi(const rtz_camera* camera, const rtz_sphere* spheres, uint64_t n_spheres,
                          int32_t num_gpus, uint8_t* rgb_out, rtz_stats* stats_out);
+
+/* rtz_render_denoised on all devices of `multi`: the same bytes and the same f32 linear colour, bit for bit, for any
+ * device count, tile size and transport.  Every device traces its tiles, resolves their linear colour in f32 and runs
+ * the guide kernel over them on its own stream (all enqueued before the first wait); the three f32 planes reach
+ * device 0 either (P2P) stored straight into its row-major planes through peer memory, or (NCCL) as compact buffers
+ * over one grouped ncclSend/ncclRecv, de-interleaved there.  Device 0 then denoises the whole frame.  One device is
+ * rtz_render_denoised on it.  Arguments, defaults (guide_samples 0 = min(spp, 16); has_seed == 0: ONE seed for the
+ * frame, reported in seed_used) and refusals as rtz_render_denoised; rgb_out / linear_out are HOST buffers.
+ * stats: the render's counters summed over the devices (the guide rays are not samples); kernel_launches counts every
+ * launch; trace_ms = slowest device's path trace; gather_ms = first launch -> the denoiser's inputs complete on
+ * device 0, minus trace_ms (it holds the guide kernels and the exchange); total_ms = first launch -> denoised bytes on
+ * device 0; gpus, gather and seed_used as rtz_multi_render. */
+int32_t rtz_multi_render_denoised(rtz_multi* multi, const rtz_camera* camera, uint64_t guide_samples,
+                                  const rtz_denoise_params* params, uint8_t* rgb_out, float* linear_out,
+                                  rtz_stats* stats_out);
+/* One-shot form with HOST buffers on num_gpus devices (<= 0: all), on the rtz_multi rtz_render_multi keeps. */
+int32_t rtz_render_multi_denoised(const rtz_camera* camera, const rtz_sphere* spheres, uint64_t n_spheres,
+                                  int32_t num_gpus, uint64_t guide_samples, const rtz_denoise_params* params,
+                                  uint8_t* rgb_out, float* linear_out, rtz_stats* stats_out);
 
 /* ---- device-side unit probes (one ray; used by the KATs that mirror the reference's
  * own unit tests, src/sphere.zig:76-136, src/hittable.zig:185-209,

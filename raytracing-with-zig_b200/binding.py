@@ -87,11 +87,14 @@ SIGNATURES = {
     "rtz_render_resident_linear": (_i32, [_vp, C.POINTER(rtz_camera), C.POINTER(rtz_shard), _vp, _vp,
                                           C.POINTER(rtz_stats)]),
     "rtz_render_guides": (_i32, [_vp, C.POINTER(rtz_camera), _u64, _vp, _vp, C.POINTER(rtz_stats)]),
+    "rtz_render_guides_sharded": (_i32, [_vp, C.POINTER(rtz_camera), C.POINTER(rtz_shard), _u64, _vp, _vp,
+                                         C.POINTER(rtz_stats)]),
     "rtz_denoise": (_i32, [_vp, _u64, _u64, _vp, _vp, _vp, C.POINTER(rtz_denoise_params), _vp, _vp,
                            C.POINTER(rtz_stats)]),
     "rtz_render_denoised": (_i32, [C.POINTER(rtz_camera), C.POINTER(rtz_sphere), _u64, _u64,
                                    C.POINTER(rtz_denoise_params), _u8p, _f32p, C.POINTER(rtz_stats)]),
     "rtz_deinterleave": (_i32, [_vp, _u64, _u64, _u32, _u32, _u32, _vp, _vp]),
+    "rtz_deinterleave_f32": (_i32, [_vp, _u64, _u64, _u32, _u32, _u32, _vp, _vp]),
     "rtz_multi_create": (_i32, [_i32, C.POINTER(_i32), _u32, _u32, _i32, C.POINTER(_vp)]),
     "rtz_multi_destroy": (_i32, [_vp]),
     "rtz_multi_gpus": (_i32, [_vp]),
@@ -99,6 +102,10 @@ SIGNATURES = {
     "rtz_multi_scene_upload": (_i32, [_vp, C.POINTER(rtz_sphere), _u64]),
     "rtz_multi_render": (_i32, [_vp, C.POINTER(rtz_camera), _u8p, C.POINTER(_vp), C.POINTER(rtz_stats)]),
     "rtz_render_multi": (_i32, [C.POINTER(rtz_camera), C.POINTER(rtz_sphere), _u64, _i32, _u8p, C.POINTER(rtz_stats)]),
+    "rtz_multi_render_denoised": (_i32, [_vp, C.POINTER(rtz_camera), _u64, C.POINTER(rtz_denoise_params), _u8p, _f32p,
+                                         C.POINTER(rtz_stats)]),
+    "rtz_render_multi_denoised": (_i32, [C.POINTER(rtz_camera), C.POINTER(rtz_sphere), _u64, _i32, _u64,
+                                         C.POINTER(rtz_denoise_params), _u8p, _f32p, C.POINTER(rtz_stats)]),
     "rtz_probe_hit": (_i32, [C.POINTER(rtz_sphere), _u64, D3, D3, _f64, _f64, C.POINTER(rtz_hit)]),
     "rtz_probe_scatter": (_i32, [C.POINTER(rtz_sphere), _u64, _i32, D3, D3, _u64, _u32, _u32, _u32,
                                  C.POINTER(rtz_scatter)]),

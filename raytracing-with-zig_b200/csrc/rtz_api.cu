@@ -137,8 +137,8 @@ struct rtz_context {
     // linear colour, albedo, normal and denoised linear colour (3 f32 per pixel each)
     DevBuf<float4> denoise;
     DevBuf<float> denoise_io;
-    // [0..3] a frame's phases, [4..5] the span of rtz_render_denoised
-    cudaEvent_t ev[6] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
+    // [0..3] a frame's phases, [4..5] the span of rtz_render_denoised, [6..7] the guide kernel
+    cudaEvent_t ev[8] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
     unsigned long long* h_counters = nullptr;  // pinned
 };
 
@@ -249,14 +249,32 @@ cudaError_t smem_rows_fit(const rtz_context* ctx, bool& fits) {
 // render asks for it, so that plain uploads (and every brute-force frame) never pay for it.
 int32_t ensure_bvh(rtz_context* c);
 
-// What one device contributes to a frame.  `image` set: the resolve stores every channel at its place in the
-// ROW-MAJOR image (possibly peer memory of device 0) instead of the compact tile buffer `d_rgb`.
+// What one device contributes to a frame.  `image` / `image_linear32` set: the resolve stores every channel at its
+// place in the ROW-MAJOR image (possibly peer memory of device 0) instead of the compact tile buffer `d_rgb`.
 struct FrameTarget {
     uint8_t* d_rgb = nullptr;
     double* d_linear = nullptr;
     float* d_linear32 = nullptr;
     uint8_t* image = nullptr;
+    float* image_linear32 = nullptr;
 };
+
+// the pixels of the frame in the shard's tiles (without the padding of the compact layout)
+uint64_t shard_real_pixels(const rtz_camera* cam, const rtz::ShardGeom& sg) {
+    uint64_t px = 0;
+    for (uint32_t t = sg.rank; t < (uint64_t)sg.tiles_x * sg.tiles_y; t += sg.world) {
+        const uint32_t ty = t / sg.tiles_x, tx = t - ty * sg.tiles_x;
+        const uint64_t w = std::min<uint64_t>(sg.tile_w, cam->width - (uint64_t)tx * sg.tile_w);
+        const uint64_t h = std::min<uint64_t>(sg.tile_h, cam->height - (uint64_t)ty * sg.tile_h);
+        px += w * h;
+    }
+    return px;
+}
+
+// ceil(2^64 / d) for rtz::div_by; 0 stands for d = 1
+unsigned long long rcp(uint64_t d) {
+    return d <= 1 ? 0ull : (unsigned long long)(((unsigned __int128)1 << 64) / d) + 1ull;  // d never divides 2^64 unless a power of two: then +1 overshoots by one ulp, still exact for n < 2^32
+}
 
 // Enqueue the frame (memsets, trace kernel, resolve, counter read-back) on the context's stream; no host wait.
 int32_t enqueue_path(rtz_context* ctx, const rtz_camera* cam, const rtz::ShardGeom& sg, const FrameTarget& out,
@@ -284,9 +302,6 @@ int32_t enqueue_path(rtz_context* ctx, const rtz_camera* cam, const rtz::ShardGe
         // sweeping those r paths once more (r/64 of a sweep); measured optimum (same-box A/B, profiles/r2_wave_ab.txt):
         // 16 of 32 lanes up to 32 spheres, 12 at 64, 8 from 128 on
         P.wave_shade_min = P.wave_regen_min = ctx->n_pad <= 32 ? 16u : ctx->n_pad <= 64 ? 12u : 8u;
-        auto rcp = [](uint64_t d) -> unsigned long long {  // ceil(2^64 / d); 0 stands for d = 1
-            return d <= 1 ? 0ull : (unsigned long long)(((unsigned __int128)1 << 64) / d) + 1ull;  // d never divides 2^64 unless a power of two: then +1 overshoots by one ulp, still exact for n < 2^32
-        };
         P.rcp_tile_pixels = rcp(sg.tile_pixels), P.rcp_tiles_x = rcp(sg.tiles_x), P.rcp_tile_w = rcp(sg.tile_w);
         P.rcp_chunks_per_pixel = rcp(P.chunks_per_pixel);
         if (const char* e = std::getenv("RTZ_WAVE_SHADE_MIN")) P.wave_shade_min = (uint32_t)std::min(32, std::max(1, std::atoi(e)));
@@ -411,9 +426,10 @@ int32_t enqueue_path(rtz_context* ctx, const rtz_camera* cam, const rtz::ShardGe
     }
     RTZ_CUDA(cudaEventRecord(ctx->ev[2], ctx->stream));
     const uint64_t n3 = 3 * n_local_pixels;
-    if (out.image)
+    if (out.image || out.image_linear32)
         rtz::resolve_scatter_kernel<<<(unsigned)((n3 + 255) / 256), 256, 0, ctx->stream>>>(
-            ctx->accum.p, sg, (uint32_t)cam->width, (uint32_t)cam->height, cam->pixel_samples_scale, out.image);
+            ctx->accum.p, sg, (uint32_t)cam->width, (uint32_t)cam->height, cam->pixel_samples_scale, out.image,
+            out.image_linear32);
     else
         rtz::resolve_kernel<<<(unsigned)((n3 + 255) / 256), 256, 0, ctx->stream>>>(
             ctx->accum.p, n_local_pixels, cam->pixel_samples_scale, out.d_rgb, out.d_linear, out.d_linear32);
@@ -440,16 +456,8 @@ int32_t collect_path(rtz_context* ctx, const rtz_camera* cam, const rtz::ShardGe
     if (st) {
         std::memset(st, 0, sizeof(*st));
         st->samples = ctx->h_counters[1], st->segments = ctx->h_counters[2];
-        if (cam->bounce_max == 0) {  // counted on the host: the kernel did not run
-            uint64_t px = 0;
-            for (uint32_t t = sg.rank; t < (uint64_t)sg.tiles_x * sg.tiles_y; t += sg.world) {
-                const uint32_t ty = t / sg.tiles_x, tx = t - ty * sg.tiles_x;
-                const uint64_t w = std::min<uint64_t>(sg.tile_w, cam->width - (uint64_t)tx * sg.tile_w);
-                const uint64_t h = std::min<uint64_t>(sg.tile_h, cam->height - (uint64_t)ty * sg.tile_h);
-                px += w * h;
-            }
-            st->samples = px * cam->samples_per_pixel;
-        }
+        if (cam->bounce_max == 0)  // counted on the host: the kernel did not run
+            st->samples = shard_real_pixels(cam, sg) * cam->samples_per_pixel;
         st->depth_capped = ctx->h_counters[3], st->absorbed = ctx->h_counters[4];
         st->sphere_tests = cam->mode == RTZ_MODE_PATH_BVH ? ctx->h_counters[5] : st->segments * (uint64_t)ctx->n_spheres;
         st->nan_samples = ctx->h_counters[6];
@@ -560,6 +568,77 @@ int32_t enqueue_denoise(rtz_context* c, uint32_t W, uint32_t H, const float* col
     rtz::denoise_finish_kernel<<<(unsigned)tiles, block, 0, c->stream>>>(e, color, albedo, linear_out, rgb_out, W, H,
                                                                          tiles_x);
     RTZ_CUDA(cudaGetLastError());
+    return RTZ_OK;
+}
+
+// Refusals of the guide pass (beyond check_camera): its rays are keyed by the frame's seed, which an OS-drawn seed
+// would not repeat
+int32_t check_guides(const rtz_camera* cam, uint64_t guide_samples) {
+    if (cam->mode != RTZ_MODE_PATH && cam->mode != RTZ_MODE_PATH_BVH) return RTZ_ERR_BAD_ARG;
+    if (!cam->has_seed || guide_samples == 0 || guide_samples > cam->samples_per_pixel) return RTZ_ERR_BAD_ARG;
+    return RTZ_OK;
+}
+
+// Enqueue the guide kernel over the local pixels of shard `sg` (K6) on the context's stream, between ev[6] and ev[7];
+// no host wait.  Outputs compact (padding 0) or, `row_major`, at their places in row-major planes.
+int32_t enqueue_guides(rtz_context* c, const rtz_camera* cam, const rtz::ShardGeom& sg, uint64_t guide_samples,
+                       float* d_albedo, float* d_normal, bool row_major) {
+    const uint64_t n_local = (uint64_t)sg.n_local_tiles * sg.tile_pixels;
+    rtz::GuideParams P{};
+    P.cam = to_dev_camera(*cam, cam->seed);
+    P.pairs = c->pairs.p, P.geom = c->geom.p, P.aux = c->aux.p, P.albedo = c->albedo.p, P.wexp = c->wexp.p;
+    P.orig = nullptr;
+    P.n_pad = c->n_pad;
+    P.g = (uint32_t)guide_samples;
+    P.pix_per_item = guide_samples >= 64 ? 1u : (uint32_t)(64 / guide_samples);
+    const uint64_t n_items = (n_local + P.pix_per_item - 1) / P.pix_per_item;
+    if (n_items > 0x7FFFFFFFull) return RTZ_ERR_BAD_ARG;  // one block (warp) per item: the grid's x limit
+    P.n_items = (uint32_t)n_items;
+    P.sh = sg, P.n_local = (uint32_t)n_local, P.row_major = row_major ? 1u : 0u;
+    P.rcp_tile_pixels = rcp(sg.tile_pixels), P.rcp_tiles_x = rcp(sg.tiles_x), P.rcp_tile_w = rcp(sg.tile_w);
+    P.albedo_out = d_albedo, P.normal_out = d_normal;
+    const unsigned blocks = P.n_items;
+    // every mode sweeps by brute force here (the BVH finds the same hits), on the rows the render's sweep reads
+    RTZ_CUDA(cudaEventRecord(c->ev[6], c->stream));
+    if (c->n_pad <= rtz::kMaxConstSpheres && c->geo_const) {
+        static thread_local rtz::GuideParamsConst C;  // 8.5 KiB: keep it off the stack
+        if (c->cull) {
+            P.geom = c->rg_geom.p, P.aux = c->rg_aux.p, P.albedo = c->rg_albedo.p, P.wexp = c->rg_wexp.p;
+            P.orig = c->rg_orig.p, P.pairs = nullptr;
+            std::memcpy(C.pairs, c->h_rg_pairs.data(), (size_t)c->n_pad * sizeof(float4));
+            std::memcpy(C.boxes, c->h_boxes.data(), c->h_boxes.size() * sizeof(float4));
+            C.cull_r2 = c->cull_r2;
+            C.split_max = rtz::kSplitMax;
+        } else {
+            std::memcpy(C.pairs, c->h_pairs.data(), (size_t)c->n_pad * sizeof(float4));
+        }
+        C.p = P;
+        if (c->cull)
+            rtz::guide_kernel_const<true><<<blocks, 32, 0, c->stream>>>(C);
+        else
+            rtz::guide_kernel_const<false><<<blocks, 32, 0, c->stream>>>(C);
+    } else {
+        rtz::guide_kernel_global<<<blocks, 32, 0, c->stream>>>(P);
+    }
+    RTZ_CUDA(cudaGetLastError());
+    RTZ_CUDA(cudaEventRecord(c->ev[7], c->stream));
+    return RTZ_OK;
+}
+
+// Arguments of a denoised frame (rtz_render_denoised, rtz_multi_render_denoised): the checked params `k`, the guide
+// samples `g` (0 = min(spp, 16)) and the frame's camera `fc` with its ONE seed drawn here when it has none
+int32_t denoised_args(const rtz_camera* cam, uint64_t guide_samples, const rtz_denoise_params* prm, DenoiseConsts& k,
+                      uint64_t& g, rtz_camera& fc) {
+    int32_t rc = check_camera(cam);
+    if (rc != RTZ_OK) return rc;
+    if (cam->mode != RTZ_MODE_PATH && cam->mode != RTZ_MODE_PATH_BVH) return RTZ_ERR_BAD_ARG;
+    if (guide_samples > cam->samples_per_pixel) return RTZ_ERR_BAD_ARG;
+    if (cam->width * cam->height > 0x7FFFFFFFull) return RTZ_ERR_BAD_ARG;
+    rc = denoise_consts(prm, k);
+    if (rc != RTZ_OK) return rc;
+    g = guide_samples ? guide_samples : std::min<uint64_t>(cam->samples_per_pixel, 16);
+    fc = *cam;
+    if (!fc.has_seed) fc.seed = os_seed(), fc.has_seed = 1;
     return RTZ_OK;
 }
 
@@ -1064,64 +1143,37 @@ int32_t rtz_render_resident_linear(rtz_context* c, const rtz_camera* cam, const 
     return render_resident_impl(c, cam, shard, d_rgb, nullptr, st, d_linear);
 }
 
-int32_t rtz_render_guides(rtz_context* c, const rtz_camera* cam, uint64_t guide_samples, float* d_albedo,
-                          float* d_normal, rtz_stats* st) {
+int32_t rtz_render_guides_sharded(rtz_context* c, const rtz_camera* cam, const rtz_shard* shard, uint64_t guide_samples,
+                                  float* d_albedo, float* d_normal, rtz_stats* st) {
     if (!c) return RTZ_ERR_BAD_ARG;
     int32_t rc = check_camera(cam);
     if (rc != RTZ_OK) return rc;
-    if (cam->mode != RTZ_MODE_PATH && cam->mode != RTZ_MODE_PATH_BVH) return RTZ_ERR_BAD_ARG;
-    // the guides belong to a frame: its rays are keyed by the frame's seed, which an OS-drawn seed would not repeat
-    if (!cam->has_seed || guide_samples == 0 || guide_samples > cam->samples_per_pixel) return RTZ_ERR_BAD_ARG;
+    rc = check_guides(cam, guide_samples);
+    if (rc != RTZ_OK) return rc;
     if (!d_albedo && !d_normal) return RTZ_ERR_BAD_ARG;
+    rtz::ShardGeom sg;
+    rc = shard_geom(cam->width, cam->height, shard, sg);
+    if (rc != RTZ_OK) return rc;
     DeviceGuard guard;
     RTZ_CUDA(cudaSetDevice(c->device));
-    const uint64_t n_pix = cam->width * cam->height;
-    rtz::GuideParams P{};
-    P.cam = to_dev_camera(*cam, cam->seed);
-    P.pairs = c->pairs.p, P.geom = c->geom.p, P.aux = c->aux.p, P.albedo = c->albedo.p, P.wexp = c->wexp.p;
-    P.orig = nullptr;
-    P.n_pad = c->n_pad;
-    P.g = (uint32_t)guide_samples;
-    P.pix_per_item = guide_samples >= 64 ? 1u : (uint32_t)(64 / guide_samples);
-    P.n_items = (uint32_t)((n_pix + P.pix_per_item - 1) / P.pix_per_item);
-    if (P.n_items > 0x7FFFFFFFu) return RTZ_ERR_BAD_ARG;  // one block (warp) per item: the grid's x limit
-    P.albedo_out = d_albedo, P.normal_out = d_normal;
-    const unsigned blocks = P.n_items;
-    // every mode sweeps by brute force here (the BVH finds the same hits), on the rows the render's sweep reads
-    RTZ_CUDA(cudaEventRecord(c->ev[0], c->stream));
-    if (c->n_pad <= rtz::kMaxConstSpheres && c->geo_const) {
-        static thread_local rtz::GuideParamsConst C;  // 8.5 KiB: keep it off the stack
-        if (c->cull) {
-            P.geom = c->rg_geom.p, P.aux = c->rg_aux.p, P.albedo = c->rg_albedo.p, P.wexp = c->rg_wexp.p;
-            P.orig = c->rg_orig.p, P.pairs = nullptr;
-            std::memcpy(C.pairs, c->h_rg_pairs.data(), (size_t)c->n_pad * sizeof(float4));
-            std::memcpy(C.boxes, c->h_boxes.data(), c->h_boxes.size() * sizeof(float4));
-            C.cull_r2 = c->cull_r2;
-            C.split_max = rtz::kSplitMax;
-        } else {
-            std::memcpy(C.pairs, c->h_pairs.data(), (size_t)c->n_pad * sizeof(float4));
-        }
-        C.p = P;
-        if (c->cull)
-            rtz::guide_kernel_const<true><<<blocks, 32, 0, c->stream>>>(C);
-        else
-            rtz::guide_kernel_const<false><<<blocks, 32, 0, c->stream>>>(C);
-    } else {
-        rtz::guide_kernel_global<<<blocks, 32, 0, c->stream>>>(P);
-    }
-    RTZ_CUDA(cudaGetLastError());
-    RTZ_CUDA(cudaEventRecord(c->ev[1], c->stream));
+    rc = enqueue_guides(c, cam, sg, guide_samples, d_albedo, d_normal, false);
+    if (rc != RTZ_OK) return rc;
     RTZ_CUDA(cudaStreamSynchronize(c->stream));
     if (st) {
         std::memset(st, 0, sizeof(*st));
-        st->samples = st->segments = n_pix * guide_samples;
+        st->samples = st->segments = shard_real_pixels(cam, sg) * guide_samples;
         st->sphere_tests = st->segments * (uint64_t)c->n_spheres;
         st->kernel_launches = 1;
         float ms = 0;
-        cudaEventElapsedTime(&ms, c->ev[0], c->ev[1]), st->trace_ms = st->total_ms = ms;
+        cudaEventElapsedTime(&ms, c->ev[6], c->ev[7]), st->trace_ms = st->total_ms = ms;
         st->seed_used = cam->seed;
     }
     return RTZ_OK;
+}
+
+int32_t rtz_render_guides(rtz_context* c, const rtz_camera* cam, uint64_t guide_samples, float* d_albedo,
+                          float* d_normal, rtz_stats* st) {
+    return rtz_render_guides_sharded(c, cam, nullptr, guide_samples, d_albedo, d_normal, st);
 }
 
 int32_t rtz_denoise(rtz_context* c, uint64_t W, uint64_t H, const float* d_color, const float* d_albedo,
@@ -1153,9 +1205,12 @@ int32_t rtz_denoise(rtz_context* c, uint64_t W, uint64_t H, const float* d_color
     return RTZ_OK;
 }
 
-int32_t rtz_deinterleave(rtz_context* c, uint64_t W, uint64_t H, uint32_t world, uint32_t tw, uint32_t th,
-                         const uint8_t* d_gathered, uint8_t* d_rgb) {
-    if (!c || !d_gathered || !d_rgb || !W || !H) return RTZ_ERR_BAD_ARG;
+}  // extern "C"
+
+template <class T>
+static int32_t deinterleave_impl(rtz_context* c, uint64_t W, uint64_t H, uint32_t world, uint32_t tw, uint32_t th,
+                                 const T* d_gathered, T* d_out) {
+    if (!c || !d_gathered || !d_out || !W || !H) return RTZ_ERR_BAD_ARG;
     rtz_shard s{0, world, tw, th};
     rtz::ShardGeom g;
     int32_t rc = shard_geom(W, H, &s, g);
@@ -1164,11 +1219,23 @@ int32_t rtz_deinterleave(rtz_context* c, uint64_t W, uint64_t H, uint32_t world,
     DeviceGuard guard;
     RTZ_CUDA(cudaSetDevice(c->device));
     const uint64_t n = W * H;
-    rtz::deinterleave_kernel<<<(unsigned)((n + 255) / 256), 256, 0, c->stream>>>(
-        d_gathered, (uint64_t)g.n_local_tiles * g.tile_pixels, (uint32_t)W, (uint32_t)H, world, tw, th, g.tiles_x, d_rgb);
+    rtz::deinterleave_kernel<T><<<(unsigned)((n + 255) / 256), 256, 0, c->stream>>>(
+        d_gathered, (uint64_t)g.n_local_tiles * g.tile_pixels, (uint32_t)W, (uint32_t)H, world, tw, th, g.tiles_x, d_out);
     RTZ_CUDA(cudaGetLastError());
     RTZ_CUDA(cudaStreamSynchronize(c->stream));
     return RTZ_OK;
+}
+
+extern "C" {
+
+int32_t rtz_deinterleave(rtz_context* c, uint64_t W, uint64_t H, uint32_t world, uint32_t tw, uint32_t th,
+                         const uint8_t* d_gathered, uint8_t* d_rgb) {
+    return deinterleave_impl(c, W, H, world, tw, th, d_gathered, d_rgb);
+}
+
+int32_t rtz_deinterleave_f32(rtz_context* c, uint64_t W, uint64_t H, uint32_t world, uint32_t tw, uint32_t th,
+                             const float* d_gathered, float* d_out) {
+    return deinterleave_impl(c, W, H, world, tw, th, d_gathered, d_out);
 }
 
 // The host-buffer entry points keep ONE lazily created context per DEVICE (buffers and stream are reused
@@ -1222,31 +1289,13 @@ int32_t rtz_render(const rtz_camera* cam, const rtz_sphere* sp, uint64_t n, uint
     return rtz_render_linear(cam, sp, n, rgb_out, nullptr, st);
 }
 
-int32_t rtz_render_denoised(const rtz_camera* cam, const rtz_sphere* sp, uint64_t n, uint64_t guide_samples,
-                            const rtz_denoise_params* prm, uint8_t* rgb_out, float* linear_out, rtz_stats* st) {
-    if ((!rgb_out && !linear_out) || (!sp && n)) return RTZ_ERR_BAD_ARG;
-    int32_t rc = check_camera(cam);
-    if (rc != RTZ_OK) return rc;
-    if (cam->mode != RTZ_MODE_PATH && cam->mode != RTZ_MODE_PATH_BVH) return RTZ_ERR_BAD_ARG;
-    if (guide_samples > cam->samples_per_pixel) return RTZ_ERR_BAD_ARG;
-    const uint64_t px = cam->width * cam->height;
-    if (px > 0x7FFFFFFFull) return RTZ_ERR_BAD_ARG;
-    DenoiseConsts k;
-    rc = denoise_consts(prm, k);
-    if (rc != RTZ_OK) return rc;
-    const uint64_t g = guide_samples ? guide_samples : std::min<uint64_t>(cam->samples_per_pixel, 16);
-    rtz_camera fc = *cam;  // the guides need the frame's seed: draw it once, here
-    if (!fc.has_seed) fc.seed = os_seed(), fc.has_seed = 1;
-    int cnt = 0;
-    rc = rtz_device_count(&cnt);
-    if (rc != RTZ_OK) return rc;
-    std::lock_guard<std::mutex> lock(g_default_mu);
-    DeviceGuard guard;
-    rtz_context* c = nullptr;
-    rc = default_context(&c);
-    if (rc != RTZ_OK) return rc;
-    rc = rtz_scene_upload(c, sp, n);
-    if (rc != RTZ_OK) return rc;
+}  // extern "C"
+
+// The linear colour, the guides and the denoise of a whole frame on one context with its scene uploaded; host outputs.
+// `fc` has its seed.
+static int32_t denoise_frame(rtz_context* c, const rtz_camera* fc, uint64_t g, const DenoiseConsts& k, uint8_t* rgb_out,
+                             float* linear_out, rtz_stats* st) {
+    const uint64_t px = fc->width * fc->height;
     RTZ_CUDA(cudaSetDevice(c->device));
     RTZ_CUDA(c->rgb.reserve(3 * px));
     RTZ_CUDA(c->denoise_io.reserve(12 * px));
@@ -1256,12 +1305,12 @@ int32_t rtz_render_denoised(const rtz_camera* cam, const rtz_sphere* sp, uint64_
     float* const out = nrm + 3 * px;
     RTZ_CUDA(cudaEventRecord(c->ev[4], c->stream));
     rtz_stats rs, gs;
-    rc = render_resident_impl(c, &fc, nullptr, c->rgb.p, nullptr, &rs, lin);
+    int32_t rc = render_resident_impl(c, fc, nullptr, c->rgb.p, nullptr, &rs, lin);
     if (rc != RTZ_OK) return rc;
-    rc = rtz_render_guides(c, &fc, g, alb, nrm, &gs);
+    rc = rtz_render_guides(c, fc, g, alb, nrm, &gs);
     if (rc != RTZ_OK) return rc;
     uint64_t launches = 0;
-    rc = enqueue_denoise(c, (uint32_t)cam->width, (uint32_t)cam->height, lin, alb, nrm, k, linear_out ? out : nullptr,
+    rc = enqueue_denoise(c, (uint32_t)fc->width, (uint32_t)fc->height, lin, alb, nrm, k, linear_out ? out : nullptr,
                          rgb_out ? c->rgb.p : nullptr, launches);
     if (rc != RTZ_OK) return rc;
     RTZ_CUDA(cudaEventRecord(c->ev[5], c->stream));
@@ -1276,6 +1325,29 @@ int32_t rtz_render_denoised(const rtz_camera* cam, const rtz_sphere* sp, uint64_
         cudaEventElapsedTime(&ms, c->ev[4], c->ev[5]), st->total_ms = ms;
     }
     return RTZ_OK;
+}
+
+extern "C" {
+
+int32_t rtz_render_denoised(const rtz_camera* cam, const rtz_sphere* sp, uint64_t n, uint64_t guide_samples,
+                            const rtz_denoise_params* prm, uint8_t* rgb_out, float* linear_out, rtz_stats* st) {
+    if ((!rgb_out && !linear_out) || (!sp && n)) return RTZ_ERR_BAD_ARG;
+    DenoiseConsts k;
+    uint64_t g = 0;
+    rtz_camera fc;
+    int32_t rc = denoised_args(cam, guide_samples, prm, k, g, fc);
+    if (rc != RTZ_OK) return rc;
+    int cnt = 0;
+    rc = rtz_device_count(&cnt);
+    if (rc != RTZ_OK) return rc;
+    std::lock_guard<std::mutex> lock(g_default_mu);
+    DeviceGuard guard;
+    rtz_context* c = nullptr;
+    rc = default_context(&c);
+    if (rc != RTZ_OK) return rc;
+    rc = rtz_scene_upload(c, sp, n);
+    if (rc != RTZ_OK) return rc;
+    return denoise_frame(c, &fc, g, k, rgb_out, linear_out, st);
 }
 
 int32_t rtz_write_ppm(const char* path, uint64_t w, uint64_t h, const uint8_t* rgb) {
@@ -1407,7 +1479,11 @@ struct rtz_multi {
     std::vector<size_t> local_cap;
     DevBuf<uint8_t> gathered;             // RTZ_GATHER_NCCL, device 0: `world` compact buffers back to back
     DevBuf<uint8_t> image;                // device 0: the row-major frame
+    // rtz_multi_render_denoised, RTZ_GATHER_NCCL, device 0: the linear colour, albedo and normal planes, each `world`
+    // compact f32 buffers back to back (the other devices' compact buffers are their contexts' denoise_io)
+    DevBuf<float> gathered_f32;
     cudaEvent_t ev_start = nullptr, ev_traced = nullptr, ev_end = nullptr;  // device 0's stream
+    cudaEvent_t ev_inputs = nullptr;  // rtz_multi_render_denoised: the denoiser's inputs are complete on device 0
 };
 
 namespace {
@@ -1442,8 +1518,8 @@ int32_t rtz_multi_destroy(rtz_multi* m) {
         if (c && g_nccl.CommDestroy) g_nccl.CommDestroy(c);
     if (!m->dev.empty()) {
         cudaSetDevice(m->dev[0]);
-        m->gathered.release(), m->image.release();
-        for (cudaEvent_t e : {m->ev_start, m->ev_traced, m->ev_end})
+        m->gathered.release(), m->image.release(), m->gathered_f32.release();
+        for (cudaEvent_t e : {m->ev_start, m->ev_traced, m->ev_end, m->ev_inputs})
             if (e) cudaEventDestroy(e);
     }
     for (rtz_context* c : m->ctx)
@@ -1489,6 +1565,7 @@ int32_t rtz_multi_create(int32_t num_gpus, const int32_t* devices, uint32_t tile
     }
     cudaSetDevice(m->dev[0]);
     cudaEventCreate(&m->ev_start), cudaEventCreate(&m->ev_traced), cudaEventCreate(&m->ev_end);
+    cudaEventCreate(&m->ev_inputs);
     if (const char* e = std::getenv("RTZ_GATHER")) {
         if (!std::strcmp(e, "p2p")) gather = RTZ_GATHER_P2P;
         if (!std::strcmp(e, "nccl")) gather = RTZ_GATHER_NCCL;
@@ -1647,28 +1724,176 @@ int32_t rtz_multi_render(rtz_multi* m, const rtz_camera* cam, uint8_t* rgb_out, 
     return RTZ_OK;
 }
 
-// one lazily created rtz_multi per device count for the one-shot form
+int32_t rtz_multi_render_denoised(rtz_multi* m, const rtz_camera* cam, uint64_t guide_samples,
+                                  const rtz_denoise_params* prm, uint8_t* rgb_out, float* linear_out, rtz_stats* st) {
+    if (!m || (!rgb_out && !linear_out)) return RTZ_ERR_BAD_ARG;
+    DenoiseConsts k;
+    uint64_t g = 0;
+    rtz_camera fc;
+    int32_t rc = denoised_args(cam, guide_samples, prm, k, g, fc);
+    if (rc != RTZ_OK) return rc;
+    DeviceGuard guard;
+    const int world = (int)m->ctx.size();
+    rtz_context* c0 = m->ctx[0];
+    if (world == 1) return denoise_frame(c0, &fc, g, k, rgb_out, linear_out, st);
+    const uint32_t W = (uint32_t)fc.width, H = (uint32_t)fc.height;
+    const uint64_t px = (uint64_t)W * H, seed = fc.seed;
+    std::vector<rtz::ShardGeom> sg(world);
+    for (int r = 0; r < world; ++r) {
+        const rtz_shard sh{(uint32_t)r, (uint32_t)world, m->tile_w, m->tile_h};
+        rc = shard_geom(W, H, &sh, sg[r]);
+        if (rc != RTZ_OK) return rc;
+    }
+    const uint64_t per_px = (uint64_t)sg[0].n_local_tiles * sg[0].tile_pixels;  // equal on every rank
+    const uint64_t per_rank = 3 * per_px;                                        // f32 of one quantity of one rank
+    const bool nccl = m->gather == RTZ_GATHER_NCCL;
+    // device 0: the row-major linear colour, albedo, normal and denoised colour (3 f32 per pixel each) and the bytes;
+    // for NCCL the compact buffers of every device too (each device's resolve also needs its compact bytes)
+    RTZ_CUDA(cudaSetDevice(m->dev[0]));
+    RTZ_CUDA(c0->denoise_io.reserve(12 * px));
+    RTZ_CUDA(c0->rgb.reserve(std::max(3 * px, per_rank)));
+    float* const lin = c0->denoise_io.p;
+    float* const alb = lin + 3 * px;
+    float* const nrm = alb + 3 * px;
+    float* const out = nrm + 3 * px;
+    if (nccl) {
+        RTZ_CUDA(m->gathered_f32.reserve(3 * per_rank * world));
+        for (int r = 1; r < world; ++r) {
+            RTZ_CUDA(cudaSetDevice(m->dev[r]));
+            RTZ_CUDA(m->ctx[r]->denoise_io.reserve(3 * per_rank));
+            RTZ_CUDA(m->ctx[r]->rgb.reserve(per_rank));
+        }
+        RTZ_CUDA(cudaSetDevice(m->dev[0]));
+    }
+    float* const G = m->gathered_f32.p;
+    RTZ_CUDA(cudaEventRecord(m->ev_start, c0->stream));
+    // every device's tiles and guides are enqueued (by its own host thread) before the first wait
+    rc = on_every_device(m, [&](int r) -> int32_t {
+        RTZ_CUDA(cudaSetDevice(m->dev[r]));
+        rtz_context* c = m->ctx[r];
+        FrameTarget t;
+        float *a = alb, *n = nrm;  // P2P: device 0's row-major planes (peer memory for r >= 1)
+        if (nccl) {
+            // the compact linear colour, albedo and normal of rank r: rank 0 writes into the gathered planes, the
+            // others into their own buffer, sent below
+            float* const base = r == 0 ? G : c->denoise_io.p;
+            const uint64_t plane = r == 0 ? per_rank * world : per_rank;
+            t.d_rgb = c->rgb.p, t.d_linear32 = base, a = base + plane, n = base + 2 * plane;
+        } else {
+            t.image_linear32 = lin;
+        }
+        int32_t e = enqueue_path(c, &fc, sg[r], t, seed);
+        if (e != RTZ_OK) return e;
+        e = enqueue_guides(c, &fc, sg[r], g, a, n, !nccl);
+        if (e != RTZ_OK) return e;
+        RTZ_CUDA(cudaEventRecord(m->done[r], c->stream));
+        return RTZ_OK;
+    });
+    if (rc != RTZ_OK) return rc;
+    RTZ_CUDA(cudaSetDevice(m->dev[0]));
+    if (nccl) {
+        RTZ_NCCL(g_nccl.GroupStart());
+        for (int r = 1; r < world; ++r)
+            for (uint64_t q = 0; q < 3; ++q) {
+                RTZ_NCCL(g_nccl.Send(m->ctx[r]->denoise_io.p + q * per_rank, per_rank, ncclFloat32, 0, m->comms[r],
+                                     m->ctx[r]->stream));
+                RTZ_NCCL(g_nccl.Recv(G + q * per_rank * world + r * per_rank, per_rank, ncclFloat32, r, m->comms[0],
+                                     c0->stream));
+            }
+        RTZ_NCCL(g_nccl.GroupEnd());
+        RTZ_CUDA(cudaSetDevice(m->dev[0]));
+        for (uint64_t q = 0; q < 3; ++q) {
+            rtz::deinterleave_kernel<float><<<(unsigned)((px + 255) / 256), 256, 0, c0->stream>>>(
+                G + q * per_rank * world, per_px, W, H, (uint32_t)world, m->tile_w, m->tile_h, sg[0].tiles_x,
+                lin + q * 3 * px);
+            RTZ_CUDA(cudaGetLastError());
+        }
+    } else {
+        for (int r = 1; r < world; ++r) RTZ_CUDA(cudaStreamWaitEvent(c0->stream, m->done[r], 0));
+    }
+    RTZ_CUDA(cudaEventRecord(m->ev_inputs, c0->stream));
+    uint64_t launches = 0;
+    rc = enqueue_denoise(c0, W, H, lin, alb, nrm, k, linear_out ? out : nullptr, rgb_out ? c0->rgb.p : nullptr,
+                         launches);
+    if (rc != RTZ_OK) return rc;
+    RTZ_CUDA(cudaEventRecord(m->ev_end, c0->stream));
+    if (rgb_out) RTZ_CUDA(cudaMemcpyAsync(rgb_out, c0->rgb.p, 3 * px, cudaMemcpyDeviceToHost, c0->stream));
+    if (linear_out)
+        RTZ_CUDA(cudaMemcpyAsync(linear_out, out, 3 * px * sizeof(float), cudaMemcpyDeviceToHost, c0->stream));
+    rtz_stats total;
+    std::memset(&total, 0, sizeof total);
+    for (int r = 0; r < world; ++r) {
+        RTZ_CUDA(cudaSetDevice(m->dev[r]));
+        rtz_stats one;
+        rc = collect_path(m->ctx[r], &fc, sg[r], &one, seed);
+        if (rc != RTZ_OK) return rc;
+        total.samples += one.samples, total.segments += one.segments, total.sphere_tests += one.sphere_tests;
+        total.depth_capped += one.depth_capped, total.absorbed += one.absorbed, total.nan_samples += one.nan_samples;
+        total.kernel_launches += one.kernel_launches + 1;  // + the guide kernel
+        total.trace_ms = std::max(total.trace_ms, one.trace_ms);
+        total.resolve_ms = std::max(total.resolve_ms, one.resolve_ms);
+    }
+    RTZ_CUDA(cudaSetDevice(m->dev[0]));
+    RTZ_CUDA(cudaStreamSynchronize(c0->stream));
+    if (st) {
+        float ms = 0;
+        cudaEventElapsedTime(&ms, m->ev_start, m->ev_end), total.total_ms = ms;
+        cudaEventElapsedTime(&ms, m->ev_start, m->ev_inputs);
+        total.gather_ms = std::max(0.0, (double)ms - total.trace_ms);
+        total.kernel_launches += launches + (nccl ? 3 : 0);
+        total.gpus = (uint32_t)world;
+        total.gather = (uint32_t)m->gather;
+        total.seed_used = seed;
+        *st = total;
+    }
+    return RTZ_OK;
+}
+
+// one lazily created rtz_multi per device count for the one-shot forms
 static std::mutex g_multi_mu;
 static std::map<int, rtz_multi*> g_multi;
+
+// the cached rtz_multi of `num_gpus` devices (<= 0: all) with the scene uploaded; call with g_multi_mu held
+static int32_t default_multi(const rtz_sphere* sp, uint64_t n, int32_t num_gpus, rtz_multi** out) {
+    int visible = 0;
+    int32_t rc = rtz_device_count(&visible);
+    if (rc != RTZ_OK) return rc;
+    if (num_gpus <= 0) num_gpus = visible;
+    rtz_multi*& slot = g_multi[num_gpus];
+    if (!slot) {
+        rc = rtz_multi_create(num_gpus, nullptr, 0, 0, RTZ_GATHER_AUTO, &slot);
+        if (rc != RTZ_OK) return rc;
+    }
+    *out = slot;
+    return rtz_multi_scene_upload(slot, sp, n);
+}
 
 int32_t rtz_render_multi(const rtz_camera* cam, const rtz_sphere* sp, uint64_t n, int32_t num_gpus, uint8_t* rgb_out,
                          rtz_stats* st) {
     if (!rgb_out || (!sp && n)) return RTZ_ERR_BAD_ARG;
     int32_t rc = check_camera(cam);
     if (rc != RTZ_OK) return rc;
-    int visible = 0;
-    rc = rtz_device_count(&visible);
-    if (rc != RTZ_OK) return rc;
-    if (num_gpus <= 0) num_gpus = visible;
     std::lock_guard<std::mutex> lock(g_multi_mu);
-    rtz_multi*& slot = g_multi[num_gpus];
-    if (!slot) {
-        rc = rtz_multi_create(num_gpus, nullptr, 0, 0, RTZ_GATHER_AUTO, &slot);
-        if (rc != RTZ_OK) return rc;
-    }
-    rc = rtz_multi_scene_upload(slot, sp, n);
+    rtz_multi* m = nullptr;
+    rc = default_multi(sp, n, num_gpus, &m);
     if (rc != RTZ_OK) return rc;
-    return rtz_multi_render(slot, cam, rgb_out, nullptr, st);
+    return rtz_multi_render(m, cam, rgb_out, nullptr, st);
+}
+
+int32_t rtz_render_multi_denoised(const rtz_camera* cam, const rtz_sphere* sp, uint64_t n, int32_t num_gpus,
+                                  uint64_t guide_samples, const rtz_denoise_params* prm, uint8_t* rgb_out,
+                                  float* linear_out, rtz_stats* st) {
+    if ((!rgb_out && !linear_out) || (!sp && n)) return RTZ_ERR_BAD_ARG;
+    DenoiseConsts k;
+    uint64_t g = 0;
+    rtz_camera fc;
+    int32_t rc = denoised_args(cam, guide_samples, prm, k, g, fc);  // refused before any device is touched
+    if (rc != RTZ_OK) return rc;
+    std::lock_guard<std::mutex> lock(g_multi_mu);
+    rtz_multi* m = nullptr;
+    rc = default_multi(sp, n, num_gpus, &m);
+    if (rc != RTZ_OK) return rc;
+    return rtz_multi_render_denoised(m, &fc, guide_samples, prm, rgb_out, linear_out, st);
 }
 
 }  // extern "C"

@@ -19,6 +19,13 @@
 // floor(64 / g) of them for g < 64 (so g = 1 still fills all 64 slots), one for g >= 64, swept in rounds of 64 of its
 // samples.  A pixel never spans two warps, so its sums keep their order: after each sweep the six values of every ray
 // are staged in shared memory and each (pixel, channel) is folded by one lane.
+//
+// Shards: the items run over the local pixels of a rank's tiles (ShardGeom, the compact layout of the render), each
+// mapped to its global pixel (x, y) by local_to_global_rcp once per item (guide_slot: mapped per ray and per stored
+// channel, with divisions, the whole-frame kernel ran 4-15 % longer on a B200) and keyed by y*W + x, so a pixel's guides do not depend on the
+// shard that computes them.  The whole frame is the shard {0, 1, W, 1}, whose compact layout is the row-major image.
+// A tile-padding pixel still sweeps rays (those of pixel (min(x, W-1), min(y, H-1))) so that every lane takes part in
+// the sweep's votes; its sums are never stored into a real pixel.
 #pragma once
 #include "rtz_kernels.cuh"
 
@@ -36,8 +43,13 @@ struct GuideParams {
     uint32_t g;              // guide samples per pixel
     uint32_t pix_per_item;   // whole pixels per warp: floor(64 / g), 1 for g >= 64
     uint32_t n_items;
-    float* albedo_out;       // [W*H*3] or null
-    float* normal_out;       // [W*H*3] or null
+    ShardGeom sh;            // the pixels the items run over
+    unsigned long long rcp_tile_pixels, rcp_tiles_x, rcp_tile_w;  // its divisors as reciprocals (local_to_global_rcp)
+    uint32_t n_local;        // sh.n_local_tiles * sh.tile_pixels
+    uint32_t row_major;      // 0: outputs in the compact layout, padding written as 0; 1: at y*W + x of row-major
+                             // planes (possibly device 0's memory through peer access), padding not written
+    float* albedo_out;       // 3 f32 per pixel, or null
+    float* normal_out;       // 3 f32 per pixel, or null
 };
 
 // the constant-bank form: the rows the render's constant-bank kernels sweep (plain, or regrouped with their boxes)
@@ -51,15 +63,34 @@ struct GuideParamsConst {
 
 constexpr int kGuideStageFloats = 6 * 64;  // per warp: the six values of 64 rays
 
-// camera ray `r` of a work item (pixel pix0 + r / g, sample r % g); a slot past the item's last ray takes ray 0 of
-// the item and its result is not folded
-__device__ __forceinline__ void guide_ray(const DevCamera& cam, uint32_t g, uint32_t pix0, uint32_t r, uint32_t rays,
-                                          Path& p) {
+// Ray slot j of a work item (lane j % 32, first or second path): its local pixel pix0 + j / g (a slot past the item's
+// last ray takes ray 0 of the item and its result is not folded; for g >= 64 every slot is the item's one pixel), that
+// pixel's (x, y) (tile padding: clamped into the frame, a valid ray whose sums are never stored into a real pixel) and
+// the first sample index of the slot's pixel among the item's rays.  Mapped once per item, not per round.
+struct GuideSlot {
+    uint32_t x, y, base;
+};
+
+// where slot j's pixel is stored (low 32 bits: pixel index in the output, compact or row-major) | kGuidePadding
+constexpr unsigned long long kGuidePadding = 1ull << 32;
+
+__device__ __forceinline__ GuideSlot guide_slot(const GuideParams& P, uint32_t pix0, uint32_t j, uint32_t rays,
+                                                unsigned long long& dest) {
+    const DevCamera& cam = P.cam;
+    const uint32_t pl = (j < rays ? j : 0) / P.g;
+    GuideSlot s;
+    const bool inside = local_to_global_rcp(P.sh, P.rcp_tile_pixels, P.rcp_tiles_x, P.rcp_tile_w, cam.width, cam.height,
+                                            pix0 + pl, s.x, s.y);
+    dest = (inside ? 0ull : kGuidePadding) | (P.row_major ? (inside ? s.y * cam.width + s.x : 0u) : pix0 + pl);
+    s.x = min(s.x, cam.width - 1), s.y = min(s.y, cam.height - 1);
+    s.base = pl * P.g;
+    return s;
+}
+
+// the slot's camera ray in the round that starts at ray r0 of the item (pixel y*W + x, sample r - base)
+__device__ __forceinline__ void guide_ray(const DevCamera& cam, const GuideSlot& s, uint32_t r, uint32_t rays, Path& p) {
     if (r >= rays) r = 0;
-    const uint32_t pl = r / g, s = r - pl * g;
-    const uint32_t pixel = pix0 + pl;
-    const uint32_t y = pixel / cam.width, x = pixel - y * cam.width;
-    camera_ray(cam, RngKey{cam.key0, cam.key1, pixel, s}, x, y, p);
+    camera_ray(cam, RngKey{cam.key0, cam.key1, s.y * cam.width + s.x, r - s.base}, s.x, s.y, p);
 }
 
 // the six values of one swept ray into its column `j` of the staging rows (row c = channel c: albedo rgb, normal xyz)
@@ -87,9 +118,11 @@ __device__ __forceinline__ void guide_values(const GuideParams& P, const Path& p
     for (int c = 0; c < 6; ++c) stage[c * 64 + j] = v[c];
 }
 
-__device__ __forceinline__ void guide_store(const GuideParams& P, uint32_t pixel, uint32_t c, float value) {
+// channel c of the pixel at `dest` (guide_slot): compact padding is stored as +0, row-major padding not at all
+__device__ __forceinline__ void guide_store(const GuideParams& P, unsigned long long dest, uint32_t c, float value) {
     float* out = c < 3 ? P.albedo_out : P.normal_out;
-    if (out) out[3ull * pixel + (c < 3 ? c : c - 3)] = value;
+    if (!out || (dest >= kGuidePadding && P.row_major)) return;
+    out[3ull * (uint32_t)dest + (c < 3 ? c : c - 3)] = dest >= kGuidePadding ? 0.0f : value;
 }
 
 template <bool kConstBank, bool kCull>
@@ -104,13 +137,16 @@ __device__ __forceinline__ void guide_body(const GuideParams& P, const float4* _
     const DevCamera& cam = P.cam;
     const uint32_t g = P.g;
     const uint32_t pix0 = item * P.pix_per_item;
-    const uint32_t n_here = min(P.pix_per_item, cam.width * cam.height - pix0);  // the last item may hold fewer
+    const uint32_t n_here = min(P.pix_per_item, P.n_local - pix0);  // the last item may hold fewer
     const uint32_t rays = n_here * g;
+    __shared__ unsigned long long dest[64];  // per slot: where its pixel is stored (the fold reads slot pl * g's)
+    const GuideSlot sa = guide_slot(P, pix0, lane, rays, dest[lane]);
+    const GuideSlot sb = guide_slot(P, pix0, 32 + lane, rays, dest[32 + lane]);
     float acc = 0.0f;  // g >= 64: lane c < 6 holds the running sum of channel c of the item's one pixel
     for (uint32_t r0 = 0; r0 < rays; r0 += 64) {
         Path a, b;
-        guide_ray(cam, g, pix0, r0 + lane, rays, a);
-        guide_ray(cam, g, pix0, r0 + 32 + lane, rays, b);
+        guide_ray(cam, sa, r0 + lane, rays, a);
+        guide_ray(cam, sb, r0 + 32 + lane, rays, b);
         __syncwarp();  // converged before the sweep's votes
         float ta = 0.f, tb = 0.f;
         int ia = -1, ib = -1;
@@ -126,7 +162,7 @@ __device__ __forceinline__ void guide_body(const GuideParams& P, const float4* _
                 const float* row = stage + c * 64 + pl * g;
                 float sum = 0.0f;
                 for (uint32_t s = 0; s < g; ++s) sum += row[s];
-                guide_store(P, pix0 + pl, c, sum / (float)g);
+                guide_store(P, dest[pl * g], c, sum / (float)g);
             }
         } else if (lane < 6) {
             const uint32_t m = min(64u, rays - r0);
@@ -134,7 +170,7 @@ __device__ __forceinline__ void guide_body(const GuideParams& P, const float4* _
         }
         __syncwarp();  // the next round rewrites the rows
     }
-    if (g >= 64 && lane < 6) guide_store(P, pix0, lane, acc / (float)g);
+    if (g >= 64 && lane < 6) guide_store(P, dest[0], lane, acc / (float)g);
 }
 
 // Scenes the render sweeps from the constant bank (n_pad <= kMaxConstSpheres): the same rows, through the same

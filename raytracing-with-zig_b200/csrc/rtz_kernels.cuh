@@ -1622,14 +1622,19 @@ __global__ void resolve_kernel(const unsigned long long* __restrict__ accum, uin
 // K3 fused with the multi-GPU tile exchange (rtz_multi_*, RTZ_GATHER_P2P): the same resolve, but every channel
 // is stored at its place in the ROW-MAJOR image, which lives on device 0 — peer memory over NVLink for the
 // other devices.  A device's resolve IS its half of the gather: no staging buffer, no de-interleave pass.
+// `image` (bytes) and `linear32` (the linear colour rounded once to f32, the denoiser's input) are each optional.
 __global__ void resolve_scatter_kernel(const unsigned long long* __restrict__ accum, const ShardGeom sh, uint32_t W,
-                                       uint32_t H, double scale, uint8_t* __restrict__ image) {
+                                       uint32_t H, double scale, uint8_t* __restrict__ image,
+                                       float* __restrict__ linear32) {
     const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;  // one thread per channel
     if (i >= 3ull * sh.n_local_tiles * sh.tile_pixels) return;
     const uint32_t lp = (uint32_t)(i / 3), ch = (uint32_t)(i - 3ull * lp);
     uint32_t x, y;
     if (!local_to_global(sh, W, H, lp, x, y)) return;  // tile padding
-    image[3ull * ((uint64_t)y * W + x) + ch] = to_byte(((double)accum[i] * 0x1p-32) * scale);
+    const double lin = ((double)accum[i] * 0x1p-32) * scale;
+    const uint64_t at = 3ull * ((uint64_t)y * W + x) + ch;
+    if (image) image[at] = to_byte(lin);
+    if (linear32) linear32[at] = (float)lin;
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -1706,11 +1711,12 @@ __global__ void legacy_kernel(const __grid_constant__ LegacyParams P, uint8_t* _
 }
 
 // ---------------------------------------------------------------------------------------------
-// K4: de-interleave `world` equal-sized compact tile buffers into the row-major image.
+// K4: de-interleave `world` equal-sized compact tile buffers into the row-major image; a pixel is 3 T (the bytes,
+// or the f32 linear colour and guides of a denoised frame).
 // ---------------------------------------------------------------------------------------------
-__global__ void deinterleave_kernel(const uint8_t* __restrict__ gathered, uint64_t per_rank_pixels, uint32_t W,
-                                    uint32_t H, uint32_t world, uint32_t tw, uint32_t th, uint32_t tiles_x,
-                                    uint8_t* __restrict__ out) {
+template <class T>
+__global__ void deinterleave_kernel(const T* __restrict__ gathered, uint64_t per_rank_pixels, uint32_t W, uint32_t H,
+                                    uint32_t world, uint32_t tw, uint32_t th, uint32_t tiles_x, T* __restrict__ out) {
     const uint64_t idx = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (idx >= (uint64_t)W * H) return;
     const uint32_t y = (uint32_t)(idx / W), x = (uint32_t)(idx - (uint64_t)y * W);
@@ -1718,7 +1724,7 @@ __global__ void deinterleave_kernel(const uint8_t* __restrict__ gathered, uint64
     const uint32_t gt = ty * tiles_x + tx;
     const uint32_t rank = gt % world, lt = gt / world;
     const uint64_t lp = (uint64_t)lt * (tw * th) + (y - ty * th) * tw + (x - tx * tw);
-    const uint8_t* src = gathered + 3ull * ((uint64_t)rank * per_rank_pixels + lp);
+    const T* src = gathered + 3ull * ((uint64_t)rank * per_rank_pixels + lp);
     out[3 * idx + 0] = src[0], out[3 * idx + 1] = src[1], out[3 * idx + 2] = src[2];
 }
 

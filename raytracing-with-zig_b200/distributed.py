@@ -63,3 +63,30 @@ def render_sharded(renderer, camera, tile=DEFAULT_TILE, group=None):
         return None, st
     img = renderer.deinterleave(gathered, int(camera.width), int(camera.height), world, tile[0], tile[1])
     return img, st
+
+
+def render_sharded_denoised(renderer, camera, guide_samples: int = 0, params=None, tile=DEFAULT_TILE, group=None):
+    """`rtz_render_denoised` across the ranks of the default process group: every rank renders the linear colour
+    and the guides of its tiles, rank 0 gathers the three float32 buffers, de-interleaves them and denoises the whole
+    frame.  The camera must carry its seed (every rank has to trace the same rays).  Returns (uint8 [H,W,3],
+    float32 [H,W,3] denoised device tensors on rank 0 / (None, None) elsewhere, this rank's render stats)."""
+    import torch.distributed as dist
+
+    if not camera.has_seed:
+        raise ValueError("render_sharded_denoised needs a camera with its seed: every rank must trace the same rays")
+    rank, world = (dist.get_rank(group), dist.get_world_size(group)) if dist.is_initialized() else (0, 1)
+    spp = int(camera.samples_per_pixel)
+    g = int(guide_samples) if guide_samples else min(spp, 16)
+    shard = B.rtz_shard(rank, world, tile[0], tile[1])
+    _, linear, st = renderer.render_linear(camera, shard)
+    albedo, normal, _ = renderer.render_guides(camera, g, shard=shard)
+    W, H = int(camera.width), int(camera.height)
+    planes = []
+    for local in (linear, albedo, normal):
+        gathered = gather_tiles(local, world, rank, group)
+        if rank == 0:
+            planes.append(renderer.deinterleave(gathered, W, H, world, tile[0], tile[1]))
+    if rank != 0:
+        return None, None, st
+    rgb, lin, _ = renderer.denoise(*planes, params=params)
+    return rgb, lin, st

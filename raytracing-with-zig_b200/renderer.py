@@ -132,12 +132,16 @@ class Renderer:
                                                     C.byref(st)))
         return out, linear, st
 
-    def render_guides(self, camera, samples: int, albedo=None, normal=None):
+    def render_guides(self, camera, samples: int, albedo=None, normal=None, shard: B.rtz_shard | None = None):
         """First-hit denoiser guides of the frame's camera rays, samples 0 .. samples-1 of every pixel (the camera
-        needs its seed): float32 [H, W, 3] device tensors (albedo, normal); returns (albedo, normal, stats)."""
+        needs its seed): float32 [H, W, 3] device tensors (albedo, normal), or [shard_pixels, 3] in the compact tile
+        layout for a shard; returns (albedo, normal, stats)."""
         torch = self.torch
         cam = _cast_camera(camera)
-        shape = (int(cam.height), int(cam.width), 3)
+        if shard is None:
+            shape = (int(cam.height), int(cam.width), 3)
+        else:
+            shape = (self.shard_pixels(cam.width, cam.height, shard), 3)
         dev = f"cuda:{self.device}"
         if albedo is None:
             albedo = torch.empty(shape, dtype=torch.float32, device=dev)
@@ -147,8 +151,12 @@ class Renderer:
             assert t.is_cuda and t.is_contiguous() and t.dtype == torch.float32 and tuple(t.shape) == shape, (t.shape, t.dtype)
         st = B.rtz_stats()
         self._order_after_torch()
-        B.check(self.lib.rtz_render_guides(self._ctx, C.byref(cam), int(samples), C.c_void_p(albedo.data_ptr()),
-                                           C.c_void_p(normal.data_ptr()), C.byref(st)))
+        a, n = C.c_void_p(albedo.data_ptr()), C.c_void_p(normal.data_ptr())
+        if shard is None:
+            B.check(self.lib.rtz_render_guides(self._ctx, C.byref(cam), int(samples), a, n, C.byref(st)))
+        else:
+            B.check(self.lib.rtz_render_guides_sharded(self._ctx, C.byref(cam), C.byref(shard), int(samples), a, n,
+                                                       C.byref(st)))
         return albedo, normal, st
 
     def denoise(self, linear, albedo, normal, params: B.rtz_denoise_params | None = None, out_linear=None,
@@ -175,12 +183,17 @@ class Renderer:
         return out_rgb, out_linear, st
 
     def deinterleave(self, gathered, width: int, height: int, world: int, tile_w: int, tile_h: int, out=None):
+        """`world` compact tile buffers back to back -> the row-major [H, W, 3] frame: uint8 (the bytes) or float32
+        (linear colour, guides)."""
         torch = self.torch
+        fn = {torch.uint8: self.lib.rtz_deinterleave, torch.float32: self.lib.rtz_deinterleave_f32}[gathered.dtype]
+        assert gathered.is_cuda and gathered.is_contiguous()
         if out is None:
-            out = torch.empty((height, width, 3), dtype=torch.uint8, device=gathered.device)
+            out = torch.empty((height, width, 3), dtype=gathered.dtype, device=gathered.device)
+        assert out.dtype == gathered.dtype and out.is_contiguous() and out.numel() == height * width * 3
         self._order_after_torch()   # `gathered` may still be in flight on torch's / NCCL's streams
-        B.check(self.lib.rtz_deinterleave(self._ctx, width, height, world, tile_w, tile_h,
-                                          C.c_void_p(gathered.data_ptr()), C.c_void_p(out.data_ptr())))
+        B.check(fn(self._ctx, width, height, world, tile_w, tile_h, C.c_void_p(gathered.data_ptr()),
+                   C.c_void_p(out.data_ptr())))
         return out
 
 
@@ -227,6 +240,22 @@ class MultiRenderer:
         B.check(self.lib.rtz_multi_render(self._m, C.byref(cam), ptr, None, C.byref(st)))
         return rgb, st
 
+    def render_denoised(self, camera, guide_samples: int = 0, params: B.rtz_denoise_params | None = None):
+        """`rtz_multi_render_denoised`: the frame on every device, denoised on device 0 — the bytes and linear
+        colour of `render_host_denoised`.  Returns (numpy uint8 [H,W,3], numpy float32 [H,W,3], stats)."""
+        import numpy as np
+
+        cam = _cast_camera(camera)
+        H, W = int(cam.height), int(cam.width)
+        rgb = np.empty((H, W, 3), dtype=np.uint8)
+        lin = np.empty((H, W, 3), dtype=np.float32)
+        st = B.rtz_stats()
+        B.check(self.lib.rtz_multi_render_denoised(self._m, C.byref(cam), int(guide_samples),
+                                                   C.byref(params) if params is not None else None,
+                                                   rgb.ctypes.data_as(C.POINTER(C.c_uint8)),
+                                                   lin.ctypes.data_as(C.POINTER(C.c_float)), C.byref(st)))
+        return rgb, lin, st
+
 
 def render_host_multi(camera, spheres, n: int | None = None, num_gpus: int = 0):
     """`rtz_render_multi`: the one-shot C-ABI call with HOST buffers on `num_gpus` devices (0 = all)."""
@@ -241,6 +270,27 @@ def render_host_multi(camera, spheres, n: int | None = None, num_gpus: int = 0):
     B.check(l.rtz_render_multi(C.byref(cam), C.cast(arr, C.POINTER(B.rtz_sphere)), n, int(num_gpus),
                                rgb.ctypes.data_as(C.POINTER(C.c_uint8)), C.byref(st)))
     return rgb, st
+
+
+def render_host_multi_denoised(camera, spheres, n: int | None = None, num_gpus: int = 0, guide_samples: int = 0,
+                               params: B.rtz_denoise_params | None = None):
+    """`rtz_render_multi_denoised`: `render_host_denoised` on `num_gpus` devices (0 = all), denoised on the first.
+    Returns (numpy uint8 [H,W,3], numpy float32 [H,W,3], stats)."""
+    import numpy as np
+
+    l = B.lib()
+    cam = _cast_camera(camera)
+    arr, cnt = _as_sphere_array(spheres)
+    n = cnt if n is None else int(n)
+    H, W = int(cam.height), int(cam.width)
+    rgb = np.empty((H, W, 3), dtype=np.uint8)
+    lin = np.empty((H, W, 3), dtype=np.float32)
+    st = B.rtz_stats()
+    B.check(l.rtz_render_multi_denoised(C.byref(cam), C.cast(arr, C.POINTER(B.rtz_sphere)), n, int(num_gpus),
+                                        int(guide_samples), C.byref(params) if params is not None else None,
+                                        rgb.ctypes.data_as(C.POINTER(C.c_uint8)),
+                                        lin.ctypes.data_as(C.POINTER(C.c_float)), C.byref(st)))
+    return rgb, lin, st
 
 
 def render_host_denoised(camera, spheres, n: int | None = None, guide_samples: int = 0,
