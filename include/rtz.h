@@ -216,11 +216,15 @@ int32_t rtz_render_resident_linear(rtz_context* ctx, const rtz_camera* camera, c
  * the sky colour the render returns for that ray on a miss; normal: the unit normal against the ray, (0,0,0) on a
  * miss.  Per pixel, the samples' f32 values are added in ascending sample order from +0 and divided by
  * guide_samples once; normals are not renormalised.  Guides do not depend on bounce_max, and RTZ_MODE_PATH_BVH
- * gives the buffers of RTZ_MODE_PATH.  RTZ_ERR_BAD_ARG for a legacy mode, has_seed == 0 (an OS-drawn seed would
+ * gives the buffers of RTZ_MODE_PATH.  In RTZ_MODE_PATH_BVH, for a scene of more than 512 spheres (padded to
+ * whole 32-sphere blocks), the hits are found through the BVH (built on first use, as for a BVH render); the buffers
+ * are still those of RTZ_MODE_PATH, bit for bit.  RTZ_ERR_BAD_ARG for a legacy mode, has_seed == 0 (an OS-drawn seed would
  * give other rays than the frame's), guide_samples == 0 or > samples_per_pixel, both outputs NULL, or more than
  * 2^31 - 1 work items (pixels for guide_samples >= 64).
  * stats: samples = segments = width*height*guide_samples, sphere_tests, kernel_launches, trace_ms = total_ms
- * (the guide kernel), seed_used; the rest 0.  Blocks like rtz_render_resident. */
+ * (the guide kernel), seed_used; the rest 0.  sphere_tests is segments * n for the brute-force sweeps and, through
+ * the BVH, the tests actually made (the rays that fill a warp's last 64 slots included).  Blocks like
+ * rtz_render_resident. */
 int32_t rtz_render_guides(rtz_context* ctx, const rtz_camera* camera, uint64_t guide_samples,
                           float* d_albedo_out, float* d_normal_out, rtz_stats* stats_out);
 

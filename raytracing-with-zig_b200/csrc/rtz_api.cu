@@ -127,7 +127,8 @@ struct rtz_context {
     int n_spheres = 0, n_pad = 0;
     // frame state
     DevBuf<unsigned long long> accum;
-    DevBuf<unsigned long long> counters;  // [0] queue head, [1..4] stats, [5] BVH tests, [6] NaN samples, [8] drain pool {parked, next}
+    DevBuf<unsigned long long> counters;  // [0] queue head, [1..4] stats, [5] BVH tests, [6] NaN samples, [7] BVH guide
+                                          // tests, [8] drain pool {parked, next}
     DevBuf<float4> pool;                  // drain pool: 4 float4 per parked path, 64 paths per resident warp
     uint64_t frame_launches = 0;          // kernels launched for the frame in flight
     DevBuf<unsigned long long> timeline;  // RTZ_TIMELINE=1: per-warp {start, queue dry, done} stamps of the last frame
@@ -579,8 +580,16 @@ int32_t check_guides(const rtz_camera* cam, uint64_t guide_samples) {
     return RTZ_OK;
 }
 
+// Whether the guides of this frame find their hits through the BVH (guides_kernel_bvh): a BVH-mode frame of a scene
+// beyond the constant bank, where the brute-force guides read every sphere from global memory.  At or below 512
+// spheres the constant-bank sweeps stay: the culled one beats the BVH on the final scene (DESIGN.md §5 K6).
+bool bvh_guides(const rtz_context* c, const rtz_camera* cam) {
+    return cam->mode == RTZ_MODE_PATH_BVH && c->n_pad > rtz::kMaxConstSpheres;
+}
+
 // Enqueue the guide kernel over the local pixels of shard `sg` (K6) on the context's stream, between ev[6] and ev[7];
-// no host wait.  Outputs compact (padding 0) or, `row_major`, at their places in row-major planes.
+// no host wait (except to build and upload the BVH the first time a scene needs it).  Outputs compact (padding 0) or,
+// `row_major`, at their places in row-major planes.  The BVH kernel counts its sphere tests into counters[7].
 int32_t enqueue_guides(rtz_context* c, const rtz_camera* cam, const rtz::ShardGeom& sg, uint64_t guide_samples,
                        float* d_albedo, float* d_normal, bool row_major) {
     const uint64_t n_local = (uint64_t)sg.n_local_tiles * sg.tile_pixels;
@@ -598,9 +607,18 @@ int32_t enqueue_guides(rtz_context* c, const rtz_camera* cam, const rtz::ShardGe
     P.rcp_tile_pixels = rcp(sg.tile_pixels), P.rcp_tiles_x = rcp(sg.tiles_x), P.rcp_tile_w = rcp(sg.tile_w);
     P.albedo_out = d_albedo, P.normal_out = d_normal;
     const unsigned blocks = P.n_items;
-    // every mode sweeps by brute force here (the BVH finds the same hits), on the rows the render's sweep reads
+    const bool bvh = bvh_guides(c, cam);
+    if (bvh) {
+        const int32_t rc = ensure_bvh(c);
+        if (rc != RTZ_OK) return rc;
+    }
+    // the brute-force sweeps read the rows the render's sweep reads
     RTZ_CUDA(cudaEventRecord(c->ev[6], c->stream));
-    if (c->n_pad <= rtz::kMaxConstSpheres && c->geo_const) {
+    if (bvh) {
+        RTZ_CUDA(cudaMemsetAsync(c->counters.p + 7, 0, sizeof(unsigned long long), c->stream));
+        const rtz::GuideParamsBvh B{P, c->bvh_nodes.p, c->bvh_order.p, c->wexp.p, c->bvh_r2, c->counters.p + 7};
+        rtz::guides_kernel_bvh<<<blocks, 32, 0, c->stream>>>(B);
+    } else if (c->n_pad <= rtz::kMaxConstSpheres && c->geo_const) {
         static thread_local rtz::GuideParamsConst C;  // 8.5 KiB: keep it off the stack
         if (c->cull) {
             P.geom = c->rg_geom.p, P.aux = c->rg_aux.p, P.albedo = c->rg_albedo.p, P.wexp = c->rg_wexp.p;
@@ -1158,11 +1176,15 @@ int32_t rtz_render_guides_sharded(rtz_context* c, const rtz_camera* cam, const r
     RTZ_CUDA(cudaSetDevice(c->device));
     rc = enqueue_guides(c, cam, sg, guide_samples, d_albedo, d_normal, false);
     if (rc != RTZ_OK) return rc;
+    const bool bvh = bvh_guides(c, cam);
+    if (bvh)
+        RTZ_CUDA(cudaMemcpyAsync(c->h_counters + 7, c->counters.p + 7, sizeof(unsigned long long),
+                                 cudaMemcpyDeviceToHost, c->stream));
     RTZ_CUDA(cudaStreamSynchronize(c->stream));
     if (st) {
         std::memset(st, 0, sizeof(*st));
         st->samples = st->segments = shard_real_pixels(cam, sg) * guide_samples;
-        st->sphere_tests = st->segments * (uint64_t)c->n_spheres;
+        st->sphere_tests = bvh ? c->h_counters[7] : st->segments * (uint64_t)c->n_spheres;
         st->kernel_launches = 1;
         float ms = 0;
         cudaEventElapsedTime(&ms, c->ev[6], c->ev[7]), st->trace_ms = st->total_ms = ms;

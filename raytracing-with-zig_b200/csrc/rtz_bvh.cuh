@@ -77,8 +77,8 @@ __device__ __forceinline__ bool hit_box(const float* lo, const float* hi, float 
 }
 
 constexpr int kBvhDone = (int)0x80000000;
-template <int kBlock, bool kFar>
-__device__ __forceinline__ void bvh_walk(const BvhParams& B, const Path& p, const RayK& k, float tmin_d, float& closest,
+template <int kBlock, bool kFar, class BP>
+__device__ __forceinline__ void bvh_walk(const BP& B, const Path& p, const RayK& k, float tmin_d, float& closest,
                                          int& best, int* stack, float* tstack, unsigned long long& n_tests) {
     const float ix = 1.0f / p.dx, iy = 1.0f / p.dy, iz = 1.0f / p.dz;
     const float4* geom = B.p.geom;
@@ -127,8 +127,9 @@ __device__ __forceinline__ void bvh_walk(const BvhParams& B, const Path& p, cons
 // Closest hit through the hierarchy.  "While-while" traversal: a warp first walks inner nodes until every lane
 // holds a leaf (or is done), then all lanes test their leaves together, so that box tests and sphere tests
 // are not interleaved lane by lane.  A popped entry whose box lies beyond the current closest hit is skipped.
-template <int kBlock>
-__device__ __forceinline__ void bvh_closest_hit(const BvhParams& B, const Path& p, float tmin, float tmax, int* stack,
+// B: BvhParams, or any struct with its fields nodes, order, wexp, r2 and p.geom (GuideParamsBvh).
+template <int kBlock, class BP>
+__device__ __forceinline__ void bvh_closest_hit(const BP& B, const Path& p, float tmin, float tmax, int* stack,
                                                 float* tstack, float& t_out, int& best_out, unsigned long long& n_tests) {
     const RayK k = ray_constants(p);
     const float tmin_d = tmin * p.len;

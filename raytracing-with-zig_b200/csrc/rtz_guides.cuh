@@ -4,7 +4,8 @@
 // The guide kernel does not share a launch with the render.  It regenerates the frame's camera rays (camera_ray with
 // the key (seed, j*W + i, s), bounce 0: the render's first ray of sample s, bit for bit) and finds their closest hit
 // with the render's own sweep (sweep2, unchanged), so its hits are the ones the render's first world.hit returns:
-// the (t, original index) minimum over Scene.interval, with the same gate and roots.
+// the (t, original index) minimum over Scene.interval, with the same gate and roots.  RTZ_MODE_PATH_BVH scenes beyond
+// the constant bank find that minimum through the hierarchy instead (guides_kernel_bvh): the same buffers bit for bit.
 //
 // Per ray, six f32 values:
 //   albedo  hit: the sphere's albedo for lambertian and metal (the attenuation scatter applies), (1, 1, 1) for
@@ -27,6 +28,7 @@
 // A tile-padding pixel still sweeps rays (those of pixel (min(x, W-1), min(y, H-1))) so that every lane takes part in
 // the sweep's votes; its sums are never stored into a real pixel.
 #pragma once
+#include "rtz_bvh.cuh"
 #include "rtz_kernels.cuh"
 
 namespace rtz {
@@ -125,10 +127,11 @@ __device__ __forceinline__ void guide_store(const GuideParams& P, unsigned long 
     out[3ull * (uint32_t)dest + (c < 3 ? c : c - 3)] = dest >= kGuidePadding ? 0.0f : value;
 }
 
-template <bool kConstBank, bool kCull>
-__device__ __forceinline__ void guide_body(const GuideParams& P, const float4* __restrict__ pairs,
-                                           float* __restrict__ stage_mem, const float4* __restrict__ boxes = nullptr,
-                                           float cull_r2 = 0.0f, int split_max = 0) {
+// The work split and fold of every guide kernel, over its staging rows (kGuideStageFloats or more).
+// sweep(P, a, b, ta, ia, tb, ib, stage) finds the closest hits of the lane's two rays, called by the whole (converged)
+// warp; it may use the staging rows as scratch until it returns.
+template <class Sweep>
+__device__ __forceinline__ void guide_body(const GuideParams& P, float* __restrict__ stage_mem, Sweep sweep) {
     float* const stage = stage_mem;
     // one warp per block, so that the work item is visibly warp-uniform to ptxas: with the item derived from the warp
     // index inside a wider block, it guards the sweep's votes with divergent-branch checks (BRA.DIV)
@@ -150,8 +153,7 @@ __device__ __forceinline__ void guide_body(const GuideParams& P, const float4* _
         __syncwarp();  // converged before the sweep's votes
         float ta = 0.f, tb = 0.f;
         int ia = -1, ib = -1;
-        sweep2<kConstBank, false, kCull>(pairs, P.geom, P.n_pad, cam.tmin, cam.tmax, a, b, ta, ia, tb, ib, boxes, cull_r2,
-                                         P.orig, P.wexp, split_max, reinterpret_cast<float4*>(stage));
+        sweep(P, a, b, ta, ia, tb, ib, stage);
         __syncwarp();  // the culled sweep reads its staging rows (the same memory) until it returns
         guide_values(P, a, ta, ia, stage, lane);
         guide_values(P, b, tb, ib, stage, 32 + lane);
@@ -173,18 +175,75 @@ __device__ __forceinline__ void guide_body(const GuideParams& P, const float4* _
     if (g >= 64 && lane < 6) guide_store(P, dest[0], lane, acc / (float)g);
 }
 
-// Scenes the render sweeps from the constant bank (n_pad <= kMaxConstSpheres): the same rows, through the same
-// uniform loads; kCull = the culled kernel's regrouped rows, boxes and sphere-parallel split.
+// The render's brute-force sweep (sweep2) over the rows it reads from the constant bank (n_pad <= kMaxConstSpheres):
+// the same rows, through the same uniform loads; kCull = the culled kernel's regrouped rows, boxes and sphere-parallel
+// split.
+template <bool kCull>
+struct GuideSweepConst {
+    const GuideParamsConst& C;
+    __device__ __forceinline__ void operator()(const GuideParams& P, const Path& a, const Path& b, float& ta, int& ia,
+                                               float& tb, int& ib, float* stage) const {
+        sweep2<true, false, kCull>(C.pairs, P.geom, P.n_pad, P.cam.tmin, P.cam.tmax, a, b, ta, ia, tb, ib, C.boxes,
+                                   C.cull_r2, P.orig, P.wexp, C.split_max, reinterpret_cast<float4*>(stage));
+    }
+};
+
+// ... and over the plain pair rows in global memory (L1 / L2, warp-uniform addresses), for larger scenes
+struct GuideSweepGlobal {
+    const float4* __restrict__ pairs;
+    __device__ __forceinline__ void operator()(const GuideParams& P, const Path& a, const Path& b, float& ta, int& ia,
+                                               float& tb, int& ib, float* stage) const {
+        sweep2<false, false, false>(pairs, P.geom, P.n_pad, P.cam.tmin, P.cam.tmax, a, b, ta, ia, tb, ib, nullptr,
+                                    0.0f, P.orig, P.wexp, 0, reinterpret_cast<float4*>(stage));
+    }
+};
+
 template <bool kCull>
 __global__ void __launch_bounds__(32, 24) guide_kernel_const(const __grid_constant__ GuideParamsConst C) {
     __shared__ __align__(16) float stage[kCull ? kCullStageFloats : kGuideStageFloats];
-    guide_body<true, kCull>(C.p, C.pairs, stage, C.boxes, C.cull_r2, C.split_max);
+    guide_body(C.p, stage, GuideSweepConst<kCull>{C});
 }
 
-// Larger scenes: the plain pair rows from global memory (L1 / L2, warp-uniform addresses).
 __global__ void __launch_bounds__(32, 24) guide_kernel_global(const __grid_constant__ GuideParams P) {
     __shared__ __align__(16) float stage[kGuideStageFloats];
-    guide_body<false, false>(P, P.pairs, stage);
+    guide_body(P, stage, GuideSweepGlobal{P.pairs});
+}
+
+// The BVH form: BvhParams' fields around the guide parameters (bvh_closest_hit reads them by name).
+struct GuideParamsBvh {
+    GuideParams p;               // geom: the plain rows, which the hierarchy's `order` indexes
+    const BvhNode* nodes;
+    const int* order;
+    const float* wexp;
+    float r2;
+    unsigned long long* tests;   // += the sphere tests the traversal makes (every slot's, padding included)
+};
+
+// The lane's two rays through the hierarchy, one after the other, on trace_kernel_bvh's shared-memory stacks
+struct GuideSweepBvh {
+    const GuideParamsBvh& B;
+    int* stack;
+    float* tstack;
+    unsigned long long& n_tests;
+    __device__ __forceinline__ void operator()(const GuideParams& P, const Path& a, const Path& b, float& ta, int& ia,
+                                               float& tb, int& ib, float*) const {
+        bvh_closest_hit<32>(B, a, P.cam.tmin, P.cam.tmax, stack, tstack, ta, ia, n_tests);
+        bvh_closest_hit<32>(B, b, P.cam.tmin, P.cam.tmax, stack, tstack, tb, ib, n_tests);
+    }
+};
+
+// RTZ_MODE_PATH_BVH scenes beyond the constant bank (n_pad > kMaxConstSpheres), where guide_kernel_global would read
+// every sphere for every ray.  The traversal returns the (t, original index) minimum, which is the brute-force
+// sweep's answer, so the buffers are guide_kernel_global's bit for bit.
+__global__ void __launch_bounds__(32, 24) guides_kernel_bvh(const __grid_constant__ GuideParamsBvh B) {
+    __shared__ __align__(16) float stage[kGuideStageFloats];
+    __shared__ int s_stack[kBvhMaxDepth * 32];
+    __shared__ float s_tstack[kBvhMaxDepth * 32];
+    unsigned long long n_tests = 0;
+    guide_body(B.p, stage, GuideSweepBvh{B, s_stack + threadIdx.x, s_tstack + threadIdx.x, n_tests});
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) n_tests += __shfl_xor_sync(0xFFFFFFFFu, n_tests, o);
+    if (threadIdx.x == 0) atomicAdd(B.tests, n_tests);
 }
 
 }  // namespace rtz
