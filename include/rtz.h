@@ -180,10 +180,19 @@ int32_t rtz_context_destroy(rtz_context* ctx);
  * src/hittable.zig:60-62, for the whole list at once). */
 int32_t rtz_scene_upload(rtz_context* ctx, const rtz_sphere* spheres, uint64_t n_spheres);
 
+/* rtz_scene_upload of a list that is already in DEVICE memory: d_spheres holds n_spheres records, in device or
+ * managed memory usable from the context's device (else RTZ_ERR_BAD_ARG).  They are read on the context's stream, so
+ * the caller orders them like any other input of the resident API; the call returns once they have been read and
+ * keeps nothing of them.  The context's state afterwards is that of rtz_scene_upload of the same list, bit for bit,
+ * and so are its refusals: the same status and rtz_last_error for the same first refused sphere, the installed scene
+ * left as it was.  Up to 512 padded spheres the list comes to the host (<= 40 KiB) and takes rtz_scene_upload's path;
+ * larger lists are checked and flattened on the device, without the host pass rtz_scene_upload makes. */
+int32_t rtz_scene_upload_device(rtz_context* ctx, const rtz_sphere* d_spheres, uint64_t n_spheres);
+
 /* Scene.init(seed) followed by Scene.generateWorld / generateChapter13 (src/Scene.zig:23-46, 48-134,
  * 136-182), or BASELINE config 5's generalised final scene of exactly n_spheres spheres, generated ON THE
  * DEVICE by one thread with the reference's exact PRNG stream (Zig std DefaultPrng = Xoshiro256++ seeded by
- * SplitMix64, Random.float(f64)), then installed as the context's scene like rtz_scene_upload does.
+ * SplitMix64, Random.float(f64)), then installed from device memory as the context's scene (rtz_scene_upload_device).
  * spheres_out (optional, host, `cap` entries) receives the f64 spheres in list order, *n_out their number,
  * prng_state_out (optional) the four words of Scene.prng after generation.  (SURVEY.md 8f row 2.) */
 #define RTZ_SCENE_FINAL 0      /* generateWorld: ~485 spheres                                  */
@@ -473,6 +482,24 @@ int32_t rtz_probe_cull_bounds(const rtz_sphere* spheres, uint64_t n_spheres, flo
 #define RTZ_SWEEP_WAVE4 8
 int32_t rtz_probe_sweeps(const rtz_sphere* spheres, uint64_t n_spheres, const rtz_probe_ray* rays, uint64_t m,
                          double t_min, double t_max, int32_t kind, int32_t split_max, rtz_ray_hit* out);
+
+/* The rows a context holds for its scene, back to back, for comparing two installs byte for byte: int32 n_spheres,
+ * n_pad, cull; f32 cull_r2; then the device rows geom, pairs, aux, albedo (n_pad float4 each), wexp (n_pad f32) and the
+ * f64 spheres of the legacy kernel (n_spheres x 32 B); for n_pad <= 512 also the constant-bank pair rows and block
+ * boxes and, for a culled scene, the regrouped rows and slot -> index map.  *bytes_out receives the size; out NULL
+ * asks for the size only, a smaller cap is RTZ_ERR_BAD_ARG. */
+int32_t rtz_probe_scene_rows(rtz_context* ctx, void* out, uint64_t cap, uint64_t* bytes_out);
+
+/* The BVH of RTZ_MODE_PATH_BVH for the context's scene, built by `builder` without installing it: the nodes (64 B
+ * each, pre-order, root first) to nodes_out, the leaf ranges' sphere indices to order_out (n_spheres entries), the
+ * squared origin radius the boxes cover to r2_out; *n_nodes_out receives the node count.  Any output may be NULL;
+ * node_cap below the count is RTZ_ERR_BAD_ARG.  Both builders give the same nodes and r2 and the same set of spheres
+ * in every leaf (order inside a leaf may differ); a render picks one by scene size.  Below 5 spheres the device
+ * builder hands over to the host one. */
+#define RTZ_BVH_HOST 0
+#define RTZ_BVH_DEVICE 1
+int32_t rtz_probe_bvh(rtz_context* ctx, int32_t builder, void* nodes_out, uint64_t node_cap, int32_t* order_out,
+                      float* r2_out, uint64_t* n_nodes_out);
 
 /* Color.toRgb (src/color.zig:63-80) on the device for `n` colours (3 f64 each). */
 int32_t rtz_probe_to_rgb(const double* linear, uint64_t n, uint8_t* rgb_out);

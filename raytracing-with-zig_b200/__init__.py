@@ -9,6 +9,6 @@ Only what the hot path needs:
   distributed.py   interleaved-tile sharding + NCCL gather (one process per GPU)
 """
 from .binding import RtzError, lib, rtz_camera, rtz_denoise_params, rtz_shard, rtz_sphere, rtz_stats  # noqa: F401
-from .renderer import (MultiRenderer, Renderer, render_host, render_host_denoised, render_host_multi,  # noqa: F401
-                       render_host_multi_denoised)
+from .renderer import (MultiRenderer, Renderer, pack_spheres, render_host, render_host_denoised,  # noqa: F401
+                       render_host_multi, render_host_multi_denoised)
 from .distributed import render_sharded, render_sharded_denoised, tile_index_map  # noqa: F401

@@ -70,6 +70,7 @@ ABI_VERSION = 2
 # rtz_probe_sweeps kinds (include/rtz.h)
 (SWEEP_CONST, SWEEP_CULL, SWEEP_SKIP_SELF, SWEEP_SMEM, SWEEP_GLOBAL, SWEEP_COOP, SWEEP_COOP_REGROUPED,
  SWEEP_BVH, SWEEP_WAVE4) = range(9)
+BVH_HOST, BVH_DEVICE = 0, 1   # rtz_probe_bvh builders
 
 # every symbol include/rtz.h declares, with its signature
 _u8p, _f64p, _f32p = C.POINTER(C.c_uint8), C.POINTER(C.c_double), C.POINTER(C.c_float)
@@ -81,6 +82,7 @@ SIGNATURES = {
     "rtz_context_create": (_i32, [_i32, _vp, C.POINTER(_vp)]),
     "rtz_context_destroy": (_i32, [_vp]),
     "rtz_scene_upload": (_i32, [_vp, C.POINTER(rtz_sphere), _u64]),
+    "rtz_scene_upload_device": (_i32, [_vp, _vp, _u64]),
     "rtz_scene_generate": (_i32, [_vp, _i32, _u64, _u64, C.POINTER(rtz_sphere), _u64, C.POINTER(_u64), C.POINTER(_u64)]),
     "rtz_shard_pixels": (_u64, [_u64, _u64, C.POINTER(rtz_shard)]),
     "rtz_render_resident": (_i32, [_vp, C.POINTER(rtz_camera), C.POINTER(rtz_shard), _vp, C.POINTER(rtz_stats)]),
@@ -115,6 +117,8 @@ SIGNATURES = {
     "rtz_probe_sweep_order": (_i32, [C.POINTER(rtz_sphere), _u64, C.POINTER(_i32)]),
     "rtz_probe_cull_bounds": (_i32, [C.POINTER(rtz_sphere), _u64, _f32p, _f32p, C.POINTER(_i32)]),
     "rtz_probe_sweeps": (_i32, [C.POINTER(rtz_sphere), _u64, _vp, _u64, _f64, _f64, _i32, _i32, _vp]),
+    "rtz_probe_scene_rows": (_i32, [_vp, _vp, _u64, C.POINTER(_u64)]),
+    "rtz_probe_bvh": (_i32, [_vp, _i32, _vp, _u64, C.POINTER(_i32), _f32p, C.POINTER(_u64)]),
     "rtz_probe_uniform": (_i32, [_u64, _u32, _u32, _u32, _u64, _f32p]),
     "rtz_probe_camera_ray": (_i32, [C.POINTER(rtz_camera), _u64, _u64, _u64, _u64, _f32p, _f32p, _f32p]),
     "rtz_strerror": (C.c_char_p, [_i32]),

@@ -27,6 +27,7 @@
 #include "rtz_guides.cuh"
 #include "rtz_denoise.cuh"
 #include "rtz_bvh.cuh"
+#include "rtz_bvh_build.cuh"
 #include "rtz_scene.cuh"
 
 namespace {
@@ -124,6 +125,14 @@ struct rtz_context {
     std::vector<float> h_w;
     float bvh_r2 = 0.0f;  // BvhParams::r2
     bool bvh_ready = false;
+    // scratch of the device BVH builder (build_bvh_device): sort keys, sphere indices, per-sphere boxes, the ranges
+    // of one level and the next, their accumulators and axes, CUB's temporary storage; [0] of bb_misc: R's bits
+    DevBuf<unsigned long long> bb_keys0, bb_keys1, bb_misc;
+    DevBuf<int> bb_idx, bb_order, bb_seg, bb_axis;
+    DevBuf<float4> bb_lo, bb_hi;
+    DevBuf<rtz::BuildRange> bb_rg0, bb_rg1;
+    DevBuf<unsigned> bb_acc;
+    DevBuf<uint8_t> bb_temp;
     int n_spheres = 0, n_pad = 0;
     // frame state
     DevBuf<unsigned long long> accum;
@@ -756,6 +765,9 @@ int32_t rtz_context_destroy(rtz_context* c) {
     c->bvh_nodes.release(), c->bvh_order.release(), c->wexp.release();
     c->rg_geom.release(), c->rg_aux.release(), c->rg_albedo.release(), c->rg_wexp.release(), c->rg_orig.release();
     c->denoise.release(), c->denoise_io.release();
+    c->bb_keys0.release(), c->bb_keys1.release(), c->bb_misc.release(), c->bb_idx.release(), c->bb_order.release();
+    c->bb_seg.release(), c->bb_axis.release(), c->bb_lo.release(), c->bb_hi.release(), c->bb_rg0.release();
+    c->bb_rg1.release(), c->bb_acc.release(), c->bb_temp.release();
     for (auto& e : c->ev)
         if (e) cudaEventDestroy(e);
     if (c->h_counters) cudaFreeHost(c->h_counters);
@@ -895,7 +907,37 @@ struct HostScene {
     double R = 0.0;
     bool cull = false;
 };
-int32_t host_scene(const rtz_sphere* sp, uint64_t n, HostScene& s) {
+// Whether the renderer accepts sphere i of a list: RTZ_ERR_BAD_ARG (and g_last_error) for one it refuses.
+int32_t check_sphere(const rtz_sphere& sph, uint64_t i) {
+    if (sph.mat_type < RTZ_MAT_LAMBERTIAN || sph.mat_type > RTZ_MAT_DIELECTRIC) return RTZ_ERR_BAD_ARG;
+    const float r = (float)(sph.radius < 0 ? 0.0 : sph.radius);  // Sphere.init clamp (src/sphere.zig:21)
+    // A radius-0 sphere makes the reference panic in Vec.divScalar (src/vec.zig:39-45) when it is hit, and
+    // NaN / infinite geometry only yields NaN samples: both are refused here instead of rendered wrongly.
+    const bool mat_ok = sph.mat_type == RTZ_MAT_DIELECTRIC
+                            ? (std::isfinite(sph.refraction_index) && (float)sph.refraction_index != 0.0f)
+                            : (finite3(sph.albedo) && (sph.mat_type != RTZ_MAT_METAL || std::isfinite(sph.fuzz)));
+    if (!finite3(sph.center) || !std::isfinite(sph.radius) || !(r > 0.0f) || !mat_ok) {
+        g_last_error = "sphere " + std::to_string(i) + ": radius must be > 0 and every field of its material finite";
+        return RTZ_ERR_BAD_ARG;
+    }
+    // The pixel sums are unsigned 32.32 fixed point and every sample is clamped at 0 before it is added
+    // (to_fixed): exact only while samples lie in [0, 1], i.e. while every albedo a path multiplies does.
+    // Dielectric scatter never reads the albedo.
+    if (sph.mat_type != RTZ_MAT_DIELECTRIC)
+        for (int k = 0; k < 3; ++k)
+            if (!(sph.albedo[k] >= 0.0 && sph.albedo[k] <= 1.0)) {
+                char v[32];
+                std::snprintf(v, sizeof v, "%.17g", sph.albedo[k]);
+                g_last_error = "sphere " + std::to_string(i) + ": albedo[" + std::to_string(k) + "] = " + v +
+                               " is outside [0, 1]";
+                return RTZ_ERR_BAD_ARG;
+            }
+    return RTZ_OK;
+}
+
+// `regrouped`: also the culled kernel's order, block boxes, cull_r2 and cull decision, which a context needs only for
+// a scene the constant bank holds (n_pad <= 512): above, they are computed only when asked for.
+int32_t host_scene(const rtz_sphere* sp, uint64_t n, HostScene& s, bool regrouped = false) {
     const int n_pad = (int)((n + 7) & ~7ull);
     s.n_pad = n_pad;
     std::vector<float4>&g = s.g, &a = s.a, &al = s.al;
@@ -905,29 +947,9 @@ int32_t host_scene(const rtz_sphere* sp, uint64_t n, HostScene& s) {
     s.ds.assign(n ? n : 1, rtz::DSphere{});
     for (uint64_t i = 0; i < n; ++i) {
         const rtz_sphere& sph = sp[i];
-        if (sph.mat_type < RTZ_MAT_LAMBERTIAN || sph.mat_type > RTZ_MAT_DIELECTRIC) return RTZ_ERR_BAD_ARG;
-        const float r = (float)(sph.radius < 0 ? 0.0 : sph.radius);  // Sphere.init clamp (src/sphere.zig:21)
-        // A radius-0 sphere makes the reference panic in Vec.divScalar (src/vec.zig:39-45) when it is hit, and
-        // NaN / infinite geometry only yields NaN samples: both are refused here instead of rendered wrongly.
-        const bool mat_ok = sph.mat_type == RTZ_MAT_DIELECTRIC
-                                ? (std::isfinite(sph.refraction_index) && (float)sph.refraction_index != 0.0f)
-                                : (finite3(sph.albedo) && (sph.mat_type != RTZ_MAT_METAL || std::isfinite(sph.fuzz)));
-        if (!finite3(sph.center) || !std::isfinite(sph.radius) || !(r > 0.0f) || !mat_ok) {
-            g_last_error = "sphere " + std::to_string(i) + ": radius must be > 0 and every field of its material finite";
-            return RTZ_ERR_BAD_ARG;
-        }
-        // The pixel sums are unsigned 32.32 fixed point and every sample is clamped at 0 before it is added
-        // (to_fixed): exact only while samples lie in [0, 1], i.e. while every albedo a path multiplies does.
-        // Dielectric scatter never reads the albedo.
-        if (sph.mat_type != RTZ_MAT_DIELECTRIC)
-            for (int k = 0; k < 3; ++k)
-                if (!(sph.albedo[k] >= 0.0 && sph.albedo[k] <= 1.0)) {
-                    char v[32];
-                    std::snprintf(v, sizeof v, "%.17g", sph.albedo[k]);
-                    g_last_error = "sphere " + std::to_string(i) + ": albedo[" + std::to_string(k) + "] = " + v +
-                                   " is outside [0, 1]";
-                    return RTZ_ERR_BAD_ARG;
-                }
+        const int32_t rc = check_sphere(sph, i);
+        if (rc != RTZ_OK) return rc;
+        const float r = (float)(sph.radius < 0 ? 0.0 : sph.radius);
         const float cx = (float)sph.center[0], cy = (float)sph.center[1], cz = (float)sph.center[2];
         // q = |c|^2 - r^2 of the FP32-rounded sphere less the per-sphere half of the gate's margin (kGateSlack at
         // ray_constants), evaluated in f64 and rounded once
@@ -948,6 +970,7 @@ int32_t host_scene(const rtz_sphere* sp, uint64_t n, HostScene& s) {
         al[i] = make_float4(0.f, 0.f, 0.f, 0.f);
     }
     s.pairs = pair_rows(g, w, n_pad);
+    if (n_pad > rtz::kMaxConstSpheres && !regrouped) return RTZ_OK;
     // Bounds of the culled kernel's 32-sphere blocks, on its regrouped order (box_reach in rtz_kernels.cuh states
     // the exactness contract these paddings serve).  R covers every ray origin within twice the farthest point of
     // a sphere outside block 0; block 0 (the ground of the book's scenes) has no box: it is always swept.
@@ -1000,7 +1023,7 @@ int32_t scene_upload(rtz_context* c, const rtz_sphere* sp, uint64_t n, bool regr
     DeviceGuard guard;
     RTZ_CUDA(cudaSetDevice(c->device));
     HostScene s;
-    const int32_t rc = host_scene(sp, n, s);
+    const int32_t rc = host_scene(sp, n, s, regrouped);
     if (rc != RTZ_OK) return rc;
     const int n_pad = s.n_pad;
     const bool rows = s.cull || (regrouped && n_pad);
@@ -1059,26 +1082,175 @@ int32_t scene_upload(rtz_context* c, const rtz_sphere* sp, uint64_t n, bool regr
     c->n_spheres = (int)n, c->n_pad = n_pad;
     return RTZ_OK;
 }
+
+// rtz_scene_upload of a DEVICE list (the context's device selected, d_sp checked).  A scene the constant bank holds
+// comes to the host (<= 40 KiB) and takes scene_upload; a larger one is checked and flattened on the device, with
+// the host's tests and arithmetic (rtz_bvh_build.cuh), and skips the rows only the constant-bank kernels read.
+int32_t scene_upload_device(rtz_context* c, const rtz_sphere* d_sp, uint64_t n) {
+    const uint64_t n_pad = (n + 7) & ~7ull;
+    if (n_pad <= (uint64_t)rtz::kMaxConstSpheres) {
+        std::vector<rtz_sphere> h(n);
+        if (n) {
+            RTZ_CUDA(cudaMemcpyAsync(h.data(), d_sp, n * sizeof(rtz_sphere), cudaMemcpyDeviceToHost, c->stream));
+            RTZ_CUDA(cudaStreamSynchronize(c->stream));
+        }
+        return scene_upload(c, h.data(), n, false);
+    }
+    // the lowest refused index, and the host's verdict and message on that one sphere; the installed scene stays
+    RTZ_CUDA(c->bb_misc.reserve(2));
+    RTZ_CUDA(cudaMemsetAsync(c->bb_misc.p + 1, 0xFF, sizeof(unsigned long long), c->stream));
+    rtz::scene_check_kernel<<<(unsigned)((n + 255) / 256), 256, 0, c->stream>>>(d_sp, n, c->bb_misc.p + 1);
+    RTZ_CUDA(cudaGetLastError());
+    unsigned long long bad = 0;
+    RTZ_CUDA(cudaMemcpyAsync(&bad, c->bb_misc.p + 1, sizeof bad, cudaMemcpyDeviceToHost, c->stream));
+    RTZ_CUDA(cudaStreamSynchronize(c->stream));
+    if (bad < n) {
+        rtz_sphere rec;
+        RTZ_CUDA(cudaMemcpyAsync(&rec, d_sp + bad, sizeof rec, cudaMemcpyDeviceToHost, c->stream));
+        RTZ_CUDA(cudaStreamSynchronize(c->stream));
+        return check_sphere(rec, bad) != RTZ_OK ? RTZ_ERR_BAD_ARG : RTZ_ERR_CUDA;  // RTZ_ERR_CUDA: the tests disagree
+    }
+    // as scene_upload: no scene from here until every row is written
+    c->n_spheres = c->n_pad = 0;
+    c->h_pairs.clear(), c->h_rg_pairs.clear(), c->h_geom.clear(), c->h_w.clear(), c->h_boxes.clear();
+    c->cull_r2 = 0.0f;
+    c->cull = false;
+    c->bvh_ready = false;
+    RTZ_CUDA(c->geom.reserve(n_pad));
+    RTZ_CUDA(c->pairs.reserve(n_pad));
+    RTZ_CUDA(c->aux.reserve(n_pad));
+    RTZ_CUDA(c->albedo.reserve(n_pad));
+    RTZ_CUDA(c->wexp.reserve(n_pad));
+    RTZ_CUDA(c->dspheres.reserve(n));
+    const rtz::SceneRowsOut o{c->geom.p, c->pairs.p, c->aux.p, c->albedo.p, c->wexp.p, c->dspheres.p};
+    rtz::scene_flatten_kernel<<<(unsigned)((n_pad / 2 + 255) / 256), 256, 0, c->stream>>>(d_sp, n, (uint32_t)n_pad, o);
+    RTZ_CUDA(cudaGetLastError());
+    RTZ_CUDA(cudaStreamSynchronize(c->stream));  // the caller may reuse d_sp at return
+    c->n_spheres = (int)n, c->n_pad = (int)n_pad;
+    return RTZ_OK;
+}
 }  // namespace
 
 int32_t rtz_scene_upload(rtz_context* c, const rtz_sphere* sp, uint64_t n) { return scene_upload(c, sp, n, false); }
 
+int32_t rtz_scene_upload_device(rtz_context* c, const rtz_sphere* d_sp, uint64_t n) {
+    if (!c || (!d_sp && n) || n > (1u << 20)) return RTZ_ERR_BAD_ARG;
+    DeviceGuard guard;
+    RTZ_CUDA(cudaSetDevice(c->device));
+    if (n) {
+        cudaPointerAttributes pa{};
+        const cudaError_t e = cudaPointerGetAttributes(&pa, d_sp);
+        if (e != cudaSuccess) cudaGetLastError();
+        if (e != cudaSuccess ||
+            !(pa.type == cudaMemoryTypeManaged || (pa.type == cudaMemoryTypeDevice && pa.device == c->device))) {
+            g_last_error = "rtz_scene_upload_device: the spheres are not device or managed memory of the context's device";
+            return RTZ_ERR_BAD_ARG;
+        }
+    }
+    return scene_upload_device(c, d_sp, n);
+}
+
 }  // extern "C"
 
 namespace {
+// Scenes of at least this many spheres build their BVH on the device (build_bvh_device), smaller ones on the host
+// (BvhBuilder): the same tree either way, so only the time differs (the crossover: DESIGN.md §5 K8).
+constexpr int kDeviceBvhMinSpheres = 8192;
+
+// BvhBuilder's input: the FP32 rows {cx, cy, cz, -r^2} of the n spheres, read back for a scene installed from device
+// memory
+int32_t host_geom(rtz_context* c) {
+    const size_t n = (size_t)c->n_spheres;
+    if (c->h_geom.size() == n) return RTZ_OK;
+    c->h_geom.resize(n);
+    RTZ_CUDA(cudaMemcpyAsync(c->h_geom.data(), c->geom.p, n * sizeof(float4), cudaMemcpyDeviceToHost, c->stream));
+    RTZ_CUDA(cudaStreamSynchronize(c->stream));
+    return RTZ_OK;
+}
+
+// BvhBuilder's tree for the context's scene of n >= 5 spheres, built on the device level by level (rtz_bvh_build.cuh)
+// into nodes[bvh_inner_nodes(n)] and order[n]; *R_out = BvhBuilder::R.  Synchronises the stream.
+int32_t build_bvh_device(rtz_context* c, rtz::BvhNode* nodes, int* order, double* R_out) {
+    const int n = c->n_spheres;
+    cudaStream_t st = c->stream;
+    const unsigned gb = (unsigned)((n + 255) / 256);
+    int last = 0;  // the deepest level with ranges: the one below the last level that splits
+    while (rtz::bvh_level_splits(n, last)) ++last;
+    const int max_ranges = 1 << last;
+    size_t t0 = 0, t1 = 0;
+    RTZ_CUDA(cub::DeviceRadixSort::SortKeys(nullptr, t0, (unsigned long long*)nullptr, (unsigned long long*)nullptr, n, 0, 64, st));
+    RTZ_CUDA(cub::DeviceRadixSort::SortPairs(nullptr, t1, (unsigned long long*)nullptr, (unsigned long long*)nullptr,
+                                             (int*)nullptr, (int*)nullptr, n, 0, 64, st));
+    RTZ_CUDA(c->bb_temp.reserve(std::max(t0, t1)));
+    RTZ_CUDA(c->bb_keys0.reserve(n));
+    RTZ_CUDA(c->bb_keys1.reserve(n));
+    RTZ_CUDA(c->bb_idx.reserve(n));
+    RTZ_CUDA(c->bb_seg.reserve(n));
+    RTZ_CUDA(c->bb_lo.reserve(n));
+    RTZ_CUDA(c->bb_hi.reserve(n));
+    RTZ_CUDA(c->bb_rg0.reserve(max_ranges));
+    RTZ_CUDA(c->bb_rg1.reserve(max_ranges));
+    RTZ_CUDA(c->bb_acc.reserve((size_t)rtz::kBuildAcc * max_ranges));
+    RTZ_CUDA(c->bb_axis.reserve(max_ranges));
+    RTZ_CUDA(c->bb_misc.reserve(2));
+    RTZ_CUDA(cudaMemsetAsync(c->bb_misc.p, 0, sizeof(unsigned long long), st));
+    rtz::bvh_reach_kernel<<<gb, 256, 0, st>>>(c->geom.p, n, c->bb_misc.p);
+    rtz::bvh_boxes_kernel<<<gb, 256, 0, st>>>(c->geom.p, n, c->bb_misc.p, c->bb_lo.p, c->bb_hi.p);
+    rtz::BuildRange *rg = c->bb_rg0.p, *rg_next = c->bb_rg1.p;
+    rtz::bvh_init_kernel<<<gb, 256, 0, st>>>(n, order, c->bb_seg.p, rg, c->bb_acc.p);
+    for (int d = 0;; ++d) {
+        const int nr = 1 << d;
+        const unsigned rb = (unsigned)((nr + 255) / 256);
+        rtz::bvh_reduce_kernel<<<gb, 256, 0, st>>>(order, c->bb_seg.p, rg, c->geom.p, c->bb_lo.p, c->bb_hi.p, n, c->bb_acc.p);
+        rtz::bvh_node_kernel<<<rb, 256, 0, st>>>(rg, nr, c->bb_acc.p, nodes, c->bb_axis.p);
+        if (!rtz::bvh_level_splits(n, d)) break;
+        // the split: stable sorts by (range, index), then by (range, key); `order` takes the sorted indices
+        rtz::bvh_keys_index_kernel<<<gb, 256, 0, st>>>(order, c->bb_seg.p, n, c->bb_keys0.p);
+        size_t tb = c->bb_temp.cap;
+        RTZ_CUDA(cub::DeviceRadixSort::SortKeys(c->bb_temp.p, tb, c->bb_keys0.p, c->bb_keys1.p, n, 0, 20 + d, st));
+        rtz::bvh_keys_axis_kernel<<<gb, 256, 0, st>>>(c->bb_keys1.p, rg, c->bb_axis.p, c->geom.p, n, c->bb_keys0.p, c->bb_idx.p);
+        tb = c->bb_temp.cap;
+        RTZ_CUDA(cub::DeviceRadixSort::SortPairs(c->bb_temp.p, tb, c->bb_keys0.p, c->bb_keys1.p, c->bb_idx.p, order, n, 0,
+                                                 32 + d, st));
+        rtz::bvh_descend_kernel<<<gb, 256, 0, st>>>(rg, n, c->bb_seg.p);
+        rtz::bvh_ranges_kernel<<<(unsigned)((2 * nr + 255) / 256), 256, 0, st>>>(rg, 2 * nr, rg_next, c->bb_acc.p);
+        std::swap(rg, rg_next);
+    }
+    RTZ_CUDA(cudaGetLastError());
+    unsigned long long reach = 0;
+    RTZ_CUDA(cudaMemcpyAsync(&reach, c->bb_misc.p, sizeof reach, cudaMemcpyDeviceToHost, st));
+    RTZ_CUDA(cudaStreamSynchronize(st));
+    double r;
+    std::memcpy(&r, &reach, sizeof r);
+    *R_out = 2.0 * r;
+    return RTZ_OK;
+}
+
 int32_t ensure_bvh(rtz_context* c) {
     if (c->bvh_ready) return RTZ_OK;
-    const size_t n = (size_t)c->n_spheres;
-    BvhBuilder bvh(c->h_geom, (int)n);
-    bvh.run();
-    RTZ_CUDA(c->bvh_nodes.reserve(bvh.nodes.size()));
-    RTZ_CUDA(c->bvh_order.reserve(std::max<size_t>(1, bvh.order.size())));
-    RTZ_CUDA(cudaMemcpyAsync(c->bvh_nodes.p, bvh.nodes.data(), bvh.nodes.size() * sizeof(rtz::BvhNode), cudaMemcpyHostToDevice, c->stream));
-    if (n) {
-        RTZ_CUDA(cudaMemcpyAsync(c->bvh_order.p, bvh.order.data(), n * sizeof(int), cudaMemcpyHostToDevice, c->stream));
+    const int n = c->n_spheres;
+    double R = 0.0;
+    if (n >= kDeviceBvhMinSpheres) {
+        RTZ_CUDA(c->bvh_nodes.reserve(rtz::bvh_inner_nodes(n)));
+        RTZ_CUDA(c->bvh_order.reserve(n));
+        const int32_t rc = build_bvh_device(c, c->bvh_nodes.p, c->bvh_order.p, &R);
+        if (rc != RTZ_OK) return rc;
+    } else {
+        const int32_t rc = host_geom(c);
+        if (rc != RTZ_OK) return rc;
+        BvhBuilder bvh(c->h_geom, n);
+        bvh.run();
+        RTZ_CUDA(c->bvh_nodes.reserve(bvh.nodes.size()));
+        RTZ_CUDA(c->bvh_order.reserve(std::max<size_t>(1, bvh.order.size())));
+        RTZ_CUDA(cudaMemcpyAsync(c->bvh_nodes.p, bvh.nodes.data(), bvh.nodes.size() * sizeof(rtz::BvhNode),
+                                 cudaMemcpyHostToDevice, c->stream));
+        if (n) {
+            RTZ_CUDA(cudaMemcpyAsync(c->bvh_order.p, bvh.order.data(), n * sizeof(int), cudaMemcpyHostToDevice, c->stream));
+        }
+        RTZ_CUDA(cudaStreamSynchronize(c->stream));
+        R = bvh.R;
     }
-    RTZ_CUDA(cudaStreamSynchronize(c->stream));
-    c->bvh_r2 = (float)(bvh.R * bvh.R);
+    c->bvh_r2 = (float)(R * R);
     c->bvh_ready = true;
     return RTZ_OK;
 }
@@ -1103,26 +1275,27 @@ int32_t rtz_scene_generate(rtz_context* c, int32_t kind, uint64_t seed, uint64_t
     }
     rtz::scene_kernel<<<1, 1, 0, c->stream>>>(kind, seed, n_spheres, d_sp, dev_cap, d_res);
     rtz::SceneGenOut res{};
-    std::vector<rtz_sphere> host;
     cudaError_t e = cudaGetLastError();
     if (e == cudaSuccess) e = cudaMemcpyAsync(&res, d_res, sizeof res, cudaMemcpyDeviceToHost, c->stream);
     if (e == cudaSuccess) e = cudaStreamSynchronize(c->stream);
-    if (e == cudaSuccess && res.count > 0 && res.count <= dev_cap) {
-        host.resize(res.count);
-        e = cudaMemcpyAsync(host.data(), d_sp, res.count * sizeof(rtz_sphere), cudaMemcpyDeviceToHost, c->stream);
+    const bool full = res.count > 0 && res.count <= dev_cap;
+    if (e == cudaSuccess && full && out && cap) {  // only the spheres the caller asks for come to the host
+        e = cudaMemcpyAsync(out, d_sp, std::min(res.count, cap) * sizeof(rtz_sphere), cudaMemcpyDeviceToHost, c->stream);
         if (e == cudaSuccess) e = cudaStreamSynchronize(c->stream);
     }
+    // the device list is installed where it is (scene_upload_device synchronises before it returns)
+    int32_t rc = RTZ_OK;
+    if (e == cudaSuccess && full) rc = scene_upload_device(c, d_sp, res.count);
     cudaFree(d_sp), cudaFree(d_res);
     if (e != cudaSuccess) {
         g_last_error = cudaGetErrorString(e);
         return RTZ_ERR_CUDA;
     }
-    if (res.count == 0 || res.count > dev_cap) return RTZ_ERR_BAD_ARG;  // the sweep could not reach n spheres
+    if (!full) return RTZ_ERR_BAD_ARG;  // the sweep could not reach n spheres
+    if (rc != RTZ_OK) return rc;
     if (n_out) *n_out = res.count;
     if (state_out) std::memcpy(state_out, res.state, sizeof res.state);
-    if (out)
-        for (uint64_t i = 0; i < res.count && i < cap; ++i) out[i] = host[i];
-    return rtz_scene_upload(c, host.data(), res.count);
+    return RTZ_OK;
 }
 
 uint64_t rtz_shard_pixels(uint64_t W, uint64_t H, const rtz_shard* s) {
@@ -2040,7 +2213,7 @@ int32_t rtz_probe_cull_bounds(const rtz_sphere* sp, uint64_t n, float* boxes_out
                               int32_t* host_culls_out) {
     if ((!sp && n) || (!boxes_out && n) || !cull_r2_out || !host_culls_out || n > (1u << 20)) return RTZ_ERR_BAD_ARG;
     HostScene s;
-    const int32_t rc = host_scene(sp, n, s);
+    const int32_t rc = host_scene(sp, n, s, true);
     if (rc != RTZ_OK) return rc;
     for (int b = 0; b < (s.n_pad + 31) / 32; ++b) {
         const float4 b0 = s.boxes[2 * b], b1 = s.boxes[2 * b + 1];
@@ -2196,6 +2369,82 @@ int32_t rtz_probe_uniform(uint64_t seed, uint32_t pixel, uint32_t sample, uint32
     if (e == cudaSuccess) e = cudaStreamSynchronize(sc.c->stream);
     cudaFree(dout);
     RTZ_CUDA(e);
+    return RTZ_OK;
+}
+
+int32_t rtz_probe_scene_rows(rtz_context* c, void* out, uint64_t cap, uint64_t* bytes_out) {
+    if (!c || !bytes_out) return RTZ_ERR_BAD_ARG;
+    DeviceGuard guard;
+    RTZ_CUDA(cudaSetDevice(c->device));
+    const size_t np = (size_t)c->n_pad, n = (size_t)c->n_spheres;
+    const bool bank = np <= (size_t)rtz::kMaxConstSpheres, rg = bank && c->cull;
+    // {pointer, bytes, on the device}, in the order rtz.h lists
+    const int32_t head[4] = {c->n_spheres, c->n_pad, c->cull ? 1 : 0, 0};
+    float r2 = c->cull_r2;
+    struct Part {
+        const void* p;
+        size_t bytes;
+        bool dev;
+    };
+    const Part parts[] = {
+        {head, 12, false}, {&r2, 4, false},
+        {c->geom.p, np * 16, true}, {c->pairs.p, np * 16, true}, {c->aux.p, np * 16, true}, {c->albedo.p, np * 16, true},
+        {c->wexp.p, np * 4, true}, {c->dspheres.p, n * sizeof(rtz::DSphere), true},
+        {c->h_pairs.data(), bank ? np * 16 : 0, false}, {c->h_boxes.data(), bank ? c->h_boxes.size() * 16 : 0, false},
+        {c->rg_geom.p, rg ? np * 16 : 0, true}, {c->rg_aux.p, rg ? np * 16 : 0, true},
+        {c->rg_albedo.p, rg ? np * 16 : 0, true}, {c->rg_wexp.p, rg ? np * 4 : 0, true},
+        {c->rg_orig.p, rg ? np * 4 : 0, true}, {c->h_rg_pairs.data(), rg ? np * 16 : 0, false}};
+    size_t total = 0;
+    for (const Part& q : parts) total += q.bytes;
+    *bytes_out = total;
+    if (!out) return RTZ_OK;
+    if (cap < total) return RTZ_ERR_BAD_ARG;
+    uint8_t* dst = static_cast<uint8_t*>(out);
+    for (const Part& q : parts) {
+        if (q.bytes && q.dev) RTZ_CUDA(cudaMemcpyAsync(dst, q.p, q.bytes, cudaMemcpyDeviceToHost, c->stream));
+        if (q.bytes && !q.dev) std::memcpy(dst, q.p, q.bytes);
+        dst += q.bytes;
+    }
+    RTZ_CUDA(cudaStreamSynchronize(c->stream));
+    return RTZ_OK;
+}
+
+int32_t rtz_probe_bvh(rtz_context* c, int32_t builder, void* nodes_out, uint64_t node_cap, int32_t* order_out,
+                      float* r2_out, uint64_t* n_nodes_out) {
+    if (!c || (builder != RTZ_BVH_HOST && builder != RTZ_BVH_DEVICE)) return RTZ_ERR_BAD_ARG;
+    DeviceGuard guard;
+    RTZ_CUDA(cudaSetDevice(c->device));
+    const int n = c->n_spheres;
+    if (builder == RTZ_BVH_DEVICE && n >= 5) {  // below 5 spheres the tree is one root over one leaf: the host's
+        const uint64_t count = (uint64_t)rtz::bvh_inner_nodes(n);
+        if (n_nodes_out) *n_nodes_out = count;
+        if (nodes_out && node_cap < count) return RTZ_ERR_BAD_ARG;
+        rtz::BvhNode* d_nodes = nullptr;
+        int* d_order = nullptr;
+        RTZ_CUDA(cudaMalloc(&d_nodes, count * sizeof(rtz::BvhNode)));
+        cudaError_t e = cudaMalloc(&d_order, (size_t)n * sizeof(int));
+        double R = 0.0;
+        int32_t rc = e == cudaSuccess ? build_bvh_device(c, d_nodes, d_order, &R) : RTZ_OK;
+        if (e == cudaSuccess && rc == RTZ_OK && nodes_out)
+            e = cudaMemcpyAsync(nodes_out, d_nodes, count * sizeof(rtz::BvhNode), cudaMemcpyDeviceToHost, c->stream);
+        if (e == cudaSuccess && rc == RTZ_OK && order_out)
+            e = cudaMemcpyAsync(order_out, d_order, (size_t)n * sizeof(int), cudaMemcpyDeviceToHost, c->stream);
+        if (e == cudaSuccess) e = cudaStreamSynchronize(c->stream);
+        cudaFree(d_nodes), cudaFree(d_order);
+        if (rc != RTZ_OK) return rc;
+        RTZ_CUDA(e);
+        if (r2_out) *r2_out = (float)(R * R);
+        return RTZ_OK;
+    }
+    const int32_t rc = host_geom(c);
+    if (rc != RTZ_OK) return rc;
+    BvhBuilder bvh(c->h_geom, n);
+    bvh.run();
+    if (n_nodes_out) *n_nodes_out = bvh.nodes.size();
+    if (nodes_out && node_cap < bvh.nodes.size()) return RTZ_ERR_BAD_ARG;
+    if (nodes_out) std::memcpy(nodes_out, bvh.nodes.data(), bvh.nodes.size() * sizeof(rtz::BvhNode));
+    if (order_out) std::copy(bvh.order.begin(), bvh.order.end(), order_out);
+    if (r2_out) *r2_out = (float)(bvh.R * bvh.R);
     return RTZ_OK;
 }
 

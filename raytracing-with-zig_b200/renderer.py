@@ -19,6 +19,27 @@ def _as_sphere_array(spheres):
     return arr, len(spheres)
 
 
+def pack_spheres(center, radius, mat_type, albedo, fuzz, refraction_index):
+    """`rtz_sphere` records built on the device with torch ops: a contiguous float64 [n, 10] tensor on the device of
+    `center` (column 4 holds the int32 pair (mat_type, reserved = 0)), what `Renderer.upload` installs without a host
+    round trip.  center, albedo: [n, 3]; radius, mat_type, fuzz, refraction_index: [n] (or anything that broadcasts)."""
+    import torch
+
+    center = torch.as_tensor(center)
+    n, dev = center.shape[0], center.device
+    out = torch.empty((n, 10), dtype=torch.float64, device=dev)
+    f64 = dict(dtype=torch.float64, device=dev)
+    out[:, 0:3] = torch.as_tensor(center, **f64)
+    out[:, 3] = torch.as_tensor(radius, **f64)
+    out[:, 5:8] = torch.as_tensor(albedo, **f64)
+    out[:, 8] = torch.as_tensor(fuzz, **f64)
+    out[:, 9] = torch.as_tensor(refraction_index, **f64)
+    words = out.view(torch.int32)  # [n, 20]: column 4 is words 8 (mat_type) and 9 (reserved)
+    words[:, 8] = torch.as_tensor(mat_type, dtype=torch.int32, device=dev)
+    words[:, 9] = 0
+    return out
+
+
 def _cast_camera(cam) -> B.rtz_camera:
     """Accept any ctypes struct with the rtz_camera layout (tests use their own mirror class)."""
     if isinstance(cam, B.rtz_camera):
@@ -68,7 +89,23 @@ class Renderer:
             pass
 
     def upload(self, spheres, n: int | None = None):
-        """HittableList.add for the whole list: flatten to the device SoA and copy to HBM."""
+        """HittableList.add for the whole list: flatten to the device SoA and copy to HBM.  A CUDA tensor of
+        `rtz_sphere` records (float64 [n, 10], contiguous, on this renderer's device: `pack_spheres`) is installed
+        from device memory (`rtz_scene_upload_device`), ordered after torch's current stream."""
+        torch = self.torch
+        if isinstance(spheres, torch.Tensor):
+            t = spheres
+            if not t.is_cuda or t.device.index != self.device:
+                raise ValueError(f"spheres on {t.device}: this renderer installs device tensors of cuda:{self.device}")
+            if t.dtype != torch.float64 or t.dim() != 2 or t.shape[1] != 10 or not t.is_contiguous():
+                raise ValueError("spheres must be a contiguous float64 [n, 10] tensor of rtz_sphere records")
+            n = t.shape[0] if n is None else int(n)
+            if n > t.shape[0]:
+                raise ValueError(f"n = {n} but the tensor holds {t.shape[0]} spheres")
+            self._order_after_torch()
+            B.check(self.lib.rtz_scene_upload_device(self._ctx, C.c_void_p(t.data_ptr() if n else 0), n))
+            self.n_spheres = n
+            return
         arr, cnt = _as_sphere_array(spheres)
         n = cnt if n is None else int(n)
         ptr = C.cast(arr, C.POINTER(B.rtz_sphere))
